@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the MISA training step (BASELINE.json metric: MOSEI-shape train samples/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of solver.py:139-186 (zero_grad, forward, six losses, backward, clip, Adam)
@@ -25,6 +25,7 @@ sys.path.insert(0, ROOT)
 
 SEQ, BATCH, VOCAB = 50, 256, 20000     # BASELINE configs[1]; --seq / --batch override (configs[4] sweep)
 METRIC, UNIT = "train_samples_per_sec", "samples/s"
+DUMP_SAMPLE = 4 << 20                  # --dump-outputs: elements kept of the parameters / gradients
 
 
 def workload(batch, lengths):
@@ -153,7 +154,7 @@ def cpu_steps(steps, warmup, budget_s=150.0, batch=BATCH, lengths="full"):
 def run_reference(args, rank):
     if rank != 0:
         return
-    cb = cpu_steps(args.steps, args.warmup, batch=args.batch, lengths=args.lengths)
+    cb = cpu_steps(args.steps, args.warmup, budget_s=float("inf"), batch=args.batch, lengths=args.lengths)
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT,
             "n_gpus": args.gpus, "steps": cb["steps"], "warmup": args.warmup,
             "ms_per_step": cb["ms_per_step"], "higher_is_better": True, "scaling": "weak",
@@ -312,6 +313,27 @@ def dp_check(dist, pg, rank, world, dev):
     return out
 
 
+def dump_outputs(out_dir, tr, losses):
+    """Write what one step computed as float32 ``out_dir/<name>.npy``, so that two builds can be
+    compared output for output: ``losses`` (the vector ``FusedTrainer.step`` returns), and the
+    updated ``params`` and their ``grads``, each flattened in ``named_parameters()`` order (not the
+    arena layout, which may change) and sampled at DUMP_SAMPLE fixed, seeded positions when larger
+    (32 MiB in all for the MOSEI shape)."""
+    import numpy as np
+    named = list(tr.model.named_parameters())
+    params = torch.cat([p.detach().reshape(-1) for _, p in named])
+    grads = torch.cat([tr.G[n].reshape(-1) for n, _ in named])
+    idx = None
+    if params.numel() > DUMP_SAMPLE:
+        perm = torch.randperm(params.numel(), generator=torch.Generator().manual_seed(0))
+        idx = perm[:DUMP_SAMPLE].sort().values.to(params.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("losses", losses.reshape(-1)), ("params", params), ("grads", grads)):
+        if idx is not None and name != "losses":
+            t = t[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------
@@ -387,6 +409,8 @@ def run_ours(args):
     host_ms = 1e3 * (time.perf_counter() - h0) / args.steps    # host enqueue time (no sync)
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, tr, losses)
     launches = (args.steps * tr.launches_per_step) if graph_on else (eng.k.launches - l0)
     n_graphs = len(tr._graphs)
     ms = e0.elapsed_time(e1)
@@ -491,7 +515,11 @@ def main():
     ap.add_argument("--seq", type=int, default=SEQ)
     ap.add_argument("--precision", default="fp32", choices=["fp32", "bf16"])
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's losses, parameters and gradients as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     SEQ = args.seq
     if args.impl == "reference":
         run_reference(args, int(os.environ.get("RANK", "0")))

@@ -376,6 +376,41 @@ def test_bench_clock_sampler_covers_short_runs(tmp_path, monkeypatch):
     assert c.stop()["reasons"] == ["nvidia-smi unavailable"]
 
 
+def test_bench_dump_outputs(dryrun, tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 .npy files of the step's losses and of the parameters and
+    gradients in named_parameters() order; above DUMP_SAMPLE elements both are sampled at the same
+    positions, and every run picks the same ones."""
+    import importlib.util
+    import numpy as np
+    from mmda_b200.trainer import FusedTrainer
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("bench_mod3", os.path.join(root, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    torch.manual_seed(0)
+    model = MISA(mosei_config(vocab_size=60, batch_size=4))
+    tr = FusedTrainer(model)
+    tr.g_arena.copy_(2 * tr.p_arena + 1)
+    flat = torch.cat([p.detach().reshape(-1) for p in model.parameters()]).numpy()
+    losses = torch.arange(8, dtype=torch.float32)
+
+    def dump(name):
+        bench.dump_outputs(str(tmp_path / name), tr, losses)
+        return {k: np.load(tmp_path / name / (k + ".npy")) for k in ("losses", "params", "grads")}
+
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", flat.size)
+    full = dump("full")
+    assert all(v.dtype == np.float32 for v in full.values())
+    assert np.array_equal(full["losses"], losses.numpy())
+    assert np.array_equal(full["params"], flat) and np.array_equal(full["grads"], 2 * flat + 1)
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 1000)
+    a, b = dump("a"), dump("b")
+    assert a["params"].shape == a["grads"].shape == (1000,)
+    assert np.array_equal(a["grads"], 2 * a["params"] + 1)
+    assert np.isin(a["params"], flat).all()
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+
+
 @pytest.mark.parametrize("variant", [dict(rnncell="gru"), dict(use_cmd_sim=False),
                                      dict(rnncell="gru", use_cmd_sim=False, use_confidNet=True)])
 def test_variant_kernel_sequences(dryrun, variant):
