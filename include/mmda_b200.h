@@ -138,8 +138,12 @@ int mmda_lstm_backward(float* gates, const float* whh_f, const float* whh_r, con
                        int utt_off_r, const int* lens_sorted, const int* sorted_idx,
                        const int* offsets, float* scratch, int B, int H, int Tmax,
                        mmda_stream_t stream);
+/* Backward scratch bytes for (B, H), -1 if H is not covered.  The plan depends on (B, H) and the
+ * device only, never on Tmax, so this size and mmda_lstm_plan hold for every Tmax of a launch
+ * with the same B and H (mmda_lstm_* and mmda_gru_* alike). */
 long long mmda_lstm_scratch_bytes(int B, int H);
-/* out6 = {cluster size, units per CTA, batch tile, n batch tiles, smem fwd, smem bwd} */
+/* out6 = {cluster size, units per CTA, batch tile, n batch tiles, smem fwd, smem bwd}; the
+ * contraction split of the backward is 16 lanes for H > 128, else 4 */
 int mmda_lstm_plan(int B, int H, int* out6);
 /* stacked gate-interleaved copy of W_ih (both directions) + bias stack for the hoisted GEMMs:
  * row dir*4H+u*4+g <- row g*H+u.  mode 0 fp32 (out_a), 1 tf32 hi/lo (out_a,out_b), 2 bf16 (out_a). */

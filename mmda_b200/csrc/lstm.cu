@@ -42,7 +42,7 @@ struct LstmArgs {
   const float* dy;        // bwd: grad wrt y [N][2H] (nullable)
   float* scratch;         // bwd: partial-sum exchange [2][n_clusters][C][BT][Kpad]
   int utt_ld, utt_off0, utt_off1;
-  int B, H, Hs, Kpad, C, n_tiles, save, Tmax;
+  int B, H, Hs, Kpad, C, n_tiles, save;
   long long* dbg;         // optional per-step phase timestamps (profiling builds of the bench)
 };
 
@@ -277,7 +277,6 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_bwd_kernel(const
   float* dG_s = smem + R * Kpad;    // [R][BTP]
   int* lens_s = reinterpret_cast<int*>(dG_s + R * BTP);
   int* orig_s = lens_s + BT;
-  int* offs_s = orig_s + BT;        // [Tmax+1]
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   constexpr int BG = BT / 8;
@@ -307,7 +306,6 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_bwd_kernel(const
       Wb[idx] = (k < H && ul < Hs && ugl < H) ? W[(size_t)(g * H + ugl) * H + k] : 0.f;
     }
     for (int idx = tid; idx < R * BTP; idx += blockDim.x) dG_s[idx] = 0.f;
-    for (int idx = tid; idx <= p.Tmax; idx += blockDim.x) offs_s[idx] = p.offsets[idx];
     if (tid < BT) {
       const int b = b_base + tid;
       lens_s[tid] = b < p.B ? p.lens[b] : 0;
@@ -378,10 +376,13 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_bwd_kernel(const
     cluster_arrive();   // release: this CTA's partials are published
     // ---- fetch everything the cell update needs while the cluster barrier completes ----
     const bool a0 = u_ok && t < len0, a1 = u_ok && t < len1;
-    const int off_t = offs_s[t];
+    // offsets are read from global memory, as in the forward kernel: staging them in shared
+    // memory would make the footprint, and with it the plan and the scratch size, depend on Tmax
+    const int off_t = __ldg(p.offsets + t);
     const size_t row0 = (size_t)(off_t + b_base + ebl0), row1 = row0 + 1;
     // forward-order predecessor time (its c is c_{prev}); forward-order successor feeds dh_rec
     const int tp = dir == 0 ? t - 1 : t + 1;
+    const int off_tp = tp >= 0 ? __ldg(p.offsets + tp) : 0;   // tp <= Lmax <= Tmax
     float g0[4], g1[4], ct0 = 0.f, ct1 = 0.f, cp0 = 0.f, cp1 = 0.f, dh0 = 0.f, dh1 = 0.f;
     bool rec0 = false, rec1 = false;
     if (a0) {
@@ -391,7 +392,7 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_bwd_kernel(const
       }
       ct0 = p.c[row0 * H2 + ycol];
       const bool hp = dir == 0 ? (t >= 1) : (t + 1 < len0);
-      if (hp) cp0 = p.c[(size_t)(offs_s[tp] + b_base + ebl0) * H2 + ycol];
+      if (hp) cp0 = p.c[(size_t)(off_tp + b_base + ebl0) * H2 + ycol];
       if (p.dy) dh0 = p.dy[row0 * H2 + ycol];
       const bool fin = dir == 0 ? (t == len0 - 1) : (t == 0);
       if (fin && p.dutt) dh0 += p.dutt[(size_t)orig0 * p.utt_ld + utt_off + u_glob];
@@ -404,7 +405,7 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_bwd_kernel(const
       }
       ct1 = p.c[row1 * H2 + ycol];
       const bool hp = dir == 0 ? (t >= 1) : (t + 1 < len1);
-      if (hp) cp1 = p.c[(size_t)(offs_s[tp] + b_base + ebl0 + 1) * H2 + ycol];
+      if (hp) cp1 = p.c[(size_t)(off_tp + b_base + ebl0 + 1) * H2 + ycol];
       if (p.dy) dh1 = p.dy[row1 * H2 + ycol];
       const bool fin = dir == 0 ? (t == len1 - 1) : (t == 0);
       if (fin && p.dutt) dh1 += p.dutt[(size_t)orig1 * p.utt_ld + utt_off + u_glob];
@@ -626,7 +627,7 @@ template <int BT> static int probe_clusters8(int threads, size_t smem) {
   return n;
 }
 
-static int lstm_make_plan(int B, int H, int Tmax, LstmPlan* pl) {
+static int lstm_make_plan(int B, int H, LstmPlan* pl) {
   MmdaDeviceCtx* ctx = mmda_device_ctx();
   if (ctx == nullptr) return MMDA_ERR_CUDA;
   const size_t max_smem = (size_t)ctx->max_smem_optin;
@@ -645,7 +646,7 @@ static int lstm_make_plan(int B, int H, int Tmax, LstmPlan* pl) {
       const size_t misc = (size_t)(2 * BT) * 4 + 16;
       const int HR = C * Hs > Kpad ? C * Hs : Kpad;
       const size_t fwd = (size_t)4 * Kpad * Hs * 4 + (size_t)HR * BTP * 4 + misc;
-      const size_t bwd = (size_t)R * Kpad * 4 + (size_t)R * BTP * 4 + misc + (size_t)(Tmax + 1) * 4;
+      const size_t bwd = (size_t)R * Kpad * 4 + (size_t)R * BTP * 4 + misc;
       if (fwd > max_smem || bwd > max_smem) continue;
       const int UG = (Hs + 7) / 8, BG = BT / 8, K4 = Kpad / 4;
       const int KG = (K4 + KS - 1) / KS;
@@ -712,14 +713,14 @@ int mmda_lstm_set_debug_buffer(long long* dev_buf) {
 
 long long mmda_lstm_scratch_bytes(int B, int H) {
   LstmPlan pl;
-  if (lstm_make_plan(B, H, 1, &pl) != MMDA_OK) return -1;
+  if (lstm_make_plan(B, H, &pl) != MMDA_OK) return -1;
   return (long long)pl.scratch_bytes;
 }
 
 // cluster size / units per CTA / batch tile the plan picks (for DESIGN.md, tests and the bench)
 int mmda_lstm_plan(int B, int H, int* out6) {
   LstmPlan pl;
-  int rc = lstm_make_plan(B, H, 1, &pl);
+  int rc = lstm_make_plan(B, H, &pl);
   if (rc != MMDA_OK) return rc;
   out6[0] = pl.C; out6[1] = pl.Hs; out6[2] = pl.BT; out6[3] = pl.n_tiles;
   out6[4] = (int)pl.smem_fwd; out6[5] = (int)pl.smem_bwd;
@@ -755,16 +756,15 @@ int mmda_lstm_probe_clusters(int smem_bytes, int threads, int* out5) {
 
 static int rnn_forward(int cell, float* gates, const float* whh_f, const float* whh_r, float* y,
                        float* c, const int* lens_sorted, const int* sorted_idx, const int* offsets,
-                       float* utt, int utt_ld, int utt_off_f, int utt_off_r, int B, int H, int Tmax,
+                       float* utt, int utt_ld, int utt_off_f, int utt_off_r, int B, int H,
                        int save_for_backward, cudaStream_t stream) {
   MMDA_REQUIRE(B > 0 && H > 0, "rnn_forward: bad sizes B=%d H=%d", B, H);
   MMDA_REQUIRE(cell == 1 || !save_for_backward || c != nullptr,
                "lstm_forward: c buffer required when saving");
   LstmPlan pl;
-  int rc = lstm_make_plan(B, H, Tmax, &pl);
+  int rc = lstm_make_plan(B, H, &pl);
   if (rc != MMDA_OK) return rc;
   LstmArgs a = {};
-  a.Tmax = Tmax;
   a.gates = gates; a.whh[0] = whh_f; a.whh[1] = whh_r; a.y = y; a.c = c;
   a.lens = lens_sorted; a.sorted_idx = sorted_idx; a.offsets = offsets;
   a.utt = utt; a.utt_ld = utt_ld; a.utt_off0 = utt_off_f; a.utt_off1 = utt_off_r;
@@ -785,15 +785,14 @@ static int rnn_backward(int cell, float* gates, const float* whh_f, const float*
                         const float* c, const float* dy, const float* dutt, int utt_ld,
                         int utt_off_f, int utt_off_r, const int* lens_sorted,
                         const int* sorted_idx, const int* offsets, float* scratch, int B, int H,
-                        int Tmax, cudaStream_t stream) {
+                        cudaStream_t stream) {
   MMDA_REQUIRE(B > 0 && H > 0, "rnn_backward: bad sizes B=%d H=%d", B, H);
   MMDA_REQUIRE(c != nullptr, "rnn_backward: saved cell states (LSTM) / hidden states (GRU) required");
   MMDA_REQUIRE(scratch != nullptr, "lstm_backward: scratch required (mmda_lstm_scratch_bytes)");
   LstmPlan pl;
-  int rc = lstm_make_plan(B, H, Tmax, &pl);
+  int rc = lstm_make_plan(B, H, &pl);
   if (rc != MMDA_OK) return rc;
   LstmArgs a = {};
-  a.Tmax = Tmax;
   a.gates = gates; a.whh[0] = whh_f; a.whh[1] = whh_r; a.c = const_cast<float*>(c);
   a.dy = dy; a.dutt = dutt; a.utt_ld = utt_ld; a.utt_off0 = utt_off_f; a.utt_off1 = utt_off_r;
   a.lens = lens_sorted; a.sorted_idx = sorted_idx; a.offsets = offsets; a.scratch = scratch;
@@ -822,7 +821,7 @@ int mmda_lstm_forward(float* gates, const float* whh_f, const float* whh_r, floa
                       float* utt, int utt_ld, int utt_off_f, int utt_off_r, int B, int H, int Tmax,
                       int save_for_backward, cudaStream_t stream) {
   return rnn_forward(0, gates, whh_f, whh_r, y, c, lens_sorted, sorted_idx, offsets, utt, utt_ld,
-                     utt_off_f, utt_off_r, B, H, Tmax, save_for_backward, stream);
+                     utt_off_f, utt_off_r, B, H, save_for_backward, stream);
 }
 
 int mmda_lstm_backward(float* gates, const float* whh_f, const float* whh_r, const float* c,
@@ -831,7 +830,7 @@ int mmda_lstm_backward(float* gates, const float* whh_f, const float* whh_r, con
                        const int* offsets, float* scratch, int B, int H, int Tmax,
                        cudaStream_t stream) {
   return rnn_backward(0, gates, whh_f, whh_r, c, dy, dutt, utt_ld, utt_off_f, utt_off_r,
-                      lens_sorted, sorted_idx, offsets, scratch, B, H, Tmax, stream);
+                      lens_sorted, sorted_idx, offsets, scratch, B, H, stream);
 }
 
 // nn.GRU variant (reference src/models.py:39,168-169,177-178).  Same kernels, 4-slot layout:
@@ -842,7 +841,7 @@ int mmda_gru_forward(float* gates, const float* whh4_f, const float* whh4_r, flo
                      int utt_ld, int utt_off_f, int utt_off_r, int B, int H, int Tmax,
                      int save_for_backward, cudaStream_t stream) {
   return rnn_forward(1, gates, whh4_f, whh4_r, y, nullptr, lens_sorted, sorted_idx, offsets, utt,
-                     utt_ld, utt_off_f, utt_off_r, B, H, Tmax, save_for_backward, stream);
+                     utt_ld, utt_off_f, utt_off_r, B, H, save_for_backward, stream);
 }
 
 // After the call gates4 holds (d r_pre, d z_pre, d n_pre, d n_pre * r): slots 0,1,2 are the
@@ -852,7 +851,7 @@ int mmda_gru_backward(float* gates, const float* whh4_f, const float* whh4_r, co
                       const int* lens_sorted, const int* sorted_idx, const int* offsets,
                       float* scratch, int B, int H, int Tmax, cudaStream_t stream) {
   return rnn_backward(1, gates, whh4_f, whh4_r, y, dy, dutt, utt_ld, utt_off_f, utt_off_r,
-                      lens_sorted, sorted_idx, offsets, scratch, B, H, Tmax, stream);
+                      lens_sorted, sorted_idx, offsets, scratch, B, H, stream);
 }
 
 int mmda_gru_expand_weights(const float* w_ih, const float* w_hh, const float* b_ih,

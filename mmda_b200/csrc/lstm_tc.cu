@@ -531,7 +531,8 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
   fence_after();
   const uint32_t tm = *reinterpret_cast<uint32_t*>(sptr + misc_off + 96);
   auto w_blk = [&](int mt, int term) { return tm + (uint32_t)((mt * 2 + term) * Kc); };
-  const uint32_t tmD = tm + (uint32_t)((MT * 2 * Kc + 4 + 15) & ~15);   // [sub-tile][M tile][16 columns]
+  const int Kover = 64 - Kc;                  // columns the 8 K steps of the last block read past it
+  const uint32_t tmD = tm + (uint32_t)((MT * 2 * Kc + Kover + 15) & ~15);   // [sub-tile][M tile][16 columns]
   const uint32_t lane_sel = (uint32_t)(q * 32) << 16;
 
   if (warp < TCL_CELL_WARPS) {  // A[j][rho] = W_hh[(rho&3)*H + r*U + (rho>>2)][j], rho < 4U
@@ -553,9 +554,11 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
         tmem_st4(w_blk(mt, 1) + lane_sel + ck * 4, w2.x, w2.y, w2.z, w2.w);
       }
     }
-    // the last K step of a block may read 4 columns past it: W of the next block (finite, times
-    // the zero rows of the B operand) -- and these zero columns after the last block
-    if (hc == 0) tmem_st4(tm + lane_sel + (uint32_t)(MT * 2 * Kc), 0u, 0u, 0u, 0u);
+    // the 8 K steps of a block read 64 - Kc columns past it (up to 12 at U = 26): W of the next
+    // block (finite, times the zero rows of the B operand) -- and these zero columns after the
+    // last block (uninitialised TMEM may hold NaN, and NaN * 0 is NaN)
+    for (int ck = hc; ck < Kover / 4; ck += 2)
+      tmem_st4(tm + lane_sel + (uint32_t)(MT * 2 * Kc + ck * 4), 0u, 0u, 0u, 0u);
     tmem_wait_st();
   }
   for (uint32_t i = tid; i < BMAXSUB * BWD_SUB_BYTES / 16; i += TCL_BWD_THREADS4)
@@ -911,7 +914,7 @@ int tcl_make_plan(int B, int H, int Tmax, TclPlan* pl) {
   int Sb = pl->S, Ub = 0;
   for (;; ++Sb) {
     Ub = ((H + Sb - 1) / Sb + 1) & ~1;
-    if (((MT * 2 * 2 * Ub + 4 + 15) & ~15) + BMAXSUB * MT * BSUB <= 512 && Ub <= TCL_UNITS) break;
+    if (((MT * 2 * 2 * Ub + 64 - 2 * Ub + 15) & ~15) + BMAXSUB * MT * BSUB <= 512 && Ub <= TCL_UNITS) break;
     if (Sb > 64) return MMDA_ERR_UNSUPPORTED;
   }
   pl->Sb = Sb; pl->Ub = Ub;

@@ -15,7 +15,8 @@ TOL = 1e-5
 
 
 @pytest.mark.parametrize("B,H,T,ragged", [(40, 300, 6, 1), (256, 300, 50, 0), (64, 300, 30, 1),
-                                          (100, 200, 20, 1), (300, 300, 12, 1), (7, 160, 9, 1)])
+                                          (100, 200, 20, 1), (300, 300, 12, 1), (7, 160, 9, 1),
+                                          (37, 129, 7, 1), (50, 320, 9, 1), (1, 300, 1, 0)])
 def test_tc_recurrence_vs_fp64(B, H, T, ragged):
     import dev_lstm_tc as D
     dev = torch.device("cuda:0")
