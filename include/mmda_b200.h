@@ -396,6 +396,45 @@ int mmda_bert_attention_backward_mma(const float* qkv, const float* probs, const
                                      int head_dim, float p_drop,
                                      unsigned long long seed, const unsigned long long* seed_dev,
                                      unsigned stream_id, mmda_stream_t stream);
+/* The calls above keep the whole S x S problem of one (sample, head) in shared memory.  This
+ * returns the largest S the fp32 ones take (backward != 0: the backward; 84, else 116), from the
+ * same shared-memory budget their launchers check. */
+int mmda_bert_attention_resident_max_seq(int backward);
+/* Tiled (flash-style) self-attention for any S up to the position embeddings: 64-row query / key
+ * tiles stream through shared memory with an online softmax, so nothing of size S x S exists.
+ * Same qkv / mask / ctx layouts, masking (weight exactly 0), dropout stream and element indexing
+ * ((b*nhead + h)*S*S + i*S + j, so B*nhead*S*S < 2^32 is required) as the calls above; every
+ * query row is computed, padded ones too, as HF BertSelfAttention does (transformers, called from
+ * src/models.py:186-193).  Instead of probs the forward writes lse [B][nhead][S] fp32 = row max +
+ * log(row sum) of the scaled, masked scores (lse == NULL: eval).  The backward recomputes
+ * P = exp(s*scale - lse) tile by tile; delta ([B][nhead][S] fp32) is caller-owned scratch for
+ * D_i = rowsum(dPd o Pd): _tiled computes it as sum_c dctx[i][c]*ctx[i][c]; _tiled_mma computes
+ * it from its own bf16 products (as the _mma backward does: the ctx identity holds only up to bf16
+ * rounding, which a row with one valid key would turn into its whole gradient), so there ctx is
+ * not read and may be NULL.  It writes all of dqkv (dQ, dK, dV) without atomics: two
+ * identical launches give identical bits.  _tiled runs exact fp32 FFMA; _tiled_mma runs mma.sync
+ * m16n8k16 bf16 with fp32 accumulation and fp32 softmax, with the nullable bf16 operand copies
+ * ctx_bf16 / dqkv_bf16 as in the _mma calls.  head_dim must be 64. */
+int mmda_bert_attention_forward_tiled(const float* qkv, const long long* mask, float* ctx, float* lse,
+                                      int B, int S, int nhead, int head_dim, float p_drop,
+                                      unsigned long long seed, const unsigned long long* seed_dev,
+                                      unsigned stream_id, mmda_stream_t stream);
+int mmda_bert_attention_backward_tiled(const float* qkv, const long long* mask, const float* ctx,
+                                       const float* lse, const float* dctx, float* delta, float* dqkv,
+                                       int B, int S, int nhead, int head_dim, float p_drop,
+                                       unsigned long long seed, const unsigned long long* seed_dev,
+                                       unsigned stream_id, mmda_stream_t stream);
+int mmda_bert_attention_forward_tiled_mma(const float* qkv, const long long* mask, float* ctx,
+                                          void* ctx_bf16, float* lse, int B, int S, int nhead,
+                                          int head_dim, float p_drop, unsigned long long seed,
+                                          const unsigned long long* seed_dev, unsigned stream_id,
+                                          mmda_stream_t stream);
+int mmda_bert_attention_backward_tiled_mma(const float* qkv, const long long* mask, const float* ctx,
+                                           const float* lse, const float* dctx, float* delta,
+                                           float* dqkv, void* dqkv_bf16, int B, int S, int nhead,
+                                           int head_dim, float p_drop, unsigned long long seed,
+                                           const unsigned long long* seed_dev, unsigned stream_id,
+                                           mmda_stream_t stream);
 
 /* ---- device-resident collate (SURVEY.md 8f N3): collate_fn, src/data_loader.py:59-122, and the
  * per-tensor to_gpu copies, src/utils/convert.py:4-11.  The split lives in HBM as ragged flat

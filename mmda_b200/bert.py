@@ -19,7 +19,7 @@ import os
 
 import torch
 
-from ._lib import MmdaError
+from ._lib import LIB, MmdaError
 
 PFX = "bertmodel."
 
@@ -46,6 +46,7 @@ class BertEngine:
         self._pver = None
         self.saved = None
         self._wcache, self._par = {}, {}
+        self._resident_max = {}
 
     # ------------------------------------------------------------------ parameters ---------
     def params(self) -> Dict[str, torch.Tensor]:
@@ -138,10 +139,20 @@ class BertEngine:
         self.k._c("mmda_gelu_forward", _ptr(pre), _ptr(act), None, M * I)
         return self._op("bert_opI", act)
 
-    def _att_sfx(self, S):
-        """bf16 mode runs the attention core on the tensor pipe (sequences up to 64 tokens)"""
-        return "_mma" if self.eng.tc_kind == 1 and S <= 64 and \
-            os.environ.get("MMDA_BERT_ATT", "mma") != "simt" else ""
+    def _att_sfx(self, S, train):
+        """Entry-point suffix of the attention core at sequence length S.  bf16 mode runs it on the
+        tensor pipe up to 64 tokens; the shared-memory resident fp32 kernels take what fits them
+        (S <= 84 with a backward, S <= 116 without); longer sequences go to the tiled kernels
+        (`_tiled_mma` in bf16 mode, `_tiled` in fp32 mode), which hold no S x S buffer."""
+        bf = self.eng.tc_kind == 1
+        if bf and S <= 64 and os.environ.get("MMDA_BERT_ATT", "mma") != "simt":
+            return "_mma"
+        key = 1 if train else 0
+        if key not in self._resident_max:
+            self._resident_max[key] = int(LIB.raw("mmda_bert_attention_resident_max_seq")(key))
+        if S <= self._resident_max[key]:
+            return ""
+        return "_tiled_mma" if bf else "_tiled"
 
     def _opbuf(self, name, M):
         """bf16 operand buffer a producer kernel writes directly (bf16 mode), else None"""
@@ -212,14 +223,28 @@ class BertEngine:
                     self._mm(0, 0, M, H, H, xop, self._wop(P, Lp + f"attention.self.{nm}.weight"),
                              QKV[:, j * H:(j + 1) * H], bias=P[Lp + f"attention.self.{nm}.bias"])
             ctx = buf(f"bert_ctx_{l}", M, H)
-            probs = buf(f"bert_probs_{l}", B, nh, S, S) if train else None
-            sfx = self._att_sfx(S)
-            if sfx:      # tensor-pipe core: writes the out-projection's bf16 operand itself
+            sfx = self._att_sfx(S, train)
+            if sfx.startswith("_tiled"):     # O(S) per (sample, head): one lse per row, no probs
+                lse = buf(f"bert_lse_{l}", B, nh, S) if train else None
+                if sfx == "_tiled_mma":
+                    ctx_bf = self._opbuf("bert_opH", M)
+                    k._c("mmda_bert_attention_forward_tiled_mma", _ptr(QKV), _ptr(mask),
+                         _ptr(ctx) if train else None, _ptr(ctx_bf), _ptr(lse), B, S, nh, 64, p_a,
+                         seed, _ptr(seed_dev), 201 + 4 * l)
+                    ctx_op = (ctx_bf, None)
+                else:
+                    k._c("mmda_bert_attention_forward_tiled", _ptr(QKV), _ptr(mask), _ptr(ctx),
+                         _ptr(lse), B, S, nh, 64, p_a, seed, _ptr(seed_dev), 201 + 4 * l)
+                    ctx_op = self._op("bert_opH", ctx)
+                probs = None
+            else:
+                probs = buf(f"bert_probs_{l}", B, nh, S, S) if train else None
+            if sfx == "_mma":      # tensor-pipe core: writes the out-projection's bf16 operand itself
                 ctx_bf = self._opbuf("bert_opH", M)
                 k._c("mmda_bert_attention_forward_mma", _ptr(QKV), _ptr(mask), _ptr(ctx) if train else None,
                      _ptr(ctx_bf), _ptr(probs), B, S, nh, 64, p_a, seed, _ptr(seed_dev), 201 + 4 * l)
                 ctx_op = (ctx_bf, None)
-            else:
+            elif not sfx:
                 k._c("mmda_bert_attention_forward", _ptr(QKV), _ptr(mask), _ptr(ctx), _ptr(probs), B, S,
                      nh, 64, p_a, seed, _ptr(seed_dev), 201 + 4 * l)
                 ctx_op = self._op("bert_opH", ctx)
@@ -300,7 +325,6 @@ class BertEngine:
             Lp = f"{PFX}encoder.layer.{l}."
             x = buf(f"bert_x_{l}", M, H)
             QKV, ctx = buf(f"bert_qkv_{l}", M, 3 * H), buf(f"bert_ctx_{l}", M, H)
-            probs = buf(f"bert_probs_{l}", B, nh, S, S)
             ao, h1 = buf(f"bert_ao_{l}", M, H), buf(f"bert_h1_{l}", M, H)
             pre = buf(f"bert_pre_{l}", M, I)
             bf = eng.tc_kind == 1
@@ -361,20 +385,34 @@ class BertEngine:
                       Lp + "attention.output.dense.bias", H, H)
             qkv_names = [Lp + f"attention.self.{nm}.{wb}" for nm in ("query", "key", "value")
                          for wb in ("weight", "bias")]
-            sfx = self._att_sfx(S)
+            sfx = self._att_sfx(S, True)
+            mma = sfx.endswith("_mma")
             dQKV = buf("bert_dqkv", M, 3 * H)
-            if sfx:      # tensor-pipe core writes the bf16 operand copy of d(qkv) itself; the fp32
+            if sfx.startswith("_tiled"):
+                lse, delta = buf(f"bert_lse_{l}", B, nh, S), buf("bert_att_delta", B, nh, S)
+            else:
+                probs = buf(f"bert_probs_{l}", B, nh, S, S)
+            if mma:      # tensor-pipe core writes the bf16 operand copy of d(qkv) itself; the fp32
                          # tensor only where a bias column sum reads it
                 dq_bf = eng._prep_buf("bert_op3H_d", M, 3 * H, 1)[0]
                 need32 = any(n.endswith("bias") and n in train for n in qkv_names)
-                k._c("mmda_bert_attention_backward_mma", _ptr(QKV), _ptr(probs), _ptr(dctx),
-                     _ptr(dQKV) if need32 else None, _ptr(dq_bf), B, S, nh, 64, p_a, seed,
-                     _ptr(seed_dev), 201 + 4 * l)
+                if sfx == "_tiled_mma":
+                    k._c("mmda_bert_attention_backward_tiled_mma", _ptr(QKV), _ptr(mask), _ptr(ctx),
+                         _ptr(lse), _ptr(dctx), _ptr(delta), _ptr(dQKV) if need32 else None,
+                         _ptr(dq_bf), B, S, nh, 64, p_a, seed, _ptr(seed_dev), 201 + 4 * l)
+                else:
+                    k._c("mmda_bert_attention_backward_mma", _ptr(QKV), _ptr(probs), _ptr(dctx),
+                         _ptr(dQKV) if need32 else None, _ptr(dq_bf), B, S, nh, 64, p_a, seed,
+                         _ptr(seed_dev), 201 + 4 * l)
+            elif sfx == "_tiled":
+                k._c("mmda_bert_attention_backward_tiled", _ptr(QKV), _ptr(mask), _ptr(ctx), _ptr(lse),
+                     _ptr(dctx), _ptr(delta), _ptr(dQKV), B, S, nh, 64, p_a, seed, _ptr(seed_dev),
+                     201 + 4 * l)
             else:
                 k._c("mmda_bert_attention_backward", _ptr(QKV), _ptr(probs), _ptr(dctx), _ptr(dQKV), B, S,
                      nh, 64, p_a, seed, _ptr(seed_dev), 201 + 4 * l)
             if l > lowest or any(n in train for n in qkv_names):
-                dq_op = (dq_bf, None) if sfx else self._op("bert_op3H_d", dQKV)
+                dq_op = (dq_bf, None) if mma else self._op("bert_op3H_d", dQKV)
                 x_op = None
                 if l > lowest and bf:       # dx += d(qkv) [M x 3H] * [Wq; Wk; Wv]: one K = 3H GEMM
                     self._mm(0, 1, M, H, 3 * H, dq_op, self._wqkv(P, l)[0], dsum1, acc=True)

@@ -647,6 +647,661 @@ bert_attn_bwd_mma_kernel(const float* __restrict__ qkv, const float* __restrict_
   store_rows(dv, 2);
 }
 
+// ------------------------------------------------------------------------------------------
+// Tiled (flash-style) attention for the sequences the resident kernels above cannot hold (they
+// keep the whole S x S problem of a (sample, head) in shared memory: S <= 84 backward, S <= 116
+// forward).  One CTA per (sample, head, 64-row tile); the other operand streams through shared
+// memory in 64-row tiles.  The forward keeps an online softmax (running row max m and sum l) and,
+// in training, writes lse = m + log(l) per row; the backward recomputes P = exp(s*scale - lse)
+// tile by tile and uses D_i = sum_c dctx[i][c] ctx[i][c] (= rowsum(dPd o Pd), so dropout stays
+// exact).  Memory beyond inputs and outputs is O(S) per (sample, head): no S x S buffer exists.
+// dK / dV (one CTA per key tile) and dQ (one CTA per query tile) are separate kernels that both
+// recompute P (bf16 mode: D is a rowsum over the kernel's own products, see the dQ kernel):
+// every output element has one owner thread and a fixed summation order, so two
+// launches give identical bits without atomics.  Element (b, h, i, j) draws its dropout decision
+// at the same stream index as the resident kernels, so at S <= 84 either pair sees the same mask.
+// ------------------------------------------------------------------------------------------
+constexpr int TT = 64;           // query / key rows per tile
+constexpr int TP = TT + 4;       // pitch of the transposed probability tiles (fp32 kernels)
+
+__device__ __forceinline__ unsigned att_drop_idx(int bh, int S, int i, int j) {
+  return (unsigned)(((unsigned long long)bh * S + i) * S + j);     // < 2^32 checked at the ABI
+}
+
+// rows [r0, r0 + 64) x 64 features of a [token][ld] matrix -> k-major dst[c][s] (rows >= S zero)
+__device__ __forceinline__ void stage_t(float* dst, const float* src, int ld, int rows, int tid) {
+#pragma unroll 4
+  for (int idx = tid; idx < TT * (BHD / 4); idx += ATT_THREADS) {
+    const int s = idx % TT, c = (idx / TT) * 4;      // lanes over tokens: conflict-free transposes
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (s < rows) v = *reinterpret_cast<const float4*>(src + (size_t)s * ld + c);
+    dst[(c + 0) * TT + s] = v.x; dst[(c + 1) * TT + s] = v.y;
+    dst[(c + 2) * TT + s] = v.z; dst[(c + 3) * TT + s] = v.w;
+  }
+}
+// the same rows, row-major dst[s][c]
+__device__ __forceinline__ void stage_r(float* dst, const float* src, int ld, int rows, int tid) {
+#pragma unroll 4
+  for (int idx = tid; idx < TT * (BHD / 4); idx += ATT_THREADS) {
+    const int s = idx / (BHD / 4), c = (idx % (BHD / 4)) * 4;
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (s < rows) v = *reinterpret_cast<const float4*>(src + (size_t)s * ld + c);
+    *reinterpret_cast<float4*>(dst + s * BHD + c) = v;
+  }
+}
+
+// reduce over the 16 lanes that share a row block (xor butterfly: every lane gets the same bits)
+__device__ __forceinline__ float half_max(float v) {
+#pragma unroll
+  for (int o = 8; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
+  return v;
+}
+__device__ __forceinline__ float half_sum(float v) {
+#pragma unroll
+  for (int o = 8; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+
+// D[b][h][i] = sum_c dctx[b*S + i][h*64 + c] * ctx[b*S + i][h*64 + c]; one warp per (row, head)
+__global__ void __launch_bounds__(256)
+bert_attn_delta_kernel(const float* __restrict__ ctx, const float* __restrict__ dctx,
+                       float* __restrict__ delta, int B, int S, int nhead) {
+  const int w = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (w >= B * S * nhead) return;
+  const int m = w / nhead, h = w % nhead, b = m / S, i = m % S;
+  const size_t o = (size_t)m * nhead * BHD + h * BHD + lane * 2;
+  const float2 c = *reinterpret_cast<const float2*>(ctx + o);
+  const float2 d = *reinterpret_cast<const float2*>(dctx + o);
+  const float r = warp_sum(fmaf(c.x, d.x, c.y * d.y));
+  if (lane == 0) delta[((size_t)b * nhead + h) * S + i] = r;
+}
+
+// ---- fp32 (exact FFMA) ----------------------------------------------------------------------
+// Thread t owns the 4 x 4 block (rows 4 (t / 16), columns 4 (t % 16)) of every 64 x 64 product,
+// so the 16 lanes of a half warp hold complete row blocks and reduce rows with shuffles.
+constexpr int ATT_TILED_FWD_SMEM = (3 * TT * BHD + TT * TP) * 4;
+
+__global__ void __launch_bounds__(ATT_THREADS)
+bert_attn_fwd_tiled_kernel(const float* __restrict__ qkv, const long long* __restrict__ mask,
+                           float* __restrict__ ctx, float* __restrict__ lse, int S, int nhead,
+                           int nqt, float scale, float p_drop, unsigned long long seed,
+                           const unsigned long long* __restrict__ seed_dev, unsigned stream) {
+  extern __shared__ __align__(16) float sm[];
+  float* Qt = sm;                  // [64 dims][64 queries]
+  float* Kt = Qt + TT * BHD;       // [64 dims][64 keys]
+  float* Vs = Kt + TT * BHD;       // [64 keys][64 dims]
+  float* Pt = Vs + TT * BHD;       // [64 keys][TP] dropped, unnormalised probabilities
+  if (seed_dev) seed += seed_dev[0] * 0x9E3779B97F4A7C15ULL;
+  const int bh = blockIdx.x / nqt, r0 = (blockIdx.x % nqt) * TT;
+  const int b = bh / nhead, h = bh % nhead;
+  const int Hd = nhead * BHD, ld = 3 * Hd;
+  const int tid = threadIdx.x, i0 = (tid >> 4) * 4, x0 = (tid & 15) * 4;
+  const float* base = qkv + (size_t)b * S * ld + h * BHD;
+  stage_t(Qt, base + (size_t)r0 * ld, ld, S - r0, tid);
+  const float inv_keep = p_drop > 0.f ? 1.f / (1.f - p_drop) : 1.f;
+  float m[4], l[4], acc[4][4];
+#pragma unroll
+  for (int a = 0; a < 4; ++a) {
+    m[a] = -INFINITY; l[a] = 0.f;
+#pragma unroll
+    for (int c = 0; c < 4; ++c) acc[a][c] = 0.f;
+  }
+  for (int k0 = 0; k0 < S; k0 += TT) {
+    __syncthreads();               // previous tile's Kt / Vs / Pt fully consumed
+    stage_t(Kt, base + (size_t)k0 * ld + Hd, ld, S - k0, tid);
+    stage_r(Vs, base + (size_t)k0 * ld + 2 * Hd, ld, S - k0, tid);
+    __syncthreads();
+    float s[4][4];
+    mm_tile(Qt, TT, Kt, TT, BHD, i0, x0, s);
+    bool keep[4];      // HF adds finfo.min to masked keys: the softmax weight is exactly 0
+#pragma unroll
+    for (int c = 0; c < 4; ++c) keep[c] = k0 + x0 + c < S && mask[(size_t)b * S + k0 + x0 + c] != 0;
+    float alpha[4];
+#pragma unroll
+    for (int a = 0; a < 4; ++a) {
+      float mx = -INFINITY;
+#pragma unroll
+      for (int c = 0; c < 4; ++c) {
+        s[a][c] = keep[c] ? s[a][c] * scale : -INFINITY;
+        mx = fmaxf(mx, s[a][c]);
+      }
+      const float mn = fmaxf(m[a], half_max(mx));
+      const float mu = mn == -INFINITY ? 0.f : mn;      // no exp(-inf - -inf) while all are masked
+      alpha[a] = expf(m[a] - mu);
+      float rs = 0.f;
+#pragma unroll
+      for (int c = 0; c < 4; ++c) {
+        s[a][c] = expf(s[a][c] - mu);
+        rs += s[a][c];
+      }
+      l[a] = l[a] * alpha[a] + half_sum(rs);
+      m[a] = mn;
+    }
+#pragma unroll
+    for (int c = 0; c < 4; ++c) {
+      float pd[4];
+#pragma unroll
+      for (int a = 0; a < 4; ++a) {
+        const int i = r0 + i0 + a, j = k0 + x0 + c;
+        pd[a] = (i < S && j < S)
+            ? s[a][c] * drop_scale(seed, stream, att_drop_idx(bh, S, i, j), p_drop, inv_keep) : 0.f;
+      }
+      *reinterpret_cast<float4*>(Pt + (x0 + c) * TP + i0) = make_float4(pd[0], pd[1], pd[2], pd[3]);
+    }
+    __syncthreads();
+    float pv[4][4];
+    mm_tile(Pt, TP, Vs, BHD, TT, i0, x0, pv);
+#pragma unroll
+    for (int a = 0; a < 4; ++a)
+#pragma unroll
+      for (int c = 0; c < 4; ++c) acc[a][c] = fmaf(acc[a][c], alpha[a], pv[a][c]);
+  }
+#pragma unroll
+  for (int a = 0; a < 4; ++a) {
+    const int i = r0 + i0 + a;
+    if (i >= S) continue;
+    const float inv = 1.f / l[a];
+    *reinterpret_cast<float4*>(ctx + (size_t)(b * S + i) * Hd + h * BHD + x0) =
+        make_float4(acc[a][0] * inv, acc[a][1] * inv, acc[a][2] * inv, acc[a][3] * inv);
+    if (lse && x0 == 0) lse[(size_t)bh * S + i] = m[a] + logf(l[a]);
+  }
+}
+
+// dK, dV of one 64-key tile; the query sequence streams through.  P^T and dS^T blocks are
+// computed transposed (keys as rows) and stored [query][key] for the two accumulations.
+constexpr int ATT_TILED_DKV_SMEM = (6 * TT * BHD + 2 * TT * TP + 2 * TT) * 4;
+
+__global__ void __launch_bounds__(ATT_THREADS, 1)
+bert_attn_bwd_dkv_tiled_kernel(const float* __restrict__ qkv, const long long* __restrict__ mask,
+                               const float* __restrict__ lse, const float* __restrict__ dctx,
+                               const float* __restrict__ delta, float* __restrict__ dqkv, int S,
+                               int nhead, int nkt, float scale, float p_drop, unsigned long long seed,
+                               const unsigned long long* __restrict__ seed_dev, unsigned stream) {
+  extern __shared__ __align__(16) float sm[];
+  float* Kt = sm;                  // [64 dims][64 keys]
+  float* Vt = Kt + TT * BHD;       // [64 dims][64 keys]
+  float* Qt = Vt + TT * BHD;       // [64 dims][64 queries]
+  float* Ct = Qt + TT * BHD;       // d(ctx) [64 dims][64 queries]
+  float* Qs = Ct + TT * BHD;       // [64 queries][64 dims]
+  float* Cs = Qs + TT * BHD;       // d(ctx) [64 queries][64 dims]
+  float* Pd = Cs + TT * BHD;       // dropped probabilities [64 queries][TP keys]
+  float* Ds = Pd + TT * TP;        // d(scores) [64 queries][TP keys]
+  float* Ls = Ds + TT * TP;        // lse of the query tile
+  float* Dl = Ls + TT;             // D of the query tile
+  if (seed_dev) seed += seed_dev[0] * 0x9E3779B97F4A7C15ULL;
+  const int bh = blockIdx.x / nkt, k0 = (blockIdx.x % nkt) * TT;
+  const int b = bh / nhead, h = bh % nhead;
+  const int Hd = nhead * BHD, ld = 3 * Hd;
+  const int tid = threadIdx.x, j0 = (tid >> 4) * 4, x0 = (tid & 15) * 4;
+  const float* base = qkv + (size_t)b * S * ld + h * BHD;
+  const float* cbase = dctx + (size_t)b * S * Hd + h * BHD;
+  stage_t(Kt, base + (size_t)k0 * ld + Hd, ld, S - k0, tid);
+  stage_t(Vt, base + (size_t)k0 * ld + 2 * Hd, ld, S - k0, tid);
+  bool keep[4];
+#pragma unroll
+  for (int a = 0; a < 4; ++a) keep[a] = k0 + j0 + a < S && mask[(size_t)b * S + k0 + j0 + a] != 0;
+  const float inv_keep = p_drop > 0.f ? 1.f / (1.f - p_drop) : 1.f;
+  float dk[4][4], dv[4][4];
+#pragma unroll
+  for (int a = 0; a < 4; ++a)
+#pragma unroll
+    for (int c = 0; c < 4; ++c) dk[a][c] = dv[a][c] = 0.f;
+  for (int q0 = 0; q0 < S; q0 += TT) {
+    __syncthreads();
+    stage_t(Qt, base + (size_t)q0 * ld, ld, S - q0, tid);
+    stage_r(Qs, base + (size_t)q0 * ld, ld, S - q0, tid);
+    stage_t(Ct, cbase + (size_t)q0 * Hd, Hd, S - q0, tid);
+    stage_r(Cs, cbase + (size_t)q0 * Hd, Hd, S - q0, tid);
+    if (tid < TT) {
+      const bool in = q0 + tid < S;
+      Ls[tid] = in ? lse[(size_t)bh * S + q0 + tid] : 0.f;
+      Dl[tid] = in ? delta[(size_t)bh * S + q0 + tid] : 0.f;
+    }
+    __syncthreads();
+    float st[4][4], dpt[4][4];
+    mm_tile(Kt, TT, Qt, TT, BHD, j0, x0, st);      // s^T[j][i]
+    mm_tile(Vt, TT, Ct, TT, BHD, j0, x0, dpt);     // d(dropped P)^T[j][i]
+#pragma unroll
+    for (int c = 0; c < 4; ++c) {
+      const int i = q0 + x0 + c;
+      float pd[4], ds[4];
+#pragma unroll
+      for (int a = 0; a < 4; ++a) {
+        const int j = k0 + j0 + a;
+        pd[a] = ds[a] = 0.f;
+        if (keep[a] && i < S) {
+          const float p = expf(st[a][c] * scale - Ls[x0 + c]);
+          const float f = drop_scale(seed, stream, att_drop_idx(bh, S, i, j), p_drop, inv_keep);
+          pd[a] = p * f;
+          ds[a] = p * (dpt[a][c] * f - Dl[x0 + c]) * scale;
+        }
+      }
+      *reinterpret_cast<float4*>(Pd + (x0 + c) * TP + j0) = make_float4(pd[0], pd[1], pd[2], pd[3]);
+      *reinterpret_cast<float4*>(Ds + (x0 + c) * TP + j0) = make_float4(ds[0], ds[1], ds[2], ds[3]);
+    }
+    __syncthreads();
+    float t[4][4];
+    mm_tile(Pd, TP, Cs, BHD, TT, j0, x0, t);       // dV[j] += sum_i Pd[i][j] dC[i]
+#pragma unroll
+    for (int a = 0; a < 4; ++a)
+#pragma unroll
+      for (int c = 0; c < 4; ++c) dv[a][c] += t[a][c];
+    mm_tile(Ds, TP, Qs, BHD, TT, j0, x0, t);       // dK[j] += sum_i dS[i][j] Q[i]
+#pragma unroll
+    for (int a = 0; a < 4; ++a)
+#pragma unroll
+      for (int c = 0; c < 4; ++c) dk[a][c] += t[a][c];
+  }
+#pragma unroll
+  for (int a = 0; a < 4; ++a) {
+    const int j = k0 + j0 + a;
+    if (j >= S) continue;
+    float* o = dqkv + (size_t)(b * S + j) * ld + h * BHD + x0;
+    *reinterpret_cast<float4*>(o + Hd) = make_float4(dk[a][0], dk[a][1], dk[a][2], dk[a][3]);
+    *reinterpret_cast<float4*>(o + 2 * Hd) = make_float4(dv[a][0], dv[a][1], dv[a][2], dv[a][3]);
+  }
+}
+
+// dQ of one 64-query tile; the key sequence streams through.
+constexpr int ATT_TILED_DQ_SMEM = (5 * TT * BHD + TT * TP) * 4;
+
+__global__ void __launch_bounds__(ATT_THREADS)
+bert_attn_bwd_dq_tiled_kernel(const float* __restrict__ qkv, const long long* __restrict__ mask,
+                              const float* __restrict__ lse, const float* __restrict__ dctx,
+                              const float* __restrict__ delta, float* __restrict__ dqkv, int S,
+                              int nhead, int nqt, float scale, float p_drop, unsigned long long seed,
+                              const unsigned long long* __restrict__ seed_dev, unsigned stream) {
+  extern __shared__ __align__(16) float sm[];
+  float* Qt = sm;                  // [64 dims][64 queries]
+  float* Ct = Qt + TT * BHD;       // d(ctx) [64 dims][64 queries]
+  float* Kt = Ct + TT * BHD;       // [64 dims][64 keys]
+  float* Vt = Kt + TT * BHD;       // [64 dims][64 keys]
+  float* Ks = Vt + TT * BHD;       // [64 keys][64 dims]
+  float* Dt = Ks + TT * BHD;       // d(scores) [64 keys][TP queries]
+  if (seed_dev) seed += seed_dev[0] * 0x9E3779B97F4A7C15ULL;
+  const int bh = blockIdx.x / nqt, r0 = (blockIdx.x % nqt) * TT;
+  const int b = bh / nhead, h = bh % nhead;
+  const int Hd = nhead * BHD, ld = 3 * Hd;
+  const int tid = threadIdx.x, i0 = (tid >> 4) * 4, x0 = (tid & 15) * 4;
+  const float* base = qkv + (size_t)b * S * ld + h * BHD;
+  stage_t(Qt, base + (size_t)r0 * ld, ld, S - r0, tid);
+  stage_t(Ct, dctx + (size_t)(b * S + r0) * Hd + h * BHD, Hd, S - r0, tid);
+  float L[4], D[4];
+#pragma unroll
+  for (int a = 0; a < 4; ++a) {
+    const int i = r0 + i0 + a;
+    L[a] = i < S ? lse[(size_t)bh * S + i] : 0.f;
+    D[a] = i < S ? delta[(size_t)bh * S + i] : 0.f;
+  }
+  const float inv_keep = p_drop > 0.f ? 1.f / (1.f - p_drop) : 1.f;
+  float dq[4][4];
+#pragma unroll
+  for (int a = 0; a < 4; ++a)
+#pragma unroll
+    for (int c = 0; c < 4; ++c) dq[a][c] = 0.f;
+  for (int k0 = 0; k0 < S; k0 += TT) {
+    __syncthreads();
+    stage_t(Kt, base + (size_t)k0 * ld + Hd, ld, S - k0, tid);
+    stage_t(Vt, base + (size_t)k0 * ld + 2 * Hd, ld, S - k0, tid);
+    stage_r(Ks, base + (size_t)k0 * ld + Hd, ld, S - k0, tid);
+    __syncthreads();
+    float s[4][4], dp[4][4];
+    mm_tile(Qt, TT, Kt, TT, BHD, i0, x0, s);
+    mm_tile(Ct, TT, Vt, TT, BHD, i0, x0, dp);
+    bool keep[4];
+#pragma unroll
+    for (int c = 0; c < 4; ++c) keep[c] = k0 + x0 + c < S && mask[(size_t)b * S + k0 + x0 + c] != 0;
+#pragma unroll
+    for (int c = 0; c < 4; ++c) {
+      const int j = k0 + x0 + c;
+      float ds[4];
+#pragma unroll
+      for (int a = 0; a < 4; ++a) {
+        const int i = r0 + i0 + a;
+        ds[a] = 0.f;
+        if (keep[c] && i < S) {
+          const float p = expf(s[a][c] * scale - L[a]);
+          const float f = drop_scale(seed, stream, att_drop_idx(bh, S, i, j), p_drop, inv_keep);
+          ds[a] = p * (dp[a][c] * f - D[a]) * scale;
+        }
+      }
+      *reinterpret_cast<float4*>(Dt + (x0 + c) * TP + i0) = make_float4(ds[0], ds[1], ds[2], ds[3]);
+    }
+    __syncthreads();
+    float t[4][4];
+    mm_tile(Dt, TP, Ks, BHD, TT, i0, x0, t);       // dQ[i] += sum_j dS[i][j] K[j]
+#pragma unroll
+    for (int a = 0; a < 4; ++a)
+#pragma unroll
+      for (int c = 0; c < 4; ++c) dq[a][c] += t[a][c];
+  }
+#pragma unroll
+  for (int a = 0; a < 4; ++a) {
+    const int i = r0 + i0 + a;
+    if (i < S)
+      *reinterpret_cast<float4*>(dqkv + (size_t)(b * S + i) * ld + h * BHD + x0) =
+          make_float4(dq[a][0], dq[a][1], dq[a][2], dq[a][3]);
+  }
+}
+
+// ---- bf16 tensor pipe (mma.sync m16n8k16, fp32 accumulate) ----------------------------------
+// 4 warps, warp w owns rows 16 w .. 16 w + 15 of the CTA's 64-row tile; the streamed tiles are
+// double-buffered in shared memory (plain loads + convert), so one barrier per tile.  Fragment
+// layouts as in bert_attn_{fwd,bwd}_mma_kernel: this thread holds rows g and g + 8 of its warp's
+// 16, columns 8 n + 2 t4 + {0, 1} of each 8-column n-tile.
+__device__ __forceinline__ void keep_tile(float* dst, const long long* mask, int k0, int S, int tid) {
+  if (tid < TT) dst[tid] = (k0 + tid < S && mask[k0 + tid] != 0) ? 1.f : 0.f;
+}
+// acc[16 x 64] = A(smem X rows m0.., 64 wide) * Y^T (smem Y rows = the 64 n columns)
+__device__ __forceinline__ void mma_abt(float (&acc)[8][4], const __nv_bfloat16* X, int m0,
+                                        const __nv_bfloat16* Y, int lane) {
+  const int q = lane >> 3, r = lane & 7;
+#pragma unroll
+  for (int n = 0; n < 8; ++n) acc[n][0] = acc[n][1] = acc[n][2] = acc[n][3] = 0.f;
+#pragma unroll
+  for (int kt = 0; kt < 4; ++kt) {
+    uint32_t a[4];
+    ldsm_x4(a, &X[(m0 + (lane & 15)) * AP + kt * 16 + (lane >> 4) * 8]);
+#pragma unroll
+    for (int np = 0; np < 4; ++np) {
+      uint32_t bk[4];
+      ldsm_x4(bk, &Y[(np * 16 + (q >> 1) * 8 + r) * AP + kt * 16 + (q & 1) * 8]);
+      mma_bf16(acc[2 * np], a, bk[0], bk[1]);
+      mma_bf16(acc[2 * np + 1], a, bk[2], bk[3]);
+    }
+  }
+}
+// acc[16 x 64] += P (register fragments, 16 x 64) * Z (smem Z[k][n], 64 x 64)
+__device__ __forceinline__ void mma_pz(float (&acc)[8][4], const float (&p)[8][4],
+                                       const __nv_bfloat16* Z, int lane) {
+  const int q = lane >> 3, r = lane & 7;
+#pragma unroll
+  for (int kt = 0; kt < 4; ++kt) {
+    uint32_t a[4];
+    a[0] = pack_bf16(p[2 * kt][0], p[2 * kt][1]);
+    a[1] = pack_bf16(p[2 * kt][2], p[2 * kt][3]);
+    a[2] = pack_bf16(p[2 * kt + 1][0], p[2 * kt + 1][1]);
+    a[3] = pack_bf16(p[2 * kt + 1][2], p[2 * kt + 1][3]);
+#pragma unroll
+    for (int np = 0; np < 4; ++np) {
+      uint32_t bz[4];
+      ldsm_x4_t(bz, &Z[(kt * 16 + (q & 1) * 8 + r) * AP + np * 16 + (q >> 1) * 8]);
+      mma_bf16(acc[2 * np], a, bz[0], bz[1]);
+      mma_bf16(acc[2 * np + 1], a, bz[2], bz[3]);
+    }
+  }
+}
+// rows (i0, i1) of a [token][ld] output: fp32 and / or bf16 copy
+__device__ __forceinline__ void store_frag(const float (&v)[8][4], float* f32, __nv_bfloat16* b16,
+                                           size_t o0, size_t o1, bool ok0, bool ok1, int t4) {
+#pragma unroll
+  for (int n = 0; n < 8; ++n) {
+    const int c = n * 8 + t4 * 2;
+    if (ok0) {
+      if (f32) *reinterpret_cast<float2*>(f32 + o0 + c) = make_float2(v[n][0], v[n][1]);
+      if (b16) *reinterpret_cast<uint32_t*>(b16 + o0 + c) = pack_bf16(v[n][0], v[n][1]);
+    }
+    if (ok1) {
+      if (f32) *reinterpret_cast<float2*>(f32 + o1 + c) = make_float2(v[n][2], v[n][3]);
+      if (b16) *reinterpret_cast<uint32_t*>(b16 + o1 + c) = pack_bf16(v[n][2], v[n][3]);
+    }
+  }
+}
+
+constexpr int ATT_TILED_MMA_SMEM = 6 * TT * AP * 2 + 4 * TT * 4;
+
+__global__ void __launch_bounds__(128, 3)
+bert_attn_fwd_tiled_mma_kernel(const float* __restrict__ qkv, const long long* __restrict__ mask,
+                               float* __restrict__ ctx, __nv_bfloat16* __restrict__ ctx_bf16,
+                               float* __restrict__ lse, int S, int nhead, int nqt, float scale,
+                               float p_drop, unsigned long long seed,
+                               const unsigned long long* __restrict__ seed_dev, unsigned stream) {
+  __shared__ __align__(16) __nv_bfloat16 Qs[TT * AP], Ks[2][TT * AP], Vs[2][TT * AP];
+  __shared__ float keep_s[2][TT];
+  if (seed_dev) seed += seed_dev[0] * 0x9E3779B97F4A7C15ULL;
+  const int bh = blockIdx.x / nqt, r0 = (blockIdx.x % nqt) * TT;
+  const int b = bh / nhead, h = bh % nhead;
+  const int Hd = nhead * BHD, ld = 3 * Hd;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t4 = lane & 3;
+  const float* base = qkv + (size_t)b * S * ld + h * BHD;
+  const long long* mrow = mask + (size_t)b * S;
+  stage_bf16(Qs, base + (size_t)r0 * ld, ld, S - r0, tid);
+  stage_bf16(Ks[0], base + Hd, ld, S, tid);
+  stage_bf16(Vs[0], base + 2 * Hd, ld, S, tid);
+  keep_tile(keep_s[0], mrow, 0, S, tid);
+  __syncthreads();
+  const int m0 = warp * 16, i0 = r0 + m0 + g, i1 = i0 + 8;
+  const float inv_keep = p_drop > 0.f ? 1.f / (1.f - p_drop) : 1.f;
+  float o[8][4], sc[8][4];
+#pragma unroll
+  for (int n = 0; n < 8; ++n) o[n][0] = o[n][1] = o[n][2] = o[n][3] = 0.f;
+  float mr0 = -INFINITY, mr1 = -INFINITY, l0 = 0.f, l1 = 0.f;     // l: this thread's columns
+  const int nkt = (S + TT - 1) / TT;
+  for (int t = 0; t < nkt; ++t) {
+    const int cur = t & 1, k0 = t * TT;
+    if (t + 1 < nkt) {             // the other buffer was last read before the previous barrier
+      stage_bf16(Ks[cur ^ 1], base + (size_t)(k0 + TT) * ld + Hd, ld, S - k0 - TT, tid);
+      stage_bf16(Vs[cur ^ 1], base + (size_t)(k0 + TT) * ld + 2 * Hd, ld, S - k0 - TT, tid);
+      keep_tile(keep_s[cur ^ 1], mrow, k0 + TT, S, tid);
+    }
+    mma_abt(sc, Qs, m0, Ks[cur], lane);
+    float mx0 = -INFINITY, mx1 = -INFINITY;
+#pragma unroll
+    for (int n = 0; n < 8; ++n)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const float v = keep_s[cur][n * 8 + t4 * 2 + (e & 1)] != 0.f ? sc[n][e] * scale : -INFINITY;
+        sc[n][e] = v;
+        if (e < 2) mx0 = fmaxf(mx0, v); else mx1 = fmaxf(mx1, v);
+      }
+    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1));
+    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
+    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1));
+    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
+    const float mn0 = fmaxf(mr0, mx0), mn1 = fmaxf(mr1, mx1);
+    const float mu0 = mn0 == -INFINITY ? 0.f : mn0, mu1 = mn1 == -INFINITY ? 0.f : mn1;
+    const float al0 = expf(mr0 - mu0), al1 = expf(mr1 - mu1);
+    mr0 = mn0; mr1 = mn1;
+    float s0 = 0.f, s1 = 0.f;
+#pragma unroll
+    for (int n = 0; n < 8; ++n)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const int i = e < 2 ? i0 : i1, j = k0 + n * 8 + t4 * 2 + (e & 1);
+        const float ex = expf(sc[n][e] - (e < 2 ? mu0 : mu1));
+        if (e < 2) s0 += ex; else s1 += ex;
+        sc[n][e] = (i < S && j < S)
+            ? ex * drop_scale(seed, stream, att_drop_idx(bh, S, i, j), p_drop, inv_keep) : 0.f;
+      }
+    l0 = l0 * al0 + s0;
+    l1 = l1 * al1 + s1;
+#pragma unroll
+    for (int n = 0; n < 8; ++n) {
+      o[n][0] *= al0; o[n][1] *= al0; o[n][2] *= al1; o[n][3] *= al1;
+    }
+    mma_pz(o, sc, Vs[cur], lane);
+    __syncthreads();
+  }
+  l0 += __shfl_xor_sync(0xffffffffu, l0, 1);
+  l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
+  l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
+  l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
+  const float inv0 = 1.f / l0, inv1 = 1.f / l1;
+#pragma unroll
+  for (int n = 0; n < 8; ++n) {
+    o[n][0] *= inv0; o[n][1] *= inv0; o[n][2] *= inv1; o[n][3] *= inv1;
+  }
+  store_frag(o, ctx, ctx_bf16, (size_t)(b * S + i0) * Hd + h * BHD, (size_t)(b * S + i1) * Hd + h * BHD,
+             i0 < S, i1 < S, t4);
+  if (lse && t4 == 0) {
+    if (i0 < S) lse[(size_t)bh * S + i0] = mr0 + logf(l0);
+    if (i1 < S) lse[(size_t)bh * S + i1] = mr1 + logf(l1);
+  }
+}
+
+// dQ of one 64-query tile (keys streamed): dS = P (dPd f - D) scale stays in registers as the
+// A operand of dS K.  D_i = sum_j Pd[i][j] dPd[i][j] is computed here, in a first pass over the
+// keys, from the same bf16 products dS uses (as the resident _mma backward does): the identity
+// D_i = dctx[i] . ctx[i] holds only up to the bf16 rounding of dO, V and Pd, and where one key
+// carries the whole row (P = 1, e.g. a sample whose only valid key is [CLS]) that residue is all
+// dS would hold.  The kernel writes D to delta for the dK / dV kernel, which runs after it.
+__global__ void __launch_bounds__(128, 2)
+bert_attn_bwd_dq_tiled_mma_kernel(const float* __restrict__ qkv, const long long* __restrict__ mask,
+                                  const float* __restrict__ lse, const float* __restrict__ dctx,
+                                  float* __restrict__ delta, float* __restrict__ dqkv,
+                                  __nv_bfloat16* __restrict__ dqkv_bf16, int S, int nhead, int nqt,
+                                  float scale, float p_drop, unsigned long long seed,
+                                  const unsigned long long* __restrict__ seed_dev, unsigned stream) {
+  extern __shared__ __align__(16) unsigned char att_smem[];
+  __nv_bfloat16* Qs = reinterpret_cast<__nv_bfloat16*>(att_smem);
+  __nv_bfloat16* Cs = Qs + TT * AP;              // d(ctx)
+  __nv_bfloat16* Ks = Cs + TT * AP;              // [2][TT * AP]
+  __nv_bfloat16* Vs = Ks + 2 * TT * AP;          // [2][TT * AP]
+  float* keep_s = reinterpret_cast<float*>(Vs + 2 * TT * AP);     // [2][TT]
+  if (seed_dev) seed += seed_dev[0] * 0x9E3779B97F4A7C15ULL;
+  const int bh = blockIdx.x / nqt, r0 = (blockIdx.x % nqt) * TT;
+  const int b = bh / nhead, h = bh % nhead;
+  const int Hd = nhead * BHD, ld = 3 * Hd;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t4 = lane & 3;
+  const float* base = qkv + (size_t)b * S * ld + h * BHD;
+  const long long* mrow = mask + (size_t)b * S;
+  stage_bf16(Qs, base + (size_t)r0 * ld, ld, S - r0, tid);
+  stage_bf16(Cs, dctx + (size_t)(b * S + r0) * Hd + h * BHD, Hd, S - r0, tid);
+  stage_bf16(Ks, base + Hd, ld, S, tid);
+  stage_bf16(Vs, base + 2 * Hd, ld, S, tid);
+  keep_tile(keep_s, mrow, 0, S, tid);
+  const int m0 = warp * 16, i0 = r0 + m0 + g, i1 = i0 + 8;
+  const float L0 = i0 < S ? lse[(size_t)bh * S + i0] : 0.f, L1 = i1 < S ? lse[(size_t)bh * S + i1] : 0.f;
+  __syncthreads();
+  const float inv_keep = p_drop > 0.f ? 1.f / (1.f - p_drop) : 1.f;
+  float dq[8][4], sc[8][4], dp[8][4];
+#pragma unroll
+  for (int n = 0; n < 8; ++n) dq[n][0] = dq[n][1] = dq[n][2] = dq[n][3] = 0.f;
+  float D0 = 0.f, D1 = 0.f;
+  const int nkt = (S + TT - 1) / TT;
+  for (int t = 0; t < 2 * nkt; ++t) {            // pass 0 (t < nkt): D; pass 1: dS, dQ
+    const int cur = t & 1, tn = t + 1, k0 = (t % nkt) * TT;
+    if (tn < 2 * nkt) {
+      const int kn = (tn % nkt) * TT;
+      stage_bf16(Ks + (cur ^ 1) * TT * AP, base + (size_t)kn * ld + Hd, ld, S - kn, tid);
+      stage_bf16(Vs + (cur ^ 1) * TT * AP, base + (size_t)kn * ld + 2 * Hd, ld, S - kn, tid);
+      keep_tile(keep_s + (cur ^ 1) * TT, mrow, kn, S, tid);
+    }
+    mma_abt(sc, Qs, m0, Ks + cur * TT * AP, lane);
+    mma_abt(dp, Cs, m0, Vs + cur * TT * AP, lane);
+    const bool pass1 = t >= nkt;
+#pragma unroll
+    for (int n = 0; n < 8; ++n)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const int jl = n * 8 + t4 * 2 + (e & 1), i = e < 2 ? i0 : i1, j = k0 + jl;
+        float ds = 0.f;
+        if (keep_s[cur * TT + jl] != 0.f && i < S) {
+          const float p = expf(sc[n][e] * scale - (e < 2 ? L0 : L1));
+          const float f = drop_scale(seed, stream, att_drop_idx(bh, S, i, j), p_drop, inv_keep);
+          const float d = dp[n][e] * f;
+          if (!pass1) {
+            if (e < 2) D0 = fmaf(d, p, D0); else D1 = fmaf(d, p, D1);
+          }
+          ds = p * (d - (e < 2 ? D0 : D1)) * scale;
+        }
+        sc[n][e] = ds;
+      }
+    if (t == nkt - 1) {
+      D0 += __shfl_xor_sync(0xffffffffu, D0, 1);
+      D0 += __shfl_xor_sync(0xffffffffu, D0, 2);
+      D1 += __shfl_xor_sync(0xffffffffu, D1, 1);
+      D1 += __shfl_xor_sync(0xffffffffu, D1, 2);
+      if (t4 == 0) {
+        if (i0 < S) delta[(size_t)bh * S + i0] = D0;
+        if (i1 < S) delta[(size_t)bh * S + i1] = D1;
+      }
+    }
+    if (pass1) mma_pz(dq, sc, Ks + cur * TT * AP, lane);
+    __syncthreads();
+  }
+  store_frag(dq, dqkv, dqkv_bf16, (size_t)(b * S + i0) * ld + h * BHD, (size_t)(b * S + i1) * ld + h * BHD,
+             i0 < S, i1 < S, t4);
+}
+
+// dK, dV of one 64-key tile (queries streamed): the warp computes s^T and dPd^T with its 16 key
+// rows as the M dimension, so Pd^T and dS^T come out as A fragments of dV += Pd^T dO and
+// dK += dS^T Q without a trip through shared memory.
+__global__ void __launch_bounds__(128)
+bert_attn_bwd_dkv_tiled_mma_kernel(const float* __restrict__ qkv, const long long* __restrict__ mask,
+                                   const float* __restrict__ lse, const float* __restrict__ dctx,
+                                   const float* __restrict__ delta, float* __restrict__ dqkv,
+                                   __nv_bfloat16* __restrict__ dqkv_bf16, int S, int nhead, int nkt,
+                                   float scale, float p_drop, unsigned long long seed,
+                                   const unsigned long long* __restrict__ seed_dev, unsigned stream) {
+  extern __shared__ __align__(16) unsigned char att_smem[];
+  __nv_bfloat16* Ks = reinterpret_cast<__nv_bfloat16*>(att_smem);
+  __nv_bfloat16* Vs = Ks + TT * AP;
+  __nv_bfloat16* Qs = Vs + TT * AP;              // [2][TT * AP]
+  __nv_bfloat16* Cs = Qs + 2 * TT * AP;          // d(ctx) [2][TT * AP]
+  float* Ls = reinterpret_cast<float*>(Cs + 2 * TT * AP);     // [2][TT] lse of the query tile
+  float* Dl = Ls + 2 * TT;                                    // [2][TT] D of the query tile
+  if (seed_dev) seed += seed_dev[0] * 0x9E3779B97F4A7C15ULL;
+  const int bh = blockIdx.x / nkt, k0 = (blockIdx.x % nkt) * TT;
+  const int b = bh / nhead, h = bh % nhead;
+  const int Hd = nhead * BHD, ld = 3 * Hd;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t4 = lane & 3;
+  const float* base = qkv + (size_t)b * S * ld + h * BHD;
+  const float* cbase = dctx + (size_t)b * S * Hd + h * BHD;
+  auto stage_q = [&](int q0, int buf) {
+    stage_bf16(Qs + buf * TT * AP, base + (size_t)q0 * ld, ld, S - q0, tid);
+    stage_bf16(Cs + buf * TT * AP, cbase + (size_t)q0 * Hd, Hd, S - q0, tid);
+    if (tid < TT) {
+      const bool in = q0 + tid < S;
+      Ls[buf * TT + tid] = in ? lse[(size_t)bh * S + q0 + tid] : 0.f;
+      Dl[buf * TT + tid] = in ? delta[(size_t)bh * S + q0 + tid] : 0.f;
+    }
+  };
+  stage_bf16(Ks, base + (size_t)k0 * ld + Hd, ld, S - k0, tid);
+  stage_bf16(Vs, base + (size_t)k0 * ld + 2 * Hd, ld, S - k0, tid);
+  stage_q(0, 0);
+  const int m0 = warp * 16, j0 = k0 + m0 + g, j1 = j0 + 8;
+  const bool kp0 = j0 < S && mask[(size_t)b * S + j0] != 0, kp1 = j1 < S && mask[(size_t)b * S + j1] != 0;
+  __syncthreads();
+  const float inv_keep = p_drop > 0.f ? 1.f / (1.f - p_drop) : 1.f;
+  float dk[8][4], dv[8][4], st[8][4], dpt[8][4];
+#pragma unroll
+  for (int n = 0; n < 8; ++n) {
+    dk[n][0] = dk[n][1] = dk[n][2] = dk[n][3] = 0.f;
+    dv[n][0] = dv[n][1] = dv[n][2] = dv[n][3] = 0.f;
+  }
+  const int nqt = (S + TT - 1) / TT;
+  for (int t = 0; t < nqt; ++t) {
+    const int cur = t & 1, q0 = t * TT;
+    if (t + 1 < nqt) stage_q(q0 + TT, cur ^ 1);
+    const __nv_bfloat16* Qc = Qs + cur * TT * AP;
+    const __nv_bfloat16* Cc = Cs + cur * TT * AP;
+    mma_abt(st, Ks, m0, Qc, lane);               // s^T[j][i]
+    mma_abt(dpt, Vs, m0, Cc, lane);              // dPd^T[j][i]
+#pragma unroll
+    for (int n = 0; n < 8; ++n)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const int il = n * 8 + t4 * 2 + (e & 1), i = q0 + il, j = e < 2 ? j0 : j1;
+        float pd = 0.f, ds = 0.f;
+        if ((e < 2 ? kp0 : kp1) && i < S) {
+          const float p = expf(st[n][e] * scale - Ls[cur * TT + il]);
+          const float f = drop_scale(seed, stream, att_drop_idx(bh, S, i, j), p_drop, inv_keep);
+          pd = p * f;
+          ds = p * (dpt[n][e] * f - Dl[cur * TT + il]) * scale;
+        }
+        st[n][e] = pd;
+        dpt[n][e] = ds;
+      }
+    mma_pz(dv, st, Cc, lane);
+    mma_pz(dk, dpt, Qc, lane);
+    __syncthreads();
+  }
+  const size_t o0 = (size_t)(b * S + j0) * ld + h * BHD, o1 = (size_t)(b * S + j1) * ld + h * BHD;
+  store_frag(dk, dqkv, dqkv_bf16, o0 + Hd, o1 + Hd, j0 < S, j1 < S, t4);
+  store_frag(dv, dqkv, dqkv_bf16, o0 + 2 * Hd, o1 + 2 * Hd, j0 < S, j1 < S, t4);
+}
+
 static inline int ew_grid_b(size_t n) {
   size_t g = (n + 255) / 256;
   return (int)(g > 148 * 16 ? 148 * 16 : (g == 0 ? 1 : g));
@@ -717,13 +1372,34 @@ static int bert_attn_smem(int S, bool bwd) {
   return (int)(((bwd ? 5 : 3) * S4 * BHD + (bwd ? 3 : 2) * S4 * S4) * sizeof(float));
 }
 
+constexpr int ATT_RESIDENT_SMEM = 200 * 1024;
+
+int mmda_bert_attention_resident_max_seq(int backward) {
+  int S = 0;
+  while (bert_attn_smem(S + 1, backward != 0) <= ATT_RESIDENT_SMEM) ++S;
+  return S;
+}
+
+// shared argument checks of the tiled attention entry points
+static int tiled_args(const char* who, const float* qkv, const long long* mask, int B, int S,
+                      int nhead, int head_dim) {
+  MMDA_REQUIRE(head_dim == BHD, "%s: head_dim %d (bert-base uses 64)", who, head_dim);
+  MMDA_REQUIRE(B > 0 && S > 0 && nhead > 0, "%s: bad sizes B=%d S=%d nhead=%d", who, B, S, nhead);
+  MMDA_REQUIRE((unsigned long long)B * nhead * S * S < (1ULL << 32),
+               "%s: B*nhead*S*S = %llu dropout elements exceed the 32-bit dropout index", who,
+               (unsigned long long)B * nhead * S * S);
+  MMDA_REQUIRE(qkv != nullptr && mask != nullptr, "%s: qkv and mask are required", who);
+  MMDA_REQUIRE((reinterpret_cast<uintptr_t>(qkv) & 15) == 0, "%s: unaligned operands", who);
+  return MMDA_OK;
+}
+
 int mmda_bert_attention_forward(const float* qkv, const long long* mask, float* ctx, float* probs,
                                 int B, int S, int nhead, int head_dim, float p_drop,
                                 unsigned long long seed, const unsigned long long* seed_dev,
                                 unsigned stream_id, cudaStream_t stream) {
   MMDA_REQUIRE(head_dim == BHD, "bert_attention: head_dim %d (bert-base uses 64)", head_dim);
   const int smem = bert_attn_smem(S, false);
-  MMDA_REQUIRE(B > 0 && S > 0 && smem <= 200 * 1024,
+  MMDA_REQUIRE(B > 0 && S > 0 && smem <= ATT_RESIDENT_SMEM,
                "bert_attention: sequence %d does not fit the shared-memory resident kernel", S);
   MMDA_CUDA(cudaFuncSetAttribute(bert_attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   bert_attn_fwd_kernel<<<B * nhead, ATT_THREADS, smem, stream>>>(qkv, mask, ctx, probs, S, nhead,
@@ -739,7 +1415,7 @@ int mmda_bert_attention_backward(const float* qkv, const float* probs, const flo
                                  unsigned stream_id, cudaStream_t stream) {
   MMDA_REQUIRE(head_dim == BHD, "bert_attention: head_dim %d (bert-base uses 64)", head_dim);
   const int smem = bert_attn_smem(S, true);
-  MMDA_REQUIRE(B > 0 && S > 0 && smem <= 200 * 1024,
+  MMDA_REQUIRE(B > 0 && S > 0 && smem <= ATT_RESIDENT_SMEM,
                "bert_attention: sequence %d does not fit the shared-memory resident kernel", S);
   MMDA_CUDA(cudaFuncSetAttribute(bert_attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   bert_attn_bwd_kernel<<<B * nhead, ATT_THREADS, smem, stream>>>(qkv, probs, dctx, dqkv, S, nhead,
@@ -783,6 +1459,116 @@ int mmda_bert_attention_backward_mma(const float* qkv, const float* probs, const
   bert_attn_bwd_mma_kernel<<<B * nhead, 128, ATT_MMA_BWD_SMEM, stream>>>(
       qkv, probs, dctx, dqkv, reinterpret_cast<__nv_bfloat16*>(dqkv_bf16), S, nhead,
       1.0f / sqrtf((float)head_dim), p_drop, seed, seed_dev, stream_id);
+  MMDA_CHECK_LAUNCH();
+  return MMDA_OK;
+}
+
+// Tiled variants (any S): lse [B][nhead][S] replaces probs; lse == NULL means eval.
+int mmda_bert_attention_forward_tiled(const float* qkv, const long long* mask, float* ctx, float* lse,
+                                      int B, int S, int nhead, int head_dim, float p_drop,
+                                      unsigned long long seed, const unsigned long long* seed_dev,
+                                      unsigned stream_id, cudaStream_t stream) {
+  const int rc = tiled_args("bert_attention_tiled", qkv, mask, B, S, nhead, head_dim);
+  if (rc != MMDA_OK) return rc;
+  MMDA_REQUIRE(ctx != nullptr, "bert_attention_tiled: no output");
+  MMDA_REQUIRE((reinterpret_cast<uintptr_t>(ctx) & 15) == 0 && (reinterpret_cast<uintptr_t>(lse) & 3) == 0,
+               "bert_attention_tiled: unaligned operands");
+  const int nqt = (S + TT - 1) / TT;
+  MMDA_CUDA(cudaFuncSetAttribute(bert_attn_fwd_tiled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 ATT_TILED_FWD_SMEM));
+  bert_attn_fwd_tiled_kernel<<<B * nhead * nqt, ATT_THREADS, ATT_TILED_FWD_SMEM, stream>>>(
+      qkv, mask, ctx, lse, S, nhead, nqt, 1.0f / sqrtf((float)head_dim), p_drop, seed, seed_dev, stream_id);
+  MMDA_CHECK_LAUNCH();
+  return MMDA_OK;
+}
+
+static int launch_delta(const float* ctx, const float* dctx, float* delta, int B, int S, int nhead,
+                        cudaStream_t stream) {
+  const long long warps = (long long)B * S * nhead;
+  bert_attn_delta_kernel<<<(unsigned)((warps + 7) / 8), 256, 0, stream>>>(ctx, dctx, delta, B, S, nhead);
+  MMDA_CHECK_LAUNCH();
+  return MMDA_OK;
+}
+
+int mmda_bert_attention_backward_tiled(const float* qkv, const long long* mask, const float* ctx,
+                                       const float* lse, const float* dctx, float* delta, float* dqkv,
+                                       int B, int S, int nhead, int head_dim, float p_drop,
+                                       unsigned long long seed, const unsigned long long* seed_dev,
+                                       unsigned stream_id, cudaStream_t stream) {
+  const int rc = tiled_args("bert_attention_backward_tiled", qkv, mask, B, S, nhead, head_dim);
+  if (rc != MMDA_OK) return rc;
+  MMDA_REQUIRE(ctx != nullptr && lse != nullptr && dctx != nullptr && delta != nullptr,
+               "bert_attention_backward_tiled: ctx, lse, dctx and delta are required");
+  MMDA_REQUIRE(dqkv != nullptr, "bert_attention_backward_tiled: no output");
+  MMDA_REQUIRE(((reinterpret_cast<uintptr_t>(ctx) | reinterpret_cast<uintptr_t>(dctx) |
+                 reinterpret_cast<uintptr_t>(dqkv)) & 15) == 0 &&
+               ((reinterpret_cast<uintptr_t>(lse) | reinterpret_cast<uintptr_t>(delta)) & 3) == 0,
+               "bert_attention_backward_tiled: unaligned operands");
+  const int nt = (S + TT - 1) / TT;
+  const float scale = 1.0f / sqrtf((float)head_dim);
+  const int drc = launch_delta(ctx, dctx, delta, B, S, nhead, stream);
+  if (drc != MMDA_OK) return drc;
+  MMDA_CUDA(cudaFuncSetAttribute(bert_attn_bwd_dkv_tiled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 ATT_TILED_DKV_SMEM));
+  bert_attn_bwd_dkv_tiled_kernel<<<B * nhead * nt, ATT_THREADS, ATT_TILED_DKV_SMEM, stream>>>(
+      qkv, mask, lse, dctx, delta, dqkv, S, nhead, nt, scale, p_drop, seed, seed_dev, stream_id);
+  MMDA_CHECK_LAUNCH();
+  MMDA_CUDA(cudaFuncSetAttribute(bert_attn_bwd_dq_tiled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 ATT_TILED_DQ_SMEM));
+  bert_attn_bwd_dq_tiled_kernel<<<B * nhead * nt, ATT_THREADS, ATT_TILED_DQ_SMEM, stream>>>(
+      qkv, mask, lse, dctx, delta, dqkv, S, nhead, nt, scale, p_drop, seed, seed_dev, stream_id);
+  MMDA_CHECK_LAUNCH();
+  return MMDA_OK;
+}
+
+int mmda_bert_attention_forward_tiled_mma(const float* qkv, const long long* mask, float* ctx,
+                                          void* ctx_bf16, float* lse, int B, int S, int nhead,
+                                          int head_dim, float p_drop, unsigned long long seed,
+                                          const unsigned long long* seed_dev, unsigned stream_id,
+                                          cudaStream_t stream) {
+  const int rc = tiled_args("bert_attention_tiled_mma", qkv, mask, B, S, nhead, head_dim);
+  if (rc != MMDA_OK) return rc;
+  MMDA_REQUIRE(ctx != nullptr || ctx_bf16 != nullptr, "bert_attention_tiled_mma: no output");
+  MMDA_REQUIRE((reinterpret_cast<uintptr_t>(ctx) & 7) == 0 && (reinterpret_cast<uintptr_t>(ctx_bf16) & 3) == 0 &&
+               (reinterpret_cast<uintptr_t>(lse) & 3) == 0,
+               "bert_attention_tiled_mma: unaligned operands");
+  const int nqt = (S + TT - 1) / TT;
+  bert_attn_fwd_tiled_mma_kernel<<<B * nhead * nqt, 128, 0, stream>>>(
+      qkv, mask, ctx, reinterpret_cast<__nv_bfloat16*>(ctx_bf16), lse, S, nhead, nqt,
+      1.0f / sqrtf((float)head_dim), p_drop, seed, seed_dev, stream_id);
+  MMDA_CHECK_LAUNCH();
+  return MMDA_OK;
+}
+
+int mmda_bert_attention_backward_tiled_mma(const float* qkv, const long long* mask, const float* ctx,
+                                           const float* lse, const float* dctx, float* delta,
+                                           float* dqkv, void* dqkv_bf16, int B, int S, int nhead,
+                                           int head_dim, float p_drop, unsigned long long seed,
+                                           const unsigned long long* seed_dev, unsigned stream_id,
+                                           cudaStream_t stream) {
+  const int rc = tiled_args("bert_attention_backward_tiled_mma", qkv, mask, B, S, nhead, head_dim);
+  if (rc != MMDA_OK) return rc;
+  (void)ctx;         // D comes from the kernel's own bf16 products (see the dQ kernel)
+  MMDA_REQUIRE(lse != nullptr && dctx != nullptr && delta != nullptr,
+               "bert_attention_backward_tiled_mma: lse, dctx and delta are required");
+  MMDA_REQUIRE(dqkv != nullptr || dqkv_bf16 != nullptr, "bert_attention_backward_tiled_mma: no output");
+  MMDA_REQUIRE((reinterpret_cast<uintptr_t>(dctx) & 15) == 0 &&
+               (reinterpret_cast<uintptr_t>(dqkv) & 7) == 0 && (reinterpret_cast<uintptr_t>(dqkv_bf16) & 3) == 0 &&
+               ((reinterpret_cast<uintptr_t>(lse) | reinterpret_cast<uintptr_t>(delta)) & 3) == 0,
+               "bert_attention_backward_tiled_mma: unaligned operands");
+  const int nt = (S + TT - 1) / TT;
+  const float scale = 1.0f / sqrtf((float)head_dim);
+  __nv_bfloat16* dbf = reinterpret_cast<__nv_bfloat16*>(dqkv_bf16);
+  // the dQ kernel computes D from its bf16 products and writes delta; dK / dV read it
+  MMDA_CUDA(cudaFuncSetAttribute(bert_attn_bwd_dq_tiled_mma_kernel,
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, ATT_TILED_MMA_SMEM));
+  bert_attn_bwd_dq_tiled_mma_kernel<<<B * nhead * nt, 128, ATT_TILED_MMA_SMEM, stream>>>(
+      qkv, mask, lse, dctx, delta, dqkv, dbf, S, nhead, nt, scale, p_drop, seed, seed_dev, stream_id);
+  MMDA_CHECK_LAUNCH();
+  MMDA_CUDA(cudaFuncSetAttribute(bert_attn_bwd_dkv_tiled_mma_kernel,
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, ATT_TILED_MMA_SMEM));
+  bert_attn_bwd_dkv_tiled_mma_kernel<<<B * nhead * nt, 128, ATT_TILED_MMA_SMEM, stream>>>(
+      qkv, mask, lse, dctx, delta, dqkv, dbf, S, nhead, nt, scale, p_drop, seed, seed_dev, stream_id);
   MMDA_CHECK_LAUNCH();
   return MMDA_OK;
 }

@@ -37,7 +37,8 @@ def metrics_from_stats(stats, num_classes: int) -> Dict[str, float]:
 @torch.no_grad()
 def evaluate(model, batches: Iterable, device=None) -> Dict[str, float]:
     """batches yield objects with ``sentences, visual, acoustic, lengths, labels`` (host or device
-    tensors; ``lengths`` on the CPU)."""
+    tensors; ``lengths`` on the CPU), and with ``use_bert=True`` also ``bert_sent,
+    bert_sent_type, bert_sent_mask``."""
     was_training = model.training
     model.eval()
     eng = model.engine
@@ -46,8 +47,12 @@ def evaluate(model, batches: Iterable, device=None) -> Dict[str, float]:
     stats = torch.zeros(4 + 3 * NC, dtype=torch.float32, device=dev)
     to = lambda t: t.to(dev, non_blocking=True)
     for b in batches:
+        utt_text = None
+        if eng.use_bert:     # text branch: the BERT encoder's masked mean, no dropout
+            utt_text = eng.bert.forward(to(b.bert_sent), to(b.bert_sent_type), to(b.bert_sent_mask),
+                                        train=False, drop=False, seed=0)
         out = eng.forward(to(b.sentences), to(b.visual), to(b.acoustic), b.lengths, train=False,
-                          want_sp=False, dropout=False)
+                          want_sp=False, dropout=False, utt_text=utt_text)
         y = to(b.labels).float().contiguous()
         eng.k._c("mmda_eval_accumulate", _ptr(out["scores"]), _ptr(out["labels"]), _ptr(y),
                  _ptr(stats), y.shape[0], NC)
