@@ -49,9 +49,19 @@ loss_phase1_kernel(const float* __restrict__ X0, const float* __restrict__ O,
   float* cls = segA + NTOK * d;
   if (!(roles & (blk < NTOK ? 1 : 2))) return;      // block-uniform
   if (blk < NTOK) {
+    // Compensated (Kahan) sum over the batch.  The CMD coefficients divide differences of these
+    // column means by the norms of those differences, which magnifies the rounding of a plain
+    // serial sum (it grows like sqrt(B)) by 1 / |mean difference|.  With a plain sum, dZ was
+    // 2.7e-5 off fp64 at B = 1000 (1e-4 at B = 4096), and up to 15x further off than an fp32
+    // evaluation of the same formulas when the shared tokens' means nearly agree.
     for (int c = tid; c < d; c += 256) {
-      float s = 0.f;
-      for (int b = 0; b < B; ++b) s += X0[((size_t)b * NTOK + blk) * d + c];
+      float s = 0.f, comp = 0.f;
+      for (int b = 0; b < B; ++b) {
+        const float v = X0[((size_t)b * NTOK + blk) * d + c] - comp;
+        const float t = s + v;
+        comp = (t - s) - v;
+        s = t;
+      }
       colsum[blk * d + c] = s;
     }
   } else if (blk == NTOK) {
@@ -290,7 +300,9 @@ __global__ void loss_phase4b_kernel(const float* __restrict__ X0, const float* _
   const float* moments = segB;
   for (int c = lane; c < d; c += 32) {
     float g = DXN[((size_t)i * B + b) * d + c] - colsum2[i * d + c] / Bg;
-    if (i >= 3) {
+    // w_sim = 0 (the adversarial variant) skips the CMD term rather than scaling it by 0: its
+    // coefficients are 0/0 wherever two shared tokens' moments coincide, e.g. at B = 1
+    if (i >= 3 && w_sim != 0.f) {
       const int a = i - 3;
       const float xc = X0[(size_t)row * d + c] - segA[i * d + c] / Bg;
       float t = coef[(a * 5 + 0) * d + c];
@@ -414,6 +426,7 @@ int mmda_loss_finalize(const float* segA, const float* segB, float* losses, floa
 
 int mmda_loss_phase4a(float* DXN, const float* inv_norm, float* colsum2, int B, int d,
                       cudaStream_t stream) {
+  MMDA_REQUIRE(d >= 1 && d <= 32 * LOSS_MAXC, "loss: hidden_size=%d (max %d)", d, 32 * LOSS_MAXC);
   int rpb = (B + 23) / 24;
   rpb = (rpb + 7) / 8 * 8;
   dim3 grid(NTOK, (B + rpb - 1) / rpb);

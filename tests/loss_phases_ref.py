@@ -8,9 +8,22 @@ PAIRS = ((0, 3), (1, 4), (2, 5), (2, 0), (2, 1), (0, 1))
 CMD_PAIRS = ((0, 1), (0, 2), (2, 1))
 
 
-def phased_loss(X0, O, R, scores, tcp, y, Bg, w, reduce=lambda t: t):
+def domain_loss(DL, Bg, w_sim):
+    """Adversarial similarity term (mmda_loss_domain): cross-entropy of the 3B domain logits DL
+    (3B,3), rows [pred_t; pred_v; pred_a] with labels 0/1/2.  Returns (batch sum of the row
+    losses, d(w_sim * sum / (3 Bg)) / d DL)."""
+    B3 = DL.shape[0]
+    lab = torch.arange(3, device=DL.device).repeat_interleave(B3 // 3)
+    logp = torch.log_softmax(DL, dim=1)
+    onehot = torch.nn.functional.one_hot(lab, 3).to(DL.dtype)
+    return -(logp * onehot).sum(), w_sim / (3 * Bg) * (logp.exp() - onehot)
+
+
+def phased_loss(X0, O, R, scores, tcp, y, Bg, w, reduce=lambda t: t, DL=None, intermediates=False):
     """X0 (B,6,d) [p_t,p_v,p_a,s_t,s_v,s_a]; O,R (3,B,d); scores,tcp,y (B,NC).
-    w = dict(diff, sim, recon, conf).  Returns (losses dict, grads dict)."""
+    w = dict(diff, sim, recon, conf).  DL (3B,3): the domain logits of the adversarial variant
+    (use_cmd_sim=False): sim is then their cross-entropy and the CMD gradient is off.  Returns
+    (losses dict, grads dict), plus a dict of the phases' intermediates with intermediates=True."""
     B, _, d = X0.shape
     # phase 1
     segA = dict(colsum=X0.sum(0),
@@ -18,6 +31,8 @@ def phased_loss(X0, O, R, scores, tcp, y, Bg, w, reduce=lambda t: t):
                 sq=((tcp - y * scores) ** 2).sum(0), sys=(y * scores).sum(0), sy=y.sum(0),
                 nnz=(y != 0).to(X0.dtype).sum(0), se=torch.exp(scores).sum(0),
                 rsq=((R - O) ** 2).sum((1, 2)))
+    if DL is not None:
+        segA["dom"], d_domain = domain_loss(DL, Bg, w["sim"])
     segA = {k: reduce(v) for k, v in segA.items()}
     mu = segA["colsum"] / Bg                                   # (6,d)
     # phase 2
@@ -40,6 +55,8 @@ def phased_loss(X0, O, R, scores, tcp, y, Bg, w, reduce=lambda t: t):
             coef[a, k] += dl / nrm
             coef[b, k] -= dl / nrm
     cmd = cmd / 3
+    if DL is not None:
+        cmd = segA["dom"] / (3 * Bg)
     cls = (segA["bce"] / Bg).sum()
     recon = segA["rsq"].sum() / (Bg * d) / 3
     conf = ((segA["sq"] / Bg) / segA["nnz"] + (-segA["sys"] + segA["sy"] * torch.log(segA["se"])) / segA["nnz"]).sum()
@@ -54,11 +71,11 @@ def phased_loss(X0, O, R, scores, tcp, y, Bg, w, reduce=lambda t: t):
     dxc = DXN * inv.unsqueeze(2)
     colsum2 = reduce(dxc.sum(0))
     dZ = dxc - colsum2 / Bg
-    # cmd backward
-    for a in range(3):
+    # cmd backward (the adversarial variant has none: at B = 1 its coefficients are 0/0)
+    for a in range(3 if DL is None else 0):
         x = xc[:, 3 + a]
         t = coef[a, 0].expand_as(x).clone()
-        cprev = torch.zeros(d, dtype=X0.dtype)
+        cprev = X0.new_zeros(d)
         for k in range(2, 6):
             t = t + coef[a, k - 1] * k * (x ** (k - 1) - cprev)
             cprev = M[a, k - 2] / Bg
@@ -71,4 +88,10 @@ def phased_loss(X0, O, R, scores, tcp, y, Bg, w, reduce=lambda t: t):
         nnz = segA["nnz"]
         dt = w["conf"] * 2 * (tcp - y * scores) / (Bg * nnz)
         ds = ds - y * dt + w["conf"] * (-y + segA["sy"] * torch.exp(scores) / segA["se"]) / nnz
-    return L, dict(d_tokens=dZ, d_recon=dR, d_orig=-dR, d_scores=ds, d_tcp=dt)
+    grads = dict(d_tokens=dZ, d_recon=dR, d_orig=-dR, d_scores=ds, d_tcp=dt)
+    if DL is not None:
+        grads["d_domain"] = d_domain
+    if not intermediates:
+        return L, grads
+    return L, grads, dict(segA=segA, mu=mu, XN=XN, inv=inv, M=M, G=G, coef=coef, DXN=DXN, dxc=dxc,
+                          colsum2=colsum2)

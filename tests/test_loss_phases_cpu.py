@@ -88,3 +88,30 @@ def test_sharded_statistics_equal_global_batch():
         assert float((g["d_tokens"] - gg["d_tokens"][sl]).abs().max()) < 1e-12
         assert float((g["d_scores"] - gg["d_scores"][sl]).abs().max()) < 1e-12
         assert float((g["d_recon"] - gg["d_recon"][:, sl]).abs().max()) < 1e-12
+
+
+@pytest.mark.parametrize("B", [1, 24])
+def test_domain_term_matches_autograd(B):
+    """Adversarial variant (use_cmd_sim=False): the domain cross-entropy, its gradient wrt the 3B
+    logits (logits up to +-80, so the max subtraction matters) and the CMD-free token gradient."""
+    cfg = types.SimpleNamespace(use_cmd_sim=False, diff_weight=0.3, sim_weight=0.7, recon_weight=0.7,
+                                conf_weight=0.3, use_confidNet=True)
+    X0, O, R, s, t, y = _rand_outputs(B, 16, 6, 2)
+    g = torch.Generator().manual_seed(3)
+    DL = (torch.rand(3 * B, 3, generator=g, dtype=torch.float64) * 2 - 1) * 80
+    leaves = [v.clone().requires_grad_(True) for v in (X0, O, R, s, t, DL)]
+    out = {"scores": leaves[3], "tcp": leaves[4]}
+    for i, m in enumerate(MODS):
+        out[f"utt_private_{m}"], out[f"utt_shared_{m}"] = leaves[0][:, i], leaves[0][:, 3 + i]
+        out[f"utt_{m}_orig"], out[f"utt_{m}_recon"] = leaves[1][i], leaves[2][i]
+        out[f"domain_label_{m}"] = leaves[5][i * B:(i + 1) * B]
+    Lr = oracle_losses(out, y, cfg)
+    Lr["total"].backward()
+    w = dict(diff=0.3, sim=0.7, recon=0.7, conf=0.3)
+    L, g = phased_loss(X0, O, R, s, t, y, float(B), w, DL=DL)
+    for k in ("cls", "diff", "sim", "recon", "conf", "total"):
+        assert abs(float(L[k]) - float(Lr[k])) < 1e-10 * max(1, abs(float(Lr[k]))), k
+    ref = dict(d_tokens=leaves[0].grad, d_orig=leaves[1].grad, d_recon=leaves[2].grad,
+               d_scores=leaves[3].grad, d_tcp=leaves[4].grad, d_domain=leaves[5].grad)
+    for k in g:
+        assert float((g[k] - ref[k]).abs().max()) < 1e-10, k
