@@ -318,13 +318,29 @@ int mmda_eval_accumulate(const float* scores, const float* pred_labels, const fl
 int mmda_adam_clip_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq,
                         long long n, int step, float lr, float clip, float beta1, float beta2,
                         float eps, float grad_scale, const void* state_dev, mmda_stream_t stream);
-/* Device-resident step state (32 bytes: step counter = dropout seed offset, beta^t products, the
- * two Adam bias-correction scalars) so one captured CUDA graph replays step after step.  When
- * state_dev is passed to mmda_adam_clip_step its scalars override `step`. */
+/* ---- clip_grad_value_ + RMSprop.step, src/solver.py:185-186 with config.optimizer = RMSprop
+ * (src/config.py:24-27; constructed as RMSprop(params, lr), src/solver.py:97-99): per element
+ * g = clamp(g*grad_scale, +-clip), v = alpha*v + (1-alpha)*g^2, p -= lr * g / (sqrt(v) + eps).
+ * square_avg is a flat arena of n floats, 16-byte aligned like params / grads.  When state_dev
+ * is passed its learning rate (mmda_step_state_set_lr) overrides `lr`. */
+int mmda_rmsprop_clip_step(float* params, const float* grads, float* square_avg, long long n,
+                           float lr, float clip, float alpha, float eps, float grad_scale,
+                           const void* state_dev, mmda_stream_t stream);
+/* Device-resident step state (40 bytes: step counter = dropout seed offset, beta^t products, the
+ * two Adam bias-correction scalars, the learning rate) so one captured CUDA graph replays step
+ * after step, also under a learning-rate schedule.  When state_dev is passed to
+ * mmda_adam_clip_step its scalars override `step` and `lr`.  init rewrites everything but the
+ * learning rate; set_lr writes the learning rate alone (a stream-ordered copy from pageable host
+ * memory: call it outside a graph capture).  advance takes the learning rate as an argument,
+ * advance_device_lr reads the one set_lr stored; both give bit-identical step sizes for the same
+ * float learning rate. */
 int mmda_step_state_init(void* state_dev, long long step, float beta1, float beta2,
                          mmda_stream_t stream);
 int mmda_step_state_advance(void* state_dev, float lr, float beta1, float beta2,
                             mmda_stream_t stream);
+int mmda_step_state_set_lr(void* state_dev, float lr, mmda_stream_t stream);
+int mmda_step_state_advance_device_lr(void* state_dev, float beta1, float beta2,
+                                      mmda_stream_t stream);
 
 /* ---- nn.GRU cells (SURVEY.md 8f N4): rnn = nn.GRU when config.rnncell != 'lstm',
  * src/models.py:39,168-169,177-178.  The recurrence kernels are shared with the LSTM: GRU

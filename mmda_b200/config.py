@@ -36,6 +36,37 @@ def activation_name(act: Any) -> str:
     return name
 
 
+# optimizers the fused step implements, with the settings the reference constructs them with
+# (``config.optimizer(params, lr=...)``, reference src/solver.py:97-99: torch's defaults)
+OPTIMIZERS = {
+    "Adam": dict(betas=(0.9, 0.999), eps=1e-8, weight_decay=0, amsgrad=False, maximize=False),
+    "RMSprop": dict(alpha=0.99, eps=1e-8, weight_decay=0, momentum=0, centered=False, maximize=False),
+}
+
+
+def optimizer_name(opt: Any) -> str:
+    """Map what the reference stores in ``config.optimizer`` (a ``torch.optim`` *class*, reference
+    ``src/config.py:24-27,76-77``), an instance of one, or a plain string onto "Adam" or
+    "RMSprop".  An instance must use the reference's settings (anything but the learning rate at
+    torch's defaults); its learning rate is not read: ``learning_rate`` sets it."""
+    if isinstance(opt, str):
+        name = {k.lower(): k for k in OPTIMIZERS}.get(opt.lower())
+    else:
+        cls = opt if isinstance(opt, type) else type(opt)
+        name = cls.__name__ if cls.__name__ in OPTIMIZERS else None
+    if name is None:
+        raise ValueError(f"optimizer {opt!r} has no fused step in this build "
+                         f"(supported: {sorted(OPTIMIZERS)})")
+    defaults = getattr(opt, "defaults", None)
+    if not isinstance(opt, (str, type)) and isinstance(defaults, dict):
+        bad = {k: defaults[k] for k, v in OPTIMIZERS[name].items()
+               if k in defaults and (tuple(defaults[k]) if k == "betas" else defaults[k]) != v}
+        if bad:
+            raise ValueError(f"{name} with {bad}: only {name}(params, lr) is implemented "
+                             f"({', '.join(f'{k}={v}' for k, v in OPTIMIZERS[name].items())})")
+    return name
+
+
 @dataclass
 class MisaConfig:
     # --- model (reference src/models.py:20-47, src/config.py:146-154) ---
@@ -64,6 +95,7 @@ class MisaConfig:
     recon_weight: float = 0.7
     conf_weight: float = 0.3
     learning_rate: float = 1e-4
+    optimizer: Any = "Adam"          # torch.optim.Adam / RMSprop (class or instance) or its name
     clip: float = 1.0
     batch_size: int = 64
     model: str = "MISA"

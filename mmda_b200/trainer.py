@@ -1,7 +1,8 @@
 """Level-2 fused training step: the reference's ``Solver.train`` inner loop
 (src/solver.py:139-193: zero_grad, forward, six losses, weighted sum, backward,
-clip_grad_value_, Adam.step) with no autograd, every stage a C-ABI kernel, parameters / gradients
-/ Adam moments in flat 16-byte aligned arenas, and -- when a process group is given -- batch-
+clip_grad_value_, optimizer.step with the Adam or RMSprop that ``config.optimizer`` names) with no
+autograd, every stage a C-ABI kernel, parameters / gradients / optimizer state in flat 16-byte
+aligned arenas, and -- when a process group is given -- batch-
 sharded data parallelism with exact global-batch semantics:
 
 * the three loss statistics segments are all-reduced between loss phases (SURVEY.md row D1:
@@ -20,6 +21,7 @@ import torch
 
 from ._lib import LIB, MmdaError
 from . import engine as _engine
+from .config import OPTIMIZERS, optimizer_name
 from .engine import MODS, _ptr
 
 ALIGN = 64      # floats; every parameter starts on a 256-byte boundary of the arena
@@ -146,6 +148,10 @@ class FusedTrainer:
         self.model = model
         self.cfg = cfg = model.config
         self.use_bert = bool(getattr(cfg, "use_bert", False))
+        try:
+            self.optimizer = optimizer_name(getattr(cfg, "optimizer", "Adam"))
+        except ValueError as e:
+            raise MmdaError(str(e)) from None
         self.eng = model.engine
         self.lr = float(cfg.learning_rate if lr is None else lr)
         self.clip = float(cfg.clip)
@@ -159,15 +165,17 @@ class FusedTrainer:
         self.use_confid = bool(getattr(cfg, "use_confidNet", False))
         self.step_count = 0
         self._build_arena()
-        self.m = torch.zeros_like(self.p_arena)
-        self.v = torch.zeros_like(self.p_arena)
+        self.m = torch.zeros_like(self.p_arena)     # Adam exp_avg (unused by RMSprop)
+        self.v = torch.zeros_like(self.p_arena)     # Adam exp_avg_sq / RMSprop square_avg
         self._pending = []
         self._reduced = set()
         self._defer_ready = None
         self._equal_B = None            # local batch size last verified equal on every rank
         self.trace_ready = None         # profiling aid: {tag: timed event} of the last step
-        # device-resident step state (step counter = dropout seed offset, Adam bias corrections)
-        self.state = torch.zeros(4, dtype=torch.float64, device=self.p_arena.device)
+        # device-resident step state (step counter = dropout seed offset, Adam bias corrections,
+        # learning rate: csrc/adam.cu StepState, 40 bytes)
+        self.state = torch.zeros(5, dtype=torch.float64, device=self.p_arena.device)
+        self._lr_dev = None             # learning rate last written into self.state
         if not _engine._DRYRUN:
             self.eng.k.bind_stream()
             self.eng.k._c("mmda_step_state_init", _ptr(self.state), 0, 0.9, 0.999)
@@ -433,8 +441,9 @@ class FusedTrainer:
         self._check_alias()
         self._check_equal_batch(int(lengths.numel()))
         eng = self.eng
+        self._write_lr()
         eng.k.bind_stream()
-        eng.k._c("mmda_step_state_advance", _ptr(self.state), self.lr, 0.9, 0.999)
+        eng.k._c("mmda_step_state_advance_device_lr", _ptr(self.state), 0.9, 0.999)
         utt_text = None
         if self.use_bert:
             if bert is None or any(t is None for t in bert):
@@ -487,53 +496,108 @@ class FusedTrainer:
         self._pending = []
         return losses
 
+    def _write_lr(self):
+        """Store ``self.lr`` in the device step state when it differs from the value last written.
+        The advance kernel of every step (and RMSprop) reads it from there, so a captured step
+        replays with whatever rate a schedule has set since.  Called outside any capture (step()
+        writes it before capturing or replaying); the float the ABI takes is the rounding the
+        host-lr path applied, so a constant rate gives the same bits as before."""
+        lr = float(self.lr)
+        if lr == self._lr_dev:
+            return
+        if not _engine._DRYRUN:
+            self.eng.k.bind_stream()
+        LIB.call("mmda_step_state_set_lr", _ptr(self.state), lr, self.eng.k.stream)
+        self._lr_dev = lr
+
     def optimizer_step(self):
+        """clip_grad_value_ + the configured optimizer's step over the active arena; the learning
+        rate is the one forward_backward / step() stored in the step state."""
         self.step_count += 1
         k = self.eng.k
         k.bind_stream()
-        k._c("mmda_adam_clip_step", _ptr(self.p_arena), _ptr(self.g_arena), _ptr(self.m),
-             _ptr(self.v), self.n_active, self.step_count, self.lr, self.clip, 0.9, 0.999, 1e-8,
-             self._grad_scale(), _ptr(self.state))
+        if self.optimizer == "RMSprop":
+            o = OPTIMIZERS["RMSprop"]
+            k._c("mmda_rmsprop_clip_step", _ptr(self.p_arena), _ptr(self.g_arena), _ptr(self.v),
+                 self.n_active, self.lr, self.clip, o["alpha"], o["eps"], self._grad_scale(),
+                 _ptr(self.state))
+        else:
+            k._c("mmda_adam_clip_step", _ptr(self.p_arena), _ptr(self.g_arena), _ptr(self.m),
+                 _ptr(self.v), self.n_active, self.step_count, self.lr, self.clip, 0.9, 0.999, 1e-8,
+                 self._grad_scale(), _ptr(self.state))
 
     # -- checkpoint interop: the reference saves / reloads ``optimizer.state_dict()`` next to the
-    # model's (src/solver.py:219-220, :238-239); the fused step owns the Adam moments, so it speaks
-    # torch.optim.Adam's format in both directions ------------------------------------------------
+    # model's (src/solver.py:219-220, :238-239); the fused step owns the optimizer state, so it
+    # speaks torch.optim.Adam's or torch.optim.RMSprop's format in both directions ---------------
+    _STATE_KEYS = {"Adam": ("exp_avg", "exp_avg_sq"), "RMSprop": ("square_avg",)}
+
     def _adam_params(self):
-        """[(index, name, parameter)] in the order ``Adam(filter(requires_grad, parameters()))``
+        """[(index, name, parameter)] in the order ``optimizer(filter(requires_grad, parameters()))``
         (src/solver.py:97-99) numbers them"""
         return [(i, n, p) for i, (n, p) in enumerate(
             (n, p) for n, p in self.model.named_parameters() if p.requires_grad)]
 
+    def _state_arenas(self):
+        """{state_dict key: arena} of the configured optimizer"""
+        if self.optimizer == "RMSprop":
+            return {"square_avg": self.v}
+        return {"exp_avg": self.m, "exp_avg_sq": self.v}
+
     def optimizer_state_dict(self):
-        """The Adam state in ``torch.optim.Adam.state_dict()`` layout: loadable by the reference's
+        """The optimizer state in ``torch.optim.Adam.state_dict()`` layout (or
+        ``torch.optim.RMSprop``'s, with ``config.optimizer = RMSprop``): loadable by the reference's
         optimizer (``self.optimizer.load_state_dict``) built over the same model.  Parameters that
-        never received a gradient (``grad=None`` in the reference: Adam keeps no state for them)
+        never received a gradient (``grad=None`` in the reference: torch keeps no state for them)
         have no entry, exactly as torch leaves them."""
         params = self._adam_params()
+        arenas = self._state_arenas()
         state = {}
         if self.step_count > 0:
             for i, n, p in params:
                 off, sz = self.layout[n]
                 if off >= self.n_active:
                     continue
-                state[i] = {"step": torch.tensor(float(self.step_count)),
-                            "exp_avg": self.m[off:off + sz].view(p.shape).clone(),
-                            "exp_avg_sq": self.v[off:off + sz].view(p.shape).clone()}
-        group = {"lr": self.lr, "betas": (0.9, 0.999), "eps": 1e-8, "weight_decay": 0,
-                 "amsgrad": False, "maximize": False, "foreach": None, "capturable": False,
-                 "differentiable": False, "fused": None, "decoupled_weight_decay": False,
-                 "params": [i for i, _, _ in params]}
+                state[i] = {"step": torch.tensor(float(self.step_count))}
+                for key, arena in arenas.items():
+                    state[i][key] = arena[off:off + sz].view(p.shape).clone()
+        if self.optimizer == "RMSprop":
+            group = {"lr": self.lr, "momentum": 0, "alpha": 0.99, "eps": 1e-8, "centered": False,
+                     "weight_decay": 0, "capturable": False, "foreach": None, "maximize": False,
+                     "differentiable": False}
+        else:
+            group = {"lr": self.lr, "betas": (0.9, 0.999), "eps": 1e-8, "weight_decay": 0,
+                     "amsgrad": False, "maximize": False, "foreach": None, "capturable": False,
+                     "differentiable": False, "fused": None, "decoupled_weight_decay": False}
+        group["params"] = [i for i, _, _ in params]
         return {"state": state, "param_groups": [group]}
 
     def load_optimizer_state_dict(self, sd):
         """Inverse of ``optimizer_state_dict``; also accepts a checkpoint written by the
-        reference's ``torch.optim.Adam`` (``checkpoints/optim_*.std``).  Restores the moments, the
-        step count (bias corrections, dropout stream) and the learning rate."""
+        reference's ``torch.optim.Adam`` / ``torch.optim.RMSprop`` (``checkpoints/optim_*.std``),
+        whichever ``config.optimizer`` names.  Restores the optimizer state, the step count (bias
+        corrections, dropout stream) and the learning rate (written to the device before the next
+        step, so a captured step graph stays valid)."""
         groups = sd["param_groups"]
         if len(groups) != 1:
             raise MmdaError("optimizer state with %d param groups (the reference uses one)" % len(groups))
         g = groups[0]
-        if tuple(g.get("betas", (0.9, 0.999))) != (0.9, 0.999) or float(g.get("eps", 1e-8)) != 1e-8 \
+        keys = set(g) | {k for st in sd["state"].values() for k in st}
+        saved = [name for name, ks in self._STATE_KEYS.items()
+                 if ks[0] in keys or (name == "Adam" and "betas" in keys)
+                 or (name == "RMSprop" and "alpha" in keys)]
+        if saved and saved != [self.optimizer]:
+            raise MmdaError(f"optimizer state of {' / '.join(saved)}, but config.optimizer is "
+                            f"{self.optimizer}: load it into a trainer configured with the same "
+                            "optimizer")
+        if self.optimizer == "RMSprop":
+            o = OPTIMIZERS["RMSprop"]
+            if float(g.get("alpha", o["alpha"])) != o["alpha"] or float(g.get("eps", o["eps"])) != o["eps"] \
+                    or g.get("momentum", 0) or g.get("centered", False) or g.get("weight_decay", 0) \
+                    or g.get("maximize", False):
+                raise MmdaError("only RMSprop(alpha=0.99, eps=1e-8, momentum=0, centered=False, "
+                                "weight_decay=0) is implemented (src/solver.py:97-99 with "
+                                "config.optimizer = RMSprop)")
+        elif tuple(g.get("betas", (0.9, 0.999))) != (0.9, 0.999) or float(g.get("eps", 1e-8)) != 1e-8 \
                 or g.get("weight_decay", 0) or g.get("amsgrad", False):
             raise MmdaError("only Adam(betas=(0.9, 0.999), eps=1e-8, weight_decay=0) is implemented "
                             "(src/solver.py:97-99 with config.optimizer = Adam)")
@@ -542,6 +606,7 @@ class FusedTrainer:
             raise MmdaError(f"optimizer state covers {len(g['params'])} parameters, the model has "
                             f"{len(params)} trainable ones")
         pos = {pid: j for j, pid in enumerate(g["params"])}     # saved id -> position in the group
+        arenas = self._state_arenas()
         self.m.zero_()
         self.v.zero_()
         steps = set()
@@ -550,21 +615,24 @@ class FusedTrainer:
                 raise MmdaError(f"optimizer state for parameter id {pid!r}, which its param group does not list")
             _, n, p = params[pos[pid]]
             off, sz = self.layout[n]
-            if tuple(st["exp_avg"].shape) != tuple(p.shape):
-                raise MmdaError(f"optimizer state of {n}: shape {tuple(st['exp_avg'].shape)} != {tuple(p.shape)}")
+            for key in arenas:
+                if tuple(st[key].shape) != tuple(p.shape):
+                    raise MmdaError(f"optimizer state of {n}: shape {tuple(st[key].shape)} != {tuple(p.shape)}")
             if off >= self.n_active:
                 raise MmdaError(f"optimizer state for {n}, which this variant never differentiates")
-            self.m[off:off + sz].view(p.shape).copy_(st["exp_avg"])
-            self.v[off:off + sz].view(p.shape).copy_(st["exp_avg_sq"])
+            for key, arena in arenas.items():
+                arena[off:off + sz].view(p.shape).copy_(st[key])
             steps.add(int(st["step"]))
         if len(steps) > 1:
-            raise MmdaError(f"parameters at different Adam steps {sorted(steps)}: one fused step count only")
+            raise MmdaError(f"parameters at different {self.optimizer} steps {sorted(steps)}: one "
+                            "fused step count only")
         self.step_count = steps.pop() if steps else 0
         self.lr = float(g["lr"])
         if not _engine._DRYRUN:
             self.eng.k.bind_stream()
+        # rewrites the step counter and beta products in place: a captured step reads them by
+        # pointer, so it stays valid
         self.eng.k._c("mmda_step_state_init", _ptr(self.state), self.step_count, 0.9, 0.999)
-        self._drop_graph()       # the learning rate is a captured scalar
 
     def _grad_scale(self):
         """Per-shard losses (global_batch_stats=False) are normalised by the LOCAL batch, so the
@@ -580,8 +648,10 @@ class FusedTrainer:
              bert_sent_type=None, bert_sent_mask=None):
         """One optimisation step.  With ``use_graph`` (default on one GPU) the kernel sequence of
         a repeated (shapes, lengths) pattern is captured once into a CUDA graph -- multi-stream
-        forks included -- and replayed; per-step scalars live in ``self.state`` on the device."""
+        forks included -- and replayed; per-step scalars, the learning rate included, live in
+        ``self.state`` on the device, so changing ``self.lr`` between steps keeps the graph."""
         self._check_equal_batch(int(lengths.numel()))     # before any capture: it reads a value back
+        self._write_lr()                                   # before any capture: a host->device copy
         if self.use_bert:       # long step (12 transformer layers): launch overhead is noise
             return self._eager_step(sentences, visual, acoustic, lengths, labels,
                                     (bert_sent, bert_sent_type, bert_sent_mask))
@@ -601,7 +671,7 @@ class FusedTrainer:
         if visual.shape[0] != T or acoustic.shape[0] != T or int(lengths.max()) > T:
             return self._eager_step(sentences, visual, acoustic, lengths, labels)
         key = (tuple(sentences.shape), tuple(visual.shape), tuple(acoustic.shape), Np, N == Np,
-               self.model.training, float(self.lr))
+               self.model.training)
         alias = tuple(p.data_ptr() for p in self.model.parameters()) + \
             tuple(p.requires_grad for p in self.model.parameters())
         if self._graphs and (self._graphs_ws != self.eng.ws_version or self._graphs_alias != alias):
