@@ -109,9 +109,6 @@ int mmda_gemm_tc(int kind, int a_mn, int b_mn, int M, int N, int K, const void* 
                  const void* A_lo, int lda, const void* B_hi, const void* B_lo, int ldb, float alpha,
                  float* C, int ldc, const float* bias, const float* bias2, int mode, int split_k,
                  int c_row_interleave, mmda_stream_t stream);
-/* A/B knob: 2 = persistent tile loop, dynamic tile scheduler, epilogue overlapped with the next
- * tile's MMAs (default); 1 = one output tile per CTA. */
-int mmda_gemm_tc_set_version(int version);
 /* tile-scheduler slots owned by launches recorded into CUDA graphs: returns the number in use;
  * release_to >= 0 first hands back the slots [release_to, in use) (the graphs recorded since that
  * mark must be destroyed).  release_to = -1 only queries. */
@@ -151,8 +148,6 @@ int mmda_lstm_pack_weights(const float* w_ih_f, const float* w_ih_r, const float
                            const float* b_hh_f, const float* b_ih_r, const float* b_hh_r, int H, int I,
                            int mode, void* out_a, float* out_b, int ld, float* bias_out,
                            mmda_stream_t stream);
-/* A/B knob: batch tile of the small-hidden-size plan (8 = many small CTAs, 32 = few large ones) */
-int mmda_lstm_set_small_tile(int bt);
 /* diagnostic: per-step phase timestamps of CTA 0 of subsequent forward launches (NULL = off) */
 int mmda_lstm_set_debug_buffer(long long* dev_buf);
 /* diagnostic: co-resident clusters of the recurrent kernel for cluster sizes {1,2,4,8,16} */
@@ -185,15 +180,8 @@ int mmda_lstm_tc_backward(float* gates, const float* whh_f, const float* whh_r, 
                           int utt_off_r, const int* lens_sorted, const int* sorted_idx,
                           const int* offsets, int B, int H, int Tmax, void* ws,
                           mmda_stream_t stream);
-/* A/B knob: largest batch tile of the forward recurrence (default 64 rows; 48 gives 6 tiles /
- * 120 CTAs at B = 256 -- faster stand-alone, see DESIGN.md 3.1) */
-int mmda_lstm_tc_set_fwd_rows(int rows);
-/* A/B knob: SMs one launch may occupy (default 120: the rest serve the concurrent encoders) */
-int mmda_lstm_tc_set_max_ctas(int n);
 /* diagnostic: per-step phase timestamps of CTA 0 (NULL = off) */
 int mmda_lstm_tc_set_debug_buffer(long long* dev_buf);
-/* diagnostic, timing experiments only (results become wrong): backward kernel skips parts of a step */
-int mmda_lstm_tc_set_debug_flags(int flags);
 
 /* ---- nn.LayerNorm, src/models.py:65-80,155-157,172 and the two norms of the fusion layer ----
  * y = LN(x + res) (res may be NULL); mean/rstd saved per row for the backward. */

@@ -15,8 +15,6 @@ from __future__ import annotations
 
 from typing import Dict, Optional
 
-import os
-
 import torch
 
 from ._lib import LIB, MmdaError
@@ -145,7 +143,7 @@ class BertEngine:
         (S <= 84 with a backward, S <= 116 without); longer sequences go to the tiled kernels
         (`_tiled_mma` in bf16 mode, `_tiled` in fp32 mode), which hold no S x S buffer."""
         bf = self.eng.tc_kind == 1
-        if bf and S <= 64 and os.environ.get("MMDA_BERT_ATT", "mma") != "simt":
+        if bf and S <= 64:
             return "_mma"
         key = 1 if train else 0
         if key not in self._resident_max:

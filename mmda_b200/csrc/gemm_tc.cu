@@ -14,9 +14,10 @@
 // MN-major (the weight-gradient GEMMs contract over tokens, so dG / X / h_prev are read straight
 // from their [token][feature] layout without any transpose pass).
 //
-// One 128x128 output tile per CTA, 192 threads: warp 0 = TMA producer, warp 1 = MMA issuer +
-// TMEM allocator, warps 2..5 = epilogue (each warp drains the TMEM lane quarter warp_id % 4).
-// Split-K (grid.z) reduces with red.global.add for the long-K weight-gradient shapes.
+// One persistent CTA per SM loops over 128x128 output tiles, 192 threads: warp 0 = tile scheduler
+// + TMA producer, warp 1 = MMA issuer + TMEM allocator, warps 2..5 = epilogue (each warp drains the
+// TMEM lane quarter warp_id % 4); plain-fp32 operands add four converter warps.  Split-K slices
+// reduce with red.global.add for the long-K weight-gradient shapes.
 #include "common.cuh"
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -105,218 +106,12 @@ struct TcArgs {
   int a_mn, b_mn;       // 1 = MN-major operand
   float alpha;
   int mode;             // 0 store, 1 C += , 2 atomic add (split-K)
-  int kb_per_split;     // K blocks per grid.z slice
+  int kb_per_split;     // K blocks per split-K slice
   int c_ilv;            // H: logical C row u*4+g is stored at row g*H+u; 0: identity
 };
 
-template <int KIND>
-__global__ void __launch_bounds__(NUM_THREADS, 1)
-gemm_tc_kernel(const __grid_constant__ CUtensorMap mapAh, const __grid_constant__ CUtensorMap mapAl,
-               const __grid_constant__ CUtensorMap mapBh, const __grid_constant__ CUtensorMap mapBl,
-               const TcArgs p) {
-  constexpr int ESZ = KIND == 0 ? 4 : 2;
-  constexpr int BK = 128 / ESZ;               // 32 (tf32) / 64 (bf16): one 128-byte swizzle row
-  constexpr int UK = 32 / ESZ;                // UMMA K: 8 / 16
-  constexpr int NPART = KIND == 0 ? 2 : 1;    // hi+lo or single
-  constexpr int STAGES = KIND == 0 ? 3 : 6;
-  constexpr int STAGE_BYTES = 2 * NPART * TILE_BYTES;
-  constexpr int MN_CHUNK = 128 / ESZ;         // MN elements per 128-byte chunk (MN-major tiles)
-  constexpr int N_CHUNKS = 128 / MN_CHUNK;    // 4 / 2
-  constexpr int CHUNK_BYTES = BK * 128;       // one MN-major chunk: BK k-rows x 128 B
-  // The tensor core adds into the fp32 accumulator with truncation, so a long accumulation
-  // chain drifts (measured 8e-5 relative at K=12800).  3xTF32 therefore rotates the hi*hi
-  // products over NMAIN accumulators and keeps the small cross terms (lo*hi + hi*lo) in their
-  // own one; the epilogue adds the partials in round-to-nearest fp32.
-  constexpr int NMAIN = KIND == 0 ? 3 : 1;
-  constexpr int NACC = KIND == 0 ? 4 : 1;
-  constexpr int TMEM_COLS = NACC * 128;       // 512 / 128
-  // tf32 MN-major operands must use the "128B swizzle, 32B atom" layout (UMMA layout type 1,
-  // 4-row atoms); everything else uses the plain 128B swizzle (type 2, 8-row atoms)
-  constexpr uint32_t MN_LAYOUT = KIND == 0 ? 1u : 2u;
-  constexpr uint32_t MN_SBO = KIND == 0 ? 512u : 1024u;
-
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t bar_base = base + STAGES * STAGE_BYTES;   // full[S], empty[S], tmem_full, tmem ptr
-  auto full_bar = [&](int s) { return bar_base + 8u * s; };
-  auto empty_bar = [&](int s) { return bar_base + 8u * (STAGES + s); };
-  const uint32_t tmem_full_bar = bar_base + 8u * (2 * STAGES);
-  const uint32_t tmem_slot = bar_base + 8u * (2 * STAGES + 1);
-  uint32_t* tmem_slot_ptr = reinterpret_cast<uint32_t*>(smem_raw + (tmem_slot - smem_u32(smem_raw)));
-  // epilogue staging: 4 warps x (32 x 33) floats, after the barrier block
-  float* stage_base = reinterpret_cast<float*>(smem_raw + (bar_base + 256 - smem_u32(smem_raw)));
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int m0 = blockIdx.y * BM, n0 = blockIdx.x * BN;
-  const int kb_total = (p.K + BK - 1) / BK;
-  const int kb_beg = blockIdx.z * p.kb_per_split;
-  const int kb_end = min(kb_total, kb_beg + p.kb_per_split);
-  const int num_kb = max(0, kb_end - kb_beg);
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < STAGES; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-    mbar_init(tmem_full_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {   // TMEM: 128 fp32 accumulator columns
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot),
-                 "n"(TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_acc = *tmem_slot_ptr;
-
-  if (warp == 0) {
-    // ===================== TMA producer =====================
-    if (lane == 0) {
-      for (int i = 0; i < num_kb; ++i) {
-        const int s = i % STAGES, it = i / STAGES;
-        mbar_wait(empty_bar(s), (it & 1) ^ 1);
-        const uint32_t st = base + s * STAGE_BYTES;
-        mbar_expect_tx(full_bar(s), STAGE_BYTES);
-        const int k0 = (kb_beg + i) * BK;
-#pragma unroll
-        for (int part = 0; part < NPART; ++part) {
-          const CUtensorMap* mA = part == 0 ? &mapAh : &mapAl;
-          const CUtensorMap* mB = part == 0 ? &mapBh : &mapBl;
-          const uint32_t sa = st + part * TILE_BYTES;
-          const uint32_t sb = st + (NPART + part) * TILE_BYTES;
-          if (p.a_mn) {
-            for (int c = 0; c < N_CHUNKS; ++c)
-              tma_load_2d(sa + c * CHUNK_BYTES, mA, full_bar(s), m0 + c * MN_CHUNK, k0);
-          } else {
-            tma_load_2d(sa, mA, full_bar(s), k0, m0);
-          }
-          if (p.b_mn) {
-            for (int c = 0; c < N_CHUNKS; ++c)
-              tma_load_2d(sb + c * CHUNK_BYTES, mB, full_bar(s), n0 + c * MN_CHUNK, k0);
-          } else {
-            tma_load_2d(sb, mB, full_bar(s), k0, n0);
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===================== MMA issuer =====================
-    if (lane == 0) {
-      // instruction descriptor (cute::UMMA::InstrDescriptor): c=F32, a/b format, majors, N>>3, M>>4
-      const uint32_t fmt = KIND == 0 ? 2u : 1u;
-      const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)p.a_mn << 15) |
-                             ((uint32_t)p.b_mn << 16) | ((uint32_t)(BN >> 3) << 17) |
-                             ((uint32_t)(BM >> 4) << 24);
-      for (int i = 0; i < num_kb; ++i) {
-        const int s = i % STAGES, it = i / STAGES;
-        mbar_wait(full_bar(s), it & 1);
-        tc_fence_after();
-        const uint32_t st = base + s * STAGE_BYTES;
-#pragma unroll
-        for (int ks = 0; ks < BK / UK; ++ks) {
-          // K-major: advance 32 B inside the 128-B swizzled row; MN-major: advance UK k-rows
-          const uint32_t offA = p.a_mn ? ks * UK * 128 : ks * 32;
-          const uint32_t offB = p.b_mn ? ks * UK * 128 : ks * 32;
-          const uint32_t lboA = p.a_mn ? CHUNK_BYTES : 16, lboB = p.b_mn ? CHUNK_BYTES : 16;
-          const uint32_t sboA = p.a_mn ? MN_SBO : 1024u, sboB = p.b_mn ? MN_SBO : 1024u;
-          const uint32_t ltA = p.a_mn ? MN_LAYOUT : 2u, ltB = p.b_mn ? MN_LAYOUT : 2u;
-          const uint64_t dAh = make_desc(st + offA, lboA, sboA, ltA);
-          const uint64_t dBh = make_desc(st + NPART * TILE_BYTES + offB, lboB, sboB, ltB);
-          const int gk = i * (BK / UK) + ks;          // global k-step of this CTA
-          if (KIND == 0) {
-            const uint64_t dAl = make_desc(st + TILE_BYTES + offA, lboA, sboA, ltA);
-            const uint64_t dBl = make_desc(st + 3 * TILE_BYTES + offB, lboB, sboB, ltB);
-            const uint32_t cross = tmem_acc + NMAIN * 128;
-            tc_mma<KIND>(cross, dAl, dBh, idesc, gk > 0 ? 1u : 0u);
-            tc_mma<KIND>(cross, dAh, dBl, idesc, 1u);
-            tc_mma<KIND>(tmem_acc + (gk % NMAIN) * 128, dAh, dBh, idesc, gk >= NMAIN ? 1u : 0u);
-          } else {
-            tc_mma<KIND>(tmem_acc, dAh, dBh, idesc, gk > 0 ? 1u : 0u);
-          }
-        }
-        tc_commit(empty_bar(s));          // frees the smem stage once these MMAs retire
-      }
-      tc_commit(tmem_full_bar);           // accumulator complete
-    }
-  } else {
-    // ===================== epilogue: TMEM -> registers -> global =====================
-    const int q = warp & 3;               // TMEM lane quarter this warp may access
-    const int row = m0 + q * 32 + lane;
-    if (num_kb > 0) {
-      mbar_wait(tmem_full_bar, 0);
-      tc_fence_after();
-    }
-#pragma unroll 1
-    for (int cc = 0; cc < BN / 32; ++cc) {
-      uint32_t r[32];
-#pragma unroll
-      for (int j = 0; j < 32; ++j) r[j] = 0u;
-      if (num_kb > 0) {
-        const int ksteps = num_kb * (BK / UK);
-        const int n_used = KIND == 0 ? (ksteps < NMAIN ? ksteps : NMAIN) + 1 : 1;   // mains + cross
-#pragma unroll 1
-        for (int a = 0; a < n_used; ++a) {
-          const int acc_id = (KIND == 0 && a == n_used - 1) ? NMAIN : a;
-          const uint32_t taddr = tmem_acc + ((uint32_t)(q * 32) << 16) + acc_id * 128 + cc * 32;
-          uint32_t t[32];
-          asm volatile(
-              "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-              "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-              "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-              : "=r"(t[0]), "=r"(t[1]), "=r"(t[2]), "=r"(t[3]), "=r"(t[4]), "=r"(t[5]), "=r"(t[6]),
-                "=r"(t[7]), "=r"(t[8]), "=r"(t[9]), "=r"(t[10]), "=r"(t[11]), "=r"(t[12]), "=r"(t[13]),
-                "=r"(t[14]), "=r"(t[15]), "=r"(t[16]), "=r"(t[17]), "=r"(t[18]), "=r"(t[19]),
-                "=r"(t[20]), "=r"(t[21]), "=r"(t[22]), "=r"(t[23]), "=r"(t[24]), "=r"(t[25]),
-                "=r"(t[26]), "=r"(t[27]), "=r"(t[28]), "=r"(t[29]), "=r"(t[30]), "=r"(t[31])
-              : "r"(taddr)
-              : "memory");
-          asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-          for (int j = 0; j < 32; ++j)
-            r[j] = __float_as_uint(__uint_as_float(r[j]) + __uint_as_float(t[j]));
-        }
-      }
-      // Transpose the warp's 32x32 chunk through shared memory so that every store / atomic
-      // instruction covers 32 consecutive columns of ONE row (a single 128-byte line) instead
-      // of one column group of 32 different rows.
-      const int nb = n0 + cc * 32;
-      float* stage = stage_base + (warp - 2) * (32 * 33);
-#pragma unroll
-      for (int j = 0; j < 32; ++j) stage[lane * 33 + j] = __uint_as_float(r[j]);
-      __syncwarp();
-      const int col = nb + lane;
-      if (col < p.N) {
-        float bsum = 0.f;
-        if (blockIdx.z == 0) {
-          if (p.bias) bsum += p.bias[col];
-          if (p.bias2) bsum += p.bias2[col];
-        }
-        const int row_base = m0 + q * 32;
-#pragma unroll 4
-        for (int rr = 0; rr < 32; ++rr) {
-          const int grow = row_base + rr;
-          if (grow >= p.M) break;
-          const int row_out = p.c_ilv ? (grow & 3) * p.c_ilv + (grow >> 2) : grow;
-          float* cp = p.C + (size_t)row_out * p.ldc + col;
-          const float v = p.alpha * stage[rr * 33 + lane] + bsum;
-          if (p.mode != 0) atomicAdd(cp, v);   // RED, see the persistent kernel
-          else *cp = v;
-        }
-      }
-      __syncwarp();
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_acc),
-                 "n"(TMEM_COLS)
-                 : "memory");
-  }
-}
-
 // ------------------------------------------------------------------------------------------
-// Persistent variant (default).  One CTA per SM pulls 128x128 output tiles (m fastest, so the
+// Persistent kernel.  One CTA per SM pulls 128x128 output tiles (m fastest, so the
 // CTAs running side by side share B tiles in L2) from a global atomic counter -- dynamic, because
 // these GEMMs often run next to the 112-SM recurrence kernel and must be finished by whichever
 // SMs happen to be free.  The TMA ring and the MMA issue run ahead across tile boundaries; the
@@ -342,20 +137,26 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap mapAh, const __grid_constant
                 const TcArgs2 q2) {
   const TcArgs& p = q2.a;
   constexpr int ESZ = KIND == 0 ? 4 : 2;
-  constexpr int BK = 128 / ESZ;
-  constexpr int UK = 32 / ESZ;
-  constexpr int NPART = KIND == 0 ? 2 : 1;
+  constexpr int BK = 128 / ESZ;               // 32 (tf32) / 64 (bf16): one 128-byte swizzle row
+  constexpr int UK = 32 / ESZ;                // UMMA K: 8 / 16
+  constexpr int NPART = KIND == 0 ? 2 : 1;    // hi+lo or single
   constexpr int STAGES = KIND == 0 ? 3 : 6;
   constexpr int STAGE_BYTES = 2 * NPART * TILE_BYTES;
-  constexpr int MN_CHUNK = 128 / ESZ;
-  constexpr int N_CHUNKS = 128 / MN_CHUNK;
-  constexpr int CHUNK_BYTES = BK * 128;
+  constexpr int MN_CHUNK = 128 / ESZ;         // MN elements per 128-byte chunk (MN-major tiles)
+  constexpr int N_CHUNKS = 128 / MN_CHUNK;    // 4 / 2
+  constexpr int CHUNK_BYTES = BK * 128;       // one MN-major chunk: BK k-rows x 128 B
+  // The tensor core adds into the fp32 accumulator with truncation, so a long accumulation
+  // chain drifts (measured 8e-5 relative at K=12800).  3xTF32 therefore rotates the hi*hi
+  // products over NMAIN accumulators and keeps the small cross terms (lo*hi + hi*lo) in their
+  // own one; the epilogue adds the partials in round-to-nearest fp32.
   constexpr int NMAIN = KIND == 0 ? 3 : 1;
   constexpr int NACC = KIND == 0 ? 4 : 1;
   constexpr int NBUF = KIND == 0 ? 1 : 4;          // TMEM accumulator buffers
   constexpr int BUF_COLS = NACC * 128;
   constexpr int TMEM_COLS = 512;
   constexpr int RING = 4;                          // tile-id ring depth
+  // tf32 MN-major operands must use the "128B swizzle, 32B atom" layout (UMMA layout type 1,
+  // 4-row atoms); everything else uses the plain 128B swizzle (type 2, 8-row atoms)
   constexpr uint32_t MN_LAYOUT = KIND == 0 ? 1u : 2u;
   constexpr uint32_t MN_SBO = KIND == 0 ? 512u : 1024u;
 
@@ -782,7 +583,6 @@ int encode_map(CUtensorMap* map, int kind, const void* ptr, long rows, long cols
   return MMDA_OK;
 }
 
-int g_tc_version = 2;          // 2 = persistent kernel (default), 1 = one tile per CTA (process-wide A/B knob)
 // Scheduler slots (2 ints each, self-resetting) live in the per-device context (common.cuh): eager
 // launches rotate through a ring (a slot is re-armed by its own kernel, and 4096 launches never
 // overlap in flight); launches recorded into a CUDA graph get slots of their own that are only
@@ -833,13 +633,6 @@ int mmda_gemm_tc_graph_slots(int release_to) {
   if (ctx == nullptr) return MMDA_ERR_CUDA;
   if (release_to >= 0 && release_to <= ctx->sched_graph_next) ctx->sched_graph_next = release_to;
   return ctx->sched_graph_next;
-}
-
-// A/B knob: 2 = persistent tile loop with overlapped epilogue (default), 1 = one tile per CTA
-int mmda_gemm_tc_set_version(int v) {
-  MMDA_REQUIRE(v == 1 || v == 2, "gemm_tc: version must be 1 or 2");
-  g_tc_version = v;
-  return MMDA_OK;
 }
 
 int mmda_split_tf32(const float* x, int ldx, int rows, int cols, float* hi, float* lo, int ldo,
@@ -895,7 +688,6 @@ int mmda_gemm_tc(int kind, int a_mn, int b_mn, int M, int N, int K, const void* 
   const bool raw = kind == 2;
   const int raw_mode = !raw ? 0 : (B_lo != nullptr ? 2 : 1);    // 2: B arrives pre-split
   if (raw) { kind = 0; A_lo = A_hi; if (B_lo == nullptr) B_lo = B_hi; }
-  MMDA_REQUIRE(!raw || g_tc_version == 2, "gemm_tc: kind 2 needs the persistent kernel");
   MMDA_REQUIRE(kind == 0 || kind == 1, "gemm_tc: kind=%d", kind);
   MMDA_REQUIRE(K > 0 && A_hi && B_hi && C, "gemm_tc: bad arguments");
   MMDA_REQUIRE(kind == 1 || (A_lo && B_lo), "gemm_tc: 3xTF32 needs the lo parts");
@@ -936,43 +728,29 @@ int mmda_gemm_tc(int kind, int a_mn, int b_mn, int M, int N, int K, const void* 
   a.mode = split_k > 1 ? 2 : mode;
   a.kb_per_split = (kb_total + split_k - 1) / split_k;
   a.c_ilv = c_row_interleave;
-  if (g_tc_version == 2) {
-    TcArgs2 a2;
-    a2.a = a;
-    a2.tiles_m = (M + BM - 1) / BM; a2.tiles_n = (N + BN - 1) / BN; a2.split = split_k;
-    a2.total = a2.tiles_m * a2.tiles_n * split_k;
-    MmdaDeviceCtx* ctx = mmda_device_ctx();
-    if (ctx == nullptr) return MMDA_ERR_CUDA;
-    a2.sched = next_sched_slot(ctx, stream);
-    if (a2.sched == nullptr) return MMDA_ERR_CUDA;
-    const int n_sm = ctx->sm_count;
-    const int ctas = a2.total < n_sm ? a2.total : n_sm;
-    constexpr int smem2 = 12 * TILE_BYTES + 1024 + 512 + 4 * 32 * 33 * 4;
-    if (kind == 0 && raw_mode == 1) {
-      MMDA_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
-      gemm_tc2_kernel<0, 1><<<ctas, NUM_THREADS + 128, smem2, stream>>>(mAh, mAl, mBh, mBl, a2);
-    } else if (kind == 0 && raw_mode == 2) {
-      MMDA_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<0, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
-      gemm_tc2_kernel<0, 2><<<ctas, NUM_THREADS + 128, smem2, stream>>>(mAh, mAl, mBh, mBl, a2);
-    } else if (kind == 0) {
-      MMDA_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
-      gemm_tc2_kernel<0, 0><<<ctas, NUM_THREADS, smem2, stream>>>(mAh, mAl, mBh, mBl, a2);
-    } else {
-      MMDA_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
-      gemm_tc2_kernel<1, 0><<<ctas, NUM_THREADS, smem2, stream>>>(mAh, mAl, mBh, mBl, a2);
-    }
-    MMDA_CHECK_LAUNCH();
-    return MMDA_OK;
-  }
-  dim3 grid((N + BN - 1) / BN, (M + BM - 1) / BM, split_k);
-  if (kind == 0) {
-    constexpr int smem = 3 * 4 * TILE_BYTES + 1024 + 256 + 4 * 32 * 33 * 4;
-    MMDA_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    gemm_tc_kernel<0><<<grid, NUM_THREADS, smem, stream>>>(mAh, mAl, mBh, mBl, a);
+  TcArgs2 a2;
+  a2.a = a;
+  a2.tiles_m = (M + BM - 1) / BM; a2.tiles_n = (N + BN - 1) / BN; a2.split = split_k;
+  a2.total = a2.tiles_m * a2.tiles_n * split_k;
+  MmdaDeviceCtx* ctx = mmda_device_ctx();
+  if (ctx == nullptr) return MMDA_ERR_CUDA;
+  a2.sched = next_sched_slot(ctx, stream);
+  if (a2.sched == nullptr) return MMDA_ERR_CUDA;
+  const int n_sm = ctx->sm_count;
+  const int ctas = a2.total < n_sm ? a2.total : n_sm;
+  constexpr int smem2 = 12 * TILE_BYTES + 1024 + 512 + 4 * 32 * 33 * 4;
+  if (kind == 0 && raw_mode == 1) {
+    MMDA_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
+    gemm_tc2_kernel<0, 1><<<ctas, NUM_THREADS + 128, smem2, stream>>>(mAh, mAl, mBh, mBl, a2);
+  } else if (kind == 0 && raw_mode == 2) {
+    MMDA_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<0, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
+    gemm_tc2_kernel<0, 2><<<ctas, NUM_THREADS + 128, smem2, stream>>>(mAh, mAl, mBh, mBl, a2);
+  } else if (kind == 0) {
+    MMDA_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
+    gemm_tc2_kernel<0, 0><<<ctas, NUM_THREADS, smem2, stream>>>(mAh, mAl, mBh, mBl, a2);
   } else {
-    constexpr int smem = 6 * 2 * TILE_BYTES + 1024 + 256 + 4 * 32 * 33 * 4;
-    MMDA_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    gemm_tc_kernel<1><<<grid, NUM_THREADS, smem, stream>>>(mAh, mAl, mBh, mBl, a);
+    MMDA_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
+    gemm_tc2_kernel<1, 0><<<ctas, NUM_THREADS, smem2, stream>>>(mAh, mAl, mBh, mBl, a2);
   }
   MMDA_CHECK_LAUNCH();
   return MMDA_OK;

@@ -605,10 +605,8 @@ struct LstmPlan {
   size_t smem_fwd, smem_bwd, scratch_bytes;
 };
 
-// process-wide A/B knob; everything device-dependent (opt-in shared memory, co-resident 8-CTA
-// clusters of the big-H kernel -- B200: 15) lives in the per-device context (common.cuh)
-static int g_small_bt = 32; // batch tile of the small-H plan for B >= 64: few large CTAs leave the SMs next to the
-                            // text recurrence to the weight-gradient GEMMs (7.65 -> 7.59 ms); 8 = many small CTAs
+// everything device-dependent (opt-in shared memory, co-resident 8-CTA clusters of the big-H
+// kernel -- B200: 15) lives in the per-device context (common.cuh)
 
 template <int BT> static int probe_clusters8(int threads, size_t smem) {
   auto kern = lstm_fwd_kernel<BT, 0>;
@@ -633,13 +631,14 @@ static int lstm_make_plan(int B, int H, LstmPlan* pl) {
   const size_t max_smem = (size_t)ctx->max_smem_optin;
   const int Kpad = (H + 3) & ~3;
   // batch tile: large hidden sizes are shared-memory bound (W slice + h tile must fit), small
-  // ones want many CTAs
+  // ones want many CTAs -- except at B >= 64, where few 32-row CTAs leave the SMs next to the text
+  // recurrence to the weight-gradient GEMMs (measured 7.65 -> 7.59 ms against 8-row tiles)
   for (int C = 1; C <= 8; C *= 2) {
     const int Hs = (H + C - 1) / C;
     const int KS = (H > 128) ? 16 : 4;
     const int RS = 32 / KS, R = (4 * Hs + RS - 1) / RS * RS;
     const int cand[3] = {40, 32, 8};
-    for (int ci = (H > 128 ? 0 : (g_small_bt == 32 && B >= 64 ? 1 : 2)); ci < 3; ++ci) {
+    for (int ci = (H > 128 ? 0 : (B >= 64 ? 1 : 2)); ci < 3; ++ci) {
       const int BT = cand[ci];
       if (H > 128 && BT == 8) break;
       const int BTP = BT + (BT % 32 == 0 ? 4 : 0);
@@ -696,13 +695,6 @@ static int launch_cluster(K kern, const LstmArgs& a, const LstmPlan& pl, int thr
 static long long* g_lstm_dbg = nullptr;
 
 extern "C" {
-
-// tuning knob (A/B measurements): batch tile of the small-H plan (8 or 32)
-int mmda_lstm_set_small_tile(int bt) {
-  MMDA_REQUIRE(bt == 8 || bt == 32, "lstm: small-H batch tile must be 8 or 32");
-  g_small_bt = bt;
-  return MMDA_OK;
-}
 
 // profiling aid: when set (device buffer of >= 8*Tmax int64), CTA 0 of the NEXT forward launches
 // records clock64() at the phase boundaries of every step

@@ -669,21 +669,18 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
           const int e = mxb == 0u ? 0 : min(120, max(-120, 129 - (int)((mxb >> 23) & 0xffu)));
           const float unscale = ldexpf(1.f, -11 - e);
           float* dst = part + (((size_t)k * 2 + (s & 1)) * S + r) * slab;
+          // not unrolled: keeps the kernel at 120 registers
+#pragma unroll 1
           for (int mt = 0; mt < MT; ++mt) {
             const int j = mt * 128 + q * 32 + lane;
             uint32_t v0[8], v1[8];
             const uint32_t col = (uint32_t)(k * MT + mt) * BSUB;
-            if (!(p.save & 2)) {
-              tmem_ld8(tmD + lane_sel + col, v0);
-              tmem_ld8(tmD + lane_sel + col + 8, v1);
-              tmem_wait_ld();
-            } else {
-#pragma unroll
-              for (int jj = 0; jj < 8; ++jj) { v0[jj] = 0u; v1[jj] = 0u; }
-            }
+            tmem_ld8(tmD + lane_sel + col, v0);
+            tmem_ld8(tmD + lane_sel + col + 8, v1);
+            tmem_wait_ld();
             // plain (weak) stores: the release of the tick below publishes them
             float* dj = dst + min(j, H - 1);
-            const bool ok = j < H && !(p.save & 1);
+            const bool ok = j < H;
 #pragma unroll
             for (int jj = 0; jj < 8; ++jj) {
               if (ok && jj < n_prev) dj[(size_t)jj * XLD] = __uint_as_float(v0[jj]) * unscale;
@@ -757,7 +754,7 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
           rec[i] = false;
           ct[i] = 0.f; cp[i] = 0.f; dh[i] = 0.f;
           gt[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (act[i] && !(p.save & 16)) {
+          if (act[i]) {
             gt[i] = pre_g[slot];
             ct[i] = pre_f[slot];
             const bool hp = dir == 0 ? (t >= 1) : (t + 1 < len_c[k][i]);
@@ -765,8 +762,6 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
             if (p.dy) dh[i] = pre_f[2 * BWD_CELLS + slot];
             const bool fin = dir == 0 ? (t == len_c[k][i] - 1) : (t == 0);
             if (fin && p.dutt) dh[i] += p.dutt[(size_t)orig_c[k][i] * p.utt_ld + utt_off + u];
-            rec[i] = dir == 0 ? (t + 1 < len_c[k][i]) : (t >= 1);
-          } else if (act[i]) {
             rec[i] = dir == 0 ? (t + 1 < len_c[k][i]) : (t >= 1);
           }
         }
@@ -783,7 +778,7 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
             const int n = warp + 8 * i;
 #pragma unroll
             for (int rr = 0; rr < 12; ++rr)
-              v[i][rr] = (act[i] && rec[i] && rr < S && !(p.save & 4)) ? __ldcg(src + (size_t)rr * slab + (size_t)n * XLD) : 0.f;
+              v[i][rr] = (act[i] && rec[i] && rr < S) ? __ldcg(src + (size_t)rr * slab + (size_t)n * XLD) : 0.f;
           }
 #pragma unroll
           for (int i = 0; i < 2; ++i) {
@@ -854,7 +849,7 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
         // the GEMM operand copy of d(gates): nobody inside this launch waits for it
 #pragma unroll
         for (int i = 0; i < 2; ++i)
-          if (act[i] && !(p.save & 8))
+          if (act[i])
             *reinterpret_cast<float4*>(p.gates + (size_t)(off_t + b_base + k * BSUB + warp + 8 * i) * H8 + gcol) = dgv[i];
       }
   }
@@ -887,8 +882,7 @@ struct TclPlan {
   size_t smem_fwd, smem_bwd, flag_off, xch_off, total;
 };
 
-int g_tcl_max_ctas = 120;   // upper bound on the SMs one launch occupies
-int g_tcl_fwd_rows = TCL_N; // largest forward batch tile (A/B knob: 48 -> 6 tiles / 120 CTAs at B = 256)
+constexpr int TCL_MAX_CTAS = 120;   // upper bound on the SMs one launch occupies
 
 int tcl_make_plan(int B, int H, int Tmax, TclPlan* pl) {
   if (H <= 128 || H > 320 || B <= 0) return MMDA_ERR_UNSUPPORTED;
@@ -899,7 +893,7 @@ int tcl_make_plan(int B, int H, int Tmax, TclPlan* pl) {
   // A time step is a latency chain (MMA -> cell update -> L2 exchange), not SM-bound work: the
   // fewest tiles that cover the batch, spread evenly over the rounds.
   auto tiles = [&](int rows_max, int S, int* BT, int* NT, int* G) {
-    int Gmax = g_tcl_max_ctas / (2 * S);
+    int Gmax = TCL_MAX_CTAS / (2 * S);
     if (Gmax < 1) Gmax = 1;
     int nt = (B + rows_max - 1) / rows_max;
     *BT = (B + nt - 1) / nt;
@@ -908,7 +902,7 @@ int tcl_make_plan(int B, int H, int Tmax, TclPlan* pl) {
     *G = (*NT + rounds - 1) / rounds;
   };
   pl->S = (H + TCL_UNITS - 1) / TCL_UNITS;
-  tiles(g_tcl_fwd_rows < TCL_N ? g_tcl_fwd_rows : TCL_N, pl->S, &pl->BT, &pl->NT, &pl->G);
+  tiles(TCL_N, pl->S, &pl->BT, &pl->NT, &pl->G);
   // backward: the whole W^T slice (two fp16 terms, MT tiles of 2U columns) + the accumulators
   // (3 sub-tiles x MT tiles x 16 columns) must fit the 512 TMEM columns; U even
   int Sb = pl->S, Ub = 0;
@@ -935,7 +929,6 @@ int tcl_make_plan(int B, int H, int Tmax, TclPlan* pl) {
 }
 
 long long* g_tcl_dbg = nullptr;
-int g_tcl_dbg_flags = 0;    // timing experiments only (results become wrong): see mmda_lstm_tc_set_debug_flags
 int g_tcl_plan_bwd = 0;     // mmda_lstm_tc_plan reports the backward decomposition when set
 
 }  // namespace
@@ -971,26 +964,6 @@ int mmda_lstm_tc_plan(int B, int H, int Tmax, int* out8) {
 // ({slices, groups, batch tile, tiles, units per CTA, smem fwd, smem bwd, CTAs})
 int mmda_lstm_tc_plan_select(int backward) {
   g_tcl_plan_bwd = backward != 0;
-  return MMDA_OK;
-}
-
-// upper bound on the CTAs (= SMs) one launch may occupy
-int mmda_lstm_tc_set_fwd_rows(int rows) {
-  MMDA_REQUIRE(rows >= 16 && rows <= TCL_N, "lstm_tc_set_fwd_rows: %d (16..%d)", rows, TCL_N);
-  g_tcl_fwd_rows = rows;
-  return MMDA_OK;
-}
-
-int mmda_lstm_tc_set_max_ctas(int n) {
-  MMDA_REQUIRE(n >= 2 && n <= 1024, "lstm_tc: max CTAs must be in [2, 1024]");
-  g_tcl_max_ctas = n;
-  return MMDA_OK;
-}
-
-// timing experiments on the backward kernel (the results become WRONG): bit 0 = writers skip their
-// stores, bit 1 = writers skip the TMEM loads, bit 2 = cells skip the partial loads
-int mmda_lstm_tc_set_debug_flags(int flags) {
-  g_tcl_dbg_flags = flags;
   return MMDA_OK;
 }
 
@@ -1064,7 +1037,6 @@ int mmda_lstm_tc_backward(float* gates, const float* whh_f, const float* whh_r, 
   a.gates = gates; a.whh[0] = whh_f; a.whh[1] = whh_r; a.c = const_cast<float*>(c);
   a.dy = dy; a.dutt = dutt; a.utt_ld = utt_ld; a.utt_off0 = utt_off_f; a.utt_off1 = utt_off_r;
   a.lens = lens_sorted; a.sorted_idx = sorted_idx; a.offsets = offsets;
-  a.save = g_tcl_dbg_flags;
   return tcl_launch(true, a, B, H, Tmax, ws, stream);
 }
 

@@ -13,7 +13,6 @@ PyTorch is used for device memory, streams and (in the trainer) ``torch.distribu
 """
 from __future__ import annotations
 
-import os
 from typing import Dict, Optional
 
 import torch
@@ -30,15 +29,10 @@ LN_EPS = 1e-5
 ATT_P = 0.1            # nn.TransformerEncoderLayer default dropout (reference src/models.py:160)
 NHEAD = 2
 TL = "transformer_encoder.layers.0."
-# stream priorities (text chain, visual/acoustic chains, weight-gradient leaves); lower = sooner
-# (measured, tools/exp_prio.sh: the three encoder chains at equal priority above the leaves: 4.54 ms;
-# text above the side chains 4.64; everything equal 4.60)
-_PRIO = tuple(int(x) for x in os.environ.get("MMDA_PRIO", "-1,-1,0").split(","))
-# side BPTT layer 2 / layer 1 gate against the text BPTT launch: "pre" = wait until the text stream
-# has reached its launch point (4.54 ms), "done" = until it has completed (4.87), "none" (4.56)
-_ORDER = os.environ.get("MMDA_ORDER", "pre,pre").split(",")
+# stream priorities; lower = sooner.  Measured: the three encoder chains at equal priority above
+# the weight-gradient leaves 4.54 ms/step; text above the side chains 4.64; everything equal 4.60
+PRIO_TEXT, PRIO_SIDE, PRIO_LEAF = -1, -1, 0
 _DRYRUN = False       # tests only: exercise the host orchestration on CPU with a stubbed library
-_DRYRUN_SIMT_ONLY = False
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -51,7 +45,7 @@ class Kernels:
     def __init__(self):
         self.stream = None
         self.launches = 0
-        self.leaf_on = False            # set by the engine's backward (multi-stream mode)
+        self.leaf_on = False            # set by the engine's backward
         self._leaf_streams, self._leaf_used = {}, {}
 
     def bind_stream(self):
@@ -99,7 +93,7 @@ class Kernels:
         cur = torch.cuda.current_stream()
         st = self._leaf_streams.get(cur.cuda_stream)
         if st is None:
-            st = self._leaf_streams[cur.cuda_stream] = torch.cuda.Stream(device=cur.device, priority=_PRIO[2])
+            st = self._leaf_streams[cur.cuda_stream] = torch.cuda.Stream(device=cur.device, priority=PRIO_LEAF)
         ev = torch.cuda.Event()
         ev.record(cur)
         st.wait_event(ev)
@@ -181,38 +175,20 @@ class MisaEngine:
         self._dev = None
         self.seed = 0x5EED
         self.step_id = 0
-        import os
         prec = getattr(self.cfg, "precision", "fp32")
         if prec not in ("fp32", "bf16"):
             raise ValueError(f"precision must be 'fp32' or 'bf16', got {prec!r}")
-        # hoisted LSTM GEMMs: tcgen05 path (3xTF32 in fp32 mode, bf16 operands in bf16 mode) where
-        # the operand pitches satisfy TMA's 16-byte rule, exact-fp32 SIMT path otherwise
         # precision="bf16" selects bf16 operands for the BERT text encoder's GEMMs only (C4).  The
         # hoisted LSTM GEMMs always run 3xTF32 (fp32-accurate): a bf16 input projection moved this
         # model's text-encoder gradients by 5-15 % (measured round 1) and gained nothing once the
         # recurrence itself ran on tensor cores, so that mode was removed (DESIGN.md section 3.2).
         self.tc_kind = 0 if prec == "fp32" else 1
-        self.lstm_kind = 0
-        # 3xTF32 operands: activations are plain fp32 tensors, split into tf32 hi/lo inside the
-        # GEMM kernel's shared-memory pipeline; weights (re-read by every tile) are split once
-        self.use_tc = os.environ.get("MMDA_GEMM", "tc") != "simt"
-        self.tc_small = os.environ.get("MMDA_GEMM_SMALL", "tc") != "simt"
         # the visual / acoustic encoders run on side streams next to the text encoder (whose
-        # cluster kernel occupies 112 of the 148 SMs)
-        self.multi_stream = os.environ.get("MMDA_STREAMS", "1") != "0"
+        # recurrence occupies up to 120 of the 148 SMs)
         self._side = None
         self._text_stream = None
+        self._order_events = {}
         self.fork_log = None
-        if "MMDA_LSTM_SMALL_TILE" in os.environ and not _DRYRUN:      # A/B knob
-            LIB.call("mmda_lstm_set_small_tile", int(os.environ["MMDA_LSTM_SMALL_TILE"]))
-        self.text_priority = os.environ.get("MMDA_TEXT_PRIORITY", "1") != "0"
-        # large hidden sizes (text, H = 300): tensor-core recurrence (csrc/lstm_tc.cu) instead of
-        # the SIMT cluster kernel; MMDA_LSTM_TC=0 keeps the SIMT path (A/B measurements)
-        self.lstm_tc = os.environ.get("MMDA_LSTM_TC", "1") != "0"
-        if "MMDA_LSTM_TC_CTAS" in os.environ and not _DRYRUN:
-            LIB.call("mmda_lstm_tc_set_max_ctas", int(os.environ["MMDA_LSTM_TC_CTAS"]))
-        if "MMDA_LSTM_TC_FWD_ROWS" in os.environ and not _DRYRUN:
-            LIB.call("mmda_lstm_tc_set_fwd_rows", int(os.environ["MMDA_LSTM_TC_FWD_ROWS"]))
         # use_bert=True (SURVEY.md 8f N1): the BERT encoder runs on the hand-written kernels too
         # (mmda_b200/bert.py); its masked-mean output enters here as `utt_text` and backward()
         # returns the gradient wrt it.
@@ -321,23 +297,17 @@ class MisaEngine:
         self._pack_key = key
         return self._pack_info
 
-    # ---------------------------------------------------------------- GEMM routing ---------
-    def big_gemm(self, *a, **kw):
-        """Hoisted LSTM GEMMs on the exact-fp32 SIMT kernel (MMDA_GEMM=simt / MMDA_GEMM_SMALL=simt
-        A/B runs; the default routes them to the tcgen05 3xTF32 kernel)."""
-        self.k.gemm(*a, **kw)
-
     # ---------------------------------------------------------------- streams --------------
     def _side_streams(self):
         if self._side is None:
-            self._side = {m: torch.cuda.Stream(device=self._dev, priority=_PRIO[1]) for m in ("v", "a")}
+            self._side = {m: torch.cuda.Stream(device=self._dev, priority=PRIO_SIDE) for m in ("v", "a")}
         return self._side
 
     def _wgrad_stream(self, m):
         if not hasattr(self, "_wg"):
             self._wg = {}
         if m not in self._wg:
-            self._wg[m] = torch.cuda.Stream(device=self._dev, priority=_PRIO[2])
+            self._wg[m] = torch.cuda.Stream(device=self._dev, priority=PRIO_LEAF)
         return self._wg[m]
 
     def _mark(self, tag):
@@ -351,8 +321,9 @@ class MisaEngine:
         """Run fns[m]() for m in v, a on side streams (after everything enqueued so far on the
         current stream) and fns['t']() on the text stream; join before returning.  With
         ``text_first`` the text function is enqueued first, so the side streams can wait on events
-        it recorded (`_order_events`)."""
-        if not self.multi_stream or _DRYRUN:
+        it recorded (`_order_events`).  The CPU dry run enqueues the same functions in that order
+        on one stream."""
+        if _DRYRUN:
             for m in (("t", "v", "a") if text_first else ("v", "a", "t")):
                 fns[m]()
             return
@@ -379,23 +350,19 @@ class MisaEngine:
         def run_text():
             # the text encoder is the critical path: it runs on a high-priority stream so its
             # kernels are placed ahead of the visual / acoustic CTAs competing for SMs
-            if self.text_priority:
-                if self._text_stream is None:
-                    self._text_stream = torch.cuda.Stream(device=self._dev, priority=_PRIO[0])
-                ts = self._text_stream
-                ts.wait_event(start)
-                with torch.cuda.stream(ts):
-                    self.k.bind_stream()
-                    fns["t"]()
-                    ev = torch.cuda.Event(enable_timing=timing)
-                    ev.record(ts)
-                    done.append(ev)
-                    if timing:
-                        self.fork_log.append(("t", ev))
-                self.k.bind_stream()
-            else:
+            if self._text_stream is None:
+                self._text_stream = torch.cuda.Stream(device=self._dev, priority=PRIO_TEXT)
+            ts = self._text_stream
+            ts.wait_event(start)
+            with torch.cuda.stream(ts):
                 self.k.bind_stream()
                 fns["t"]()
+                ev = torch.cuda.Event(enable_timing=timing)
+                ev.record(ts)
+                done.append(ev)
+                if timing:
+                    self.fork_log.append(("t", ev))
+            self.k.bind_stream()
 
         if text_first:
             run_text()
@@ -408,15 +375,11 @@ class MisaEngine:
             main.wait_event(ev)
 
     # ---------------------------------------------------------------- tensor-core operands --
-    def _tc_ok(self, H, I):
-        """The hoisted LSTM GEMMs run on tcgen05 for every hidden size: operands whose natural
-        pitch breaks TMA's 16-byte rule (visual 35 / 70, acoustic 74 floats) live in buffers with
-        the pitch rounded up to 4 floats (`pbuf`); the pad columns are never read (the tensor
-        maps carry the true extents).  MMDA_GEMM_SMALL=simt keeps the old SIMT routing."""
-        return self.use_tc and (self.tc_small or (H % 4 == 0 and I % 4 == 0))
-
     def pbuf(self, name, rows, cols):
-        """(rows, cols) view of a workspace buffer whose row pitch is cols rounded up to 4 floats."""
+        """(rows, cols) view of a workspace buffer whose row pitch is cols rounded up to 4 floats.
+        The hoisted LSTM GEMMs run on tcgen05 for every hidden size: operands whose natural pitch
+        breaks TMA's 16-byte rule (visual 35 / 70, acoustic 74 floats) live in such buffers; the
+        pad columns are never read (the tensor maps carry the true extents)."""
         ld = (cols + 3) // 4 * 4
         return self.buf(name, rows, ld)[:, :cols]
 
@@ -455,19 +418,15 @@ class MisaEngine:
         ld = (cols + 7) // 8 * 8
         return self.buf(name + "_bf", rows, ld, dtype=torch.bfloat16)[:, :cols], None
 
-    def _pack_weights(self, r, P, H, I, kind, want_bias=True):
-        """Stacked gate-interleaved copy of layer r's W_ih (both directions) for GEMM kind
-        `kind` (-1: plain fp32 for the SIMT path, 0: tf32 hi/lo, 1: bf16) + the bias stack."""
-        mode = {-1: 0, 0: 1, 1: 2}[kind]
-        if kind == -1:
-            W = (self.buf(f"Wst_{r}", 8 * H, I), None)
-        else:
-            W = self._prep_buf(f"tcW_{r}", 8 * H, I, kind, split=True)
-        bst = self.buf(f"bst_{r}", 8 * H) if want_bias else None
+    def _pack_weights(self, r, P, H, I):
+        """Stacked gate-interleaved copy of layer r's W_ih (both directions), split into tf32
+        hi/lo for the 3xTF32 GEMMs (pack mode 1), + the bias stack."""
+        W = self._prep_buf(f"tcW_{r}", 8 * H, I, 0, split=True)
+        bst = self.buf(f"bst_{r}", 8 * H)
         self.k._c("mmda_lstm_pack_weights", _ptr(P[f"{r}.weight_ih_l0"]),
                   _ptr(P[f"{r}.weight_ih_l0_reverse"]), _ptr(P[f"{r}.bias_ih_l0"]),
                   _ptr(P[f"{r}.bias_hh_l0"]), _ptr(P[f"{r}.bias_ih_l0_reverse"]),
-                  _ptr(P[f"{r}.bias_hh_l0_reverse"]), H, I, mode, _ptr(W[0]), _ptr(W[1]),
+                  _ptr(P[f"{r}.bias_hh_l0_reverse"]), H, I, 1, _ptr(W[0]), _ptr(W[1]),
                   W[0].stride(0), _ptr(bst))
         return W, bst
 
@@ -496,7 +455,7 @@ class MisaEngine:
 
     # ---- dense layers big enough for the tensor-core path (the fusion layer's FFN) ----
     def _tc_lin_ok(self, M, N, K):
-        return self.use_tc and not _DRYRUN_SIMT_ONLY and M >= 512 and N % 4 == 0 and K % 4 == 0
+        return M >= 512 and N % 4 == 0 and K % 4 == 0
 
     def tc_linear(self, tag, x, w, b, out):
         """out = x w^T + b on tcgen05 (3xTF32: fp32-accurate in either precision mode)."""
@@ -526,7 +485,7 @@ class MisaEngine:
     def _lstm_tc_ws(self, m, B, H, Tmax):
         """Workspace of the tensor-core recurrence for modality m, or None when that path does
         not cover (B, H) -- small hidden sizes and GRU cells stay on the SIMT kernels."""
-        if not self.lstm_tc or self.gru or _DRYRUN:
+        if self.gru or _DRYRUN:
             return None
         nbytes = LIB.raw("mmda_lstm_tc_workspace_bytes")(B, H, Tmax)
         if nbytes <= 0:
@@ -567,14 +526,10 @@ class MisaEngine:
                 k.layernorm(Y1, None, P[f"{ln}.weight"], P[f"{ln}.bias"], Y1n, mu, rs)
             I = Xin.shape[1]
             # both directions in ONE GEMM against the stacked, gate-interleaved weight copy:
-            # G[N][2][H][4] = Xin * Wst^T + (b_ih + b_hh)
-            if self._tc_ok(H, I):
-                Wst, bst = self._pack_weights(r, P, H, I, self.lstm_kind)
-                Xp = self._prep(f"tcX_{r}", Xin, kind=self.lstm_kind)
-                k.gemm_tc(self.lstm_kind, 0, 0, N, 8 * H, I, Xp, Wst, G, bias=bst)
-            else:
-                Wst, bst = self._pack_weights(r, P, H, I, -1)
-                self.big_gemm(Xin, Wst[0], G, tb=True, bias=bst)
+            # G[N][2][H][4] = Xin * Wst^T + (b_ih + b_hh), 3xTF32 in either precision mode
+            Wst, bst = self._pack_weights(r, P, H, I)
+            Xp = self._prep(f"tcX_{r}", Xin, kind=0)
+            k.gemm_tc(0, 0, 0, N, 8 * H, I, Xp, Wst, G, bias=bst)
             Y, C = (Y1, C1) if r == r1 else (Y2, C2)
             o_f, o_r = (0, 2 * H) if r == r1 else (H, 3 * H)
             if m == "t":
@@ -586,7 +541,7 @@ class MisaEngine:
                      int(train))
                 continue
             tcws = self._lstm_tc_ws(m, B, H, Tmax)
-            if self.multi_stream and not _DRYRUN and r == r1 and self._fwd_order is not None:
+            if not _DRYRUN and r == r1 and self._fwd_order is not None:
                 # The text recurrence launches cooperatively (every CTA resident at once): the
                 # small visual / acoustic recurrences must not grab SMs just before it.  They
                 # wait for the point where the text stream reaches its own layer-1 launch; all
@@ -674,7 +629,7 @@ class MisaEngine:
             return run
 
         self.saved = dict(pk=pk, sent=sent, X=X, train=train, srcs=srcs)
-        self._fwd_order = [] if (self.lstm_tc and not self.gru and not self.use_bert) else None
+        self._fwd_order = [] if (not self.gru and not self.use_bert) else None
         self._fork({"t": enc_text, "v": enc_side("v"), "a": enc_side("a")},
                    text_first=self._fwd_order is not None)
         self._fwd_order = None
@@ -852,7 +807,7 @@ class MisaEngine:
         # weight / bias gradients of the dense layers are leaves of the step's dependency graph:
         # they run on side streams (Kernels.leaf) so that only the dx products sit on the chain
         # to the BPTT launches; joined before a data-parallel all-reduce needs them, else at the end
-        k.leaf_on = self.multi_stream and not _DRYRUN
+        k.leaf_on = not _DRYRUN
         k._leaf_used = {}
 
         # ---- classifier / confidence ----
@@ -1031,12 +986,13 @@ class MisaEngine:
         # The text BPTT launches cooperatively on ~120 SMs: if the small visual / acoustic BPTT
         # kernels get there first it has to wait for them to drain (0.3 ms, measured).  So the
         # text stream is enqueued first and the side streams hold each BPTT launch until the text
-        # stream has reached its own launch point of that layer (`_ORDER`): the launches become
-        # eligible together, the text CTAs are placed first (enqueue order) and the small kernels
-        # run on the SMs the text kernel leaves free.  The recurrence kernels clean their exchange
-        # flags themselves, so no memset node sits between that point and the launch.
+        # stream has reached its own launch point of that layer: the launches become eligible
+        # together, the text CTAs are placed first (enqueue order) and the small kernels run on the
+        # SMs the text kernel leaves free (measured 4.54 ms/step; waiting for the text launch to
+        # complete 4.87, no gate 4.56).  The recurrence kernels clean their exchange flags
+        # themselves, so no memset node sits between that point and the launch.
         self._order_events = {}
-        self._fork({m: enc_bwd(m) for m in MODS}, text_first=self.lstm_tc and not self.gru)
+        self._fork({m: enc_bwd(m) for m in MODS}, text_first=not self.gru)
         self._order_events = {}
         k.join_leaves()
         k.leaf_on = False
@@ -1062,7 +1018,7 @@ class MisaEngine:
         scratch = self.buf(f"lstm_scratch_{m}", max(1, nbytes // 4))
         dY1n = self.pbuf(f"dY1n_{m}", N, 2 * H)
         dY1 = self.buf(f"dY1_{m}", N, 2 * H)
-        use_side = self.multi_stream and not _DRYRUN
+        use_side = not _DRYRUN
         cur = torch.cuda.current_stream() if use_side else None
         side_used = []
         G_real = G
@@ -1076,10 +1032,9 @@ class MisaEngine:
                                 G[f"{ln}.bias"])
             tcws = self._lstm_tc_ws(m, B, H, Tmax)
             layer = 2 if r == r2 else 1
-            if use_side and m != "t" and layer in getattr(self, "_order_events", {}):
+            if use_side and m != "t" and layer in self._order_events:
                 cur.wait_event(self._order_events[layer])
-            gate = _ORDER[2 - layer]        # "pre": the launch point, "done": completion, "none"
-            if use_side and m == "t" and tcws is not None and gate == "pre" and hasattr(self, "_order_events"):
+            if use_side and m == "t" and tcws is not None:
                 ev = torch.cuda.Event()
                 ev.record(cur)
                 self._order_events[layer] = ev
@@ -1088,10 +1043,6 @@ class MisaEngine:
                      _ptr(P[f"{r}.weight_hh_l0_reverse"]), _ptr(C), _ptr(dy), _ptr(dutt), 4 * H, o_f,
                      o_r, _ptr(pk["lens"]), _ptr(pk["sidx"]), _ptr(pk["off"]), B, H, Tmax,
                      _ptr(tcws))
-                if use_side and m == "t" and gate == "done" and hasattr(self, "_order_events"):
-                    ev = torch.cuda.Event()
-                    ev.record(cur)
-                    self._order_events[layer] = ev
             else:
                 k._c("mmda_gru_backward" if self.gru else "mmda_lstm_backward", _ptr(Gt),
                      _ptr(P[f"{r}.weight_hh_l0"]), _ptr(P[f"{r}.weight_hh_l0_reverse"]),
@@ -1105,19 +1056,15 @@ class MisaEngine:
             if m == "t":
                 self._mark(f"  t.{r} BPTT done")
             I = Xin.shape[1]
-            tc = self._tc_ok(H, I)
-            if tc:
-                # 3xTF32 like the forward: weight / activation gradients are sums with heavy
-                # cancellation, where bf16 operands cost several percent (measured 4-13 %)
-                dGp = self._prep(f"tcdG_{r}", Gt, kind=0)
-                Xp = self._prep(f"tcX_{r}", Xin, kind=0)          # the fp32 tensor itself
-                Wst = self._prep_buf(f"tcW_{r}", 8 * H, I, 0, split=True)   # packed by the forward
-            else:
-                Wst = (self.buf(f"Wst_{r}", 8 * H, I), None)      # written by the forward
+            # 3xTF32 like the forward: weight / activation gradients are sums with heavy
+            # cancellation, where bf16 operands cost several percent (measured 4-13 %)
+            dGp = self._prep(f"tcdG_{r}", Gt, kind=0)
+            Xp = self._prep(f"tcX_{r}", Xin, kind=0)          # the fp32 tensor itself
+            Wst = self._prep_buf(f"tcW_{r}", 8 * H, I, 0, split=True)   # packed by the forward
 
             hp_box = {}
 
-            def wgrad_common(r=r, Y=Y, tc=tc):
+            def wgrad_common(r=r, Y=Y):
                 if self.gru:
                     for suf in ("", "_reverse"):
                         for kk in self._RNN_KEYS:
@@ -1126,26 +1073,19 @@ class MisaEngine:
                 HP = self.buf(f"HP_{r}", N, 2 * Hp)
                 k._c("mmda_lstm_shift_h", _ptr(Y), _ptr(HP), _ptr(pk["row_t"]), _ptr(pk["row_j"]),
                      _ptr(pk["lens"]), _ptr(pk["off"]), N, H, Hp)
-                hp_box["HP"] = [HP[:, di * Hp:di * Hp + H] for di in (0, 1)]
-                if tc:
-                    hp_box["HPp"] = [self._prep(f"tcHP_{r}_{di}", hp_box["HP"][di], kind=0) for di in (0, 1)]
+                hp_box["HPp"] = [self._prep(f"tcHP_{r}_{di}", HP[:, di * Hp:di * Hp + H], kind=0)
+                                 for di in (0, 1)]
 
-            def wgrad_dir(di, r=r, Gt=Gt, Xin=Xin, tc=tc, I=I):
+            def wgrad_dir(di, r=r, Gt=Gt, I=I):
                 # dG columns are gate-interleaved (u*4+g): c_ilv=H stores row u*4+g at g*H+u
                 suf = ("", "_reverse")[di]
-                HP = hp_box["HP"]
                 dG = Gt[:, di * 4 * H:(di + 1) * 4 * H]
-                if tc:   # contract over tokens: both operands MN-major, auto split-K
-                    dGd = self._cols(dGp, di * 4 * H, (di + 1) * 4 * H)
-                    k.gemm_tc(0, 1, 1, 4 * H, I, N, dGd, Xp, G[f"{r}.weight_ih_l0{suf}"], mode=1,
-                              split_k=0, c_ilv=H)
-                    k.gemm_tc(0, 1, 1, 4 * H, H, N, dGd, hp_box["HPp"][di],
-                              G[f"{r}.weight_hh_l0{suf}"], mode=1, split_k=0, c_ilv=H)
-                else:
-                    self.big_gemm(dG, Xin, G[f"{r}.weight_ih_l0{suf}"], ta=True, beta=1.0,
-                                  split_k=0, c_ilv=H)
-                    self.big_gemm(dG, HP[di], G[f"{r}.weight_hh_l0{suf}"],
-                                  ta=True, beta=1.0, split_k=0, c_ilv=H)
+                # contract over tokens: both operands MN-major, auto split-K
+                dGd = self._cols(dGp, di * 4 * H, (di + 1) * 4 * H)
+                k.gemm_tc(0, 1, 1, 4 * H, I, N, dGd, Xp, G[f"{r}.weight_ih_l0{suf}"], mode=1,
+                          split_k=0, c_ilv=H)
+                k.gemm_tc(0, 1, 1, 4 * H, H, N, dGd, hp_box["HPp"][di],
+                          G[f"{r}.weight_hh_l0{suf}"], mode=1, split_k=0, c_ilv=H)
                 k.colsum(dG, G[f"{r}.bias_ih_l0{suf}"], G[f"{r}.bias_hh_l0{suf}"], ilv=H)
                 if self.gru:     # 4-slot gradients -> the (3H, .) parameters' gradients
                     k._c("mmda_gru_fold_grads", *[_ptr(G[f"{r}.{kk}{suf}"]) for kk in self._RNN_KEYS],
@@ -1186,10 +1126,8 @@ class MisaEngine:
                 wgrad_dir(1)
             if r == r2 or m == "t":
                 dX = dY1n if r == r2 else self.buf("dX_t", N, H)
-                if tc:   # dX = dG [N x 8H] * [W_ih ; W_ih_reverse] (stored [8H][I]: MN-major B)
-                    k.gemm_tc(0, 0, 1, N, I, 8 * H, dGp, Wst, dX)
-                else:
-                    self.big_gemm(Gt, Wst[0], dX)
+                # dX = dG [N x 8H] * [W_ih ; W_ih_reverse] (stored [8H][I]: MN-major B)
+                k.gemm_tc(0, 0, 1, N, I, 8 * H, dGp, Wst, dX)
                 if m == "t":
                     self._mark(f"  t.{r} dX GEMM done")
                 if r == r1:

@@ -15,8 +15,6 @@ from __future__ import annotations
 
 from typing import Dict, List, Optional, Tuple
 
-import os
-
 import torch
 
 from ._lib import LIB, MmdaError
@@ -179,11 +177,8 @@ class FusedTrainer:
         if not _engine._DRYRUN:
             self.eng.k.bind_stream()
             self.eng.k._c("mmda_step_state_init", _ptr(self.state), 0, 0.9, 0.999)
-        # CUDA-graph replay of the whole step (single GPU, repeated sequence-length pattern)
-        import os
-        self.use_graph = (use_graph if use_graph is not None else
-                          os.environ.get("MMDA_GRAPH", "1") != "0") and \
-            (self.world == 1 or os.environ.get("MMDA_GRAPH_DP", "1") == "1")
+        # CUDA-graph replay of the whole step (single GPU and data parallel)
+        self.use_graph = use_graph if use_graph is not None else True
         self._graphs = {}               # key -> captured step (see step())
         self._graphs_ws = self._graphs_alias = None
         self._graphs_slots = -1
@@ -389,7 +384,7 @@ class FusedTrainer:
     # the end of the step, 0.2 ms exposed).  Encoder-phase notifications only record an event; the
     # all-reduces are issued after the backward has been enqueued, in completion order, from a
     # helper stream that waits for exactly those events.
-    _ISSUE_ORDER = tuple(os.environ.get("MMDA_AR_ORDER", "enc_a,enc_v,embed,enc_t_l2,enc_t").split(","))
+    _ISSUE_ORDER = ("enc_a", "enc_v", "embed", "enc_t_l2", "enc_t")
 
     def _on_ready(self, tag):
         if self.world == 1 or (tag == "enc_t" and self.use_bert and not self._bert_done):
@@ -454,7 +449,7 @@ class FusedTrainer:
         # the gradient arena (43 MB with a 20k-word embedding) is cleared on a side stream under
         # the forward instead of on the chain between the classifier and the losses
         zero_ev = None
-        if eng.multi_stream and not _engine._DRYRUN and os.environ.get("MMDA_ZERO_SIDE", "1") != "0":
+        if not _engine._DRYRUN:
             cur = torch.cuda.current_stream()
             if not hasattr(self, "_zero_stream"):
                 self._zero_stream = torch.cuda.Stream(device=self.g_arena.device)
@@ -467,7 +462,7 @@ class FusedTrainer:
                 zero_ev.record(self._zero_stream)
         early = {}
         hook = None
-        if eng.multi_stream and not _engine._DRYRUN and os.environ.get("MMDA_LOSS_EARLY", "1") != "0":
+        if not _engine._DRYRUN:
             def hook():
                 early["ev"] = self._loss_early(int(lengths.numel()))
         out = eng.forward(sentences, visual, acoustic, lengths, train=True, want_sp=False,
@@ -646,7 +641,7 @@ class FusedTrainer:
 
     def step(self, sentences, visual, acoustic, lengths, labels, bert_sent=None,
              bert_sent_type=None, bert_sent_mask=None):
-        """One optimisation step.  With ``use_graph`` (default on one GPU) the kernel sequence of
+        """One optimisation step.  With ``use_graph`` (the default) the kernel sequence of
         a repeated (shapes, lengths) pattern is captured once into a CUDA graph -- multi-stream
         forks included -- and replayed; per-step scalars, the learning rate included, live in
         ``self.state`` on the device, so changing ``self.lr`` between steps keeps the graph."""

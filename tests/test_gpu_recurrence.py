@@ -183,21 +183,6 @@ def test_dy_null_equals_dy_zero(cell, H, B, T, report):
     assert same_bits(D.run(c, "simt", fill=NAN)["dG"], o["dG"])
 
 
-@pytest.mark.parametrize("cell", ["lstm", "gru"])
-def test_small_tile_knob(cell, report):
-    """mmda_lstm_set_small_tile(8): the small-H plan for B >= 64 takes 8-row tiles."""
-    knob = plan(64, 35)[0][1]      # the knob in force (no getter): 32 -> BT 32, 8 -> BT 8
-    try:
-        lib().call("mmda_lstm_set_small_tile", 8)
-        case = ("small_tile_8", 35, 70, 9, 1, None, 0, False, (1, 8, 4))
-        c = make(case, cell)
-        assert plan(c["B"], c["H"])[0] == (1, 8, 4)
-        check(c, case[0], report)
-    finally:
-        lib().call("mmda_lstm_set_small_tile", knob)
-    assert plan(64, 35)[0][1] == knob
-
-
 @pytest.mark.parametrize("B", [8, 64])
 @pytest.mark.parametrize("H", [115, 116])
 @pytest.mark.parametrize("cell", ["lstm", "gru"])
