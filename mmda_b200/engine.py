@@ -13,6 +13,7 @@ PyTorch is used for device memory, streams and (in the trainer) ``torch.distribu
 """
 from __future__ import annotations
 
+import contextlib
 from typing import Dict, Optional
 
 import torch
@@ -39,21 +40,81 @@ def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else t.data_ptr()
 
 
+_HERE = object()       # Kernels.side(after=...) default: wait on the current stream
+
+
 class Kernels:
-    """Thin typed wrappers: torch tensors in, C-ABI calls out (all on one stream)."""
+    """Thin typed wrappers: torch tensors in, C-ABI calls out, on the stream ``bind_stream`` or
+    ``side`` bound.  ``side`` / ``mark`` / ``wait`` are the only code that creates side streams,
+    records or waits on events: one stream per (device, role), created on first use."""
 
     def __init__(self):
         self.stream = None
         self.launches = 0
         self.leaf_on = False            # set by the engine's backward
-        self._leaf_streams, self._leaf_used = {}, {}
+        self._leaf_used = {}            # leaf role -> None, in first-use order since the last join
+        self._role = None               # role of the stream `side` runs on; None: the caller's
+        self._streams = {}
 
     def bind_stream(self):
-        self.stream = 0 if _DRYRUN else torch.cuda.current_stream().cuda_stream
+        # the CPU dry run binds the role name, so that a stubbed library sees where launches go
+        if _DRYRUN:
+            self.stream = 0 if self._role is None else self._role
+        else:
+            self.stream = torch.cuda.current_stream().cuda_stream
 
     def _c(self, name, *args):
         self.launches += 1
         LIB.call(name, *args, self.stream)
+
+    def _stream(self, role, priority=0, device=None):
+        key = (torch.cuda.current_device() if device is None else device, role)
+        st = self._streams.get(key)
+        if st is None:
+            st = self._streams[key] = torch.cuda.Stream(device=key[0], priority=priority)
+        return st
+
+    def mark(self, role=None):
+        """Event at the current point of the current stream, or with ``role`` at the end of what
+        ``side(role)`` blocks have enqueued so far.  None in the dry run."""
+        if _DRYRUN:
+            return None
+        return (torch.cuda.current_stream() if role is None else self._stream(role)).record_event()
+
+    def wait(self, *events):
+        """Order the current stream after the events (None: nothing to wait for)."""
+        events = [ev for ev in events if ev is not None]
+        if events:
+            cur = torch.cuda.current_stream()
+            for ev in events:
+                cur.wait_event(ev)
+
+    @contextlib.contextmanager
+    def side(self, role, priority=0, after=_HERE):
+        """Run the block on ``role``'s stream of the current device, ordered after the current
+        point of the current stream, or after the events ``after`` only.  Launches and torch
+        operations in the block go to that stream; the caller's binding comes back on exit.  The
+        dry run creates no stream: it runs the block inline with the role name bound."""
+        prev = self._role, self.stream
+        ctx = contextlib.nullcontext()
+        if _DRYRUN:
+            stream = role
+        else:
+            cur = torch.cuda.current_stream()
+            st = self._stream(role, priority, cur.device_index)
+            if after is _HERE:
+                st.wait_stream(cur)
+            else:
+                for ev in after:
+                    if ev is not None:
+                        st.wait_event(ev)
+            ctx, stream = torch.cuda.stream(st), st.cuda_stream
+        try:
+            with ctx:
+                self._role, self.stream = role, stream
+                yield
+        finally:
+            self._role, self.stream = prev
 
     # C = act(alpha * op(A) op(B) + beta*C + bias + bias2); A,B,C are 2-D views with unit inner stride
     def gemm(self, A, B, C, ta=False, tb=False, alpha=1.0, beta=0.0, bias=None, bias2=None,
@@ -87,28 +148,16 @@ class Kernels:
         (weight / bias gradients) -- on a side stream paired with the current one, ordered after
         everything enqueued so far.  `join_leaves()` orders the current stream after all of them.
         The caller guarantees the operands fn reads are not overwritten before the join."""
-        if not self.leaf_on or _DRYRUN:
+        if not self.leaf_on:
             fn()
             return
-        cur = torch.cuda.current_stream()
-        st = self._leaf_streams.get(cur.cuda_stream)
-        if st is None:
-            st = self._leaf_streams[cur.cuda_stream] = torch.cuda.Stream(device=cur.device, priority=PRIO_LEAF)
-        ev = torch.cuda.Event()
-        ev.record(cur)
-        st.wait_event(ev)
-        with torch.cuda.stream(st):
-            self.bind_stream()
+        role = ("leaf", self._role)
+        with self.side(role, PRIO_LEAF):
             fn()
-        self.bind_stream()
-        self._leaf_used[st.cuda_stream] = st
+        self._leaf_used[role] = None
 
     def join_leaves(self):
-        cur = torch.cuda.current_stream() if self._leaf_used else None
-        for st in self._leaf_used.values():
-            ev = torch.cuda.Event()
-            ev.record(st)
-            cur.wait_event(ev)
+        self.wait(*[self.mark(role) for role in self._leaf_used])
         self._leaf_used = {}
 
     def linear_bwd(self, dy, x, w, dw, db, dx=None, dx_beta=0.0, db2=None, dw_split=0):
@@ -168,7 +217,6 @@ class MisaEngine:
         self.NC = self.cfg.num_classes
         self.H = dict(zip(MODS, model.hidden_sizes))
         self._pack_key = None
-        self._fwd_order = None
         self.pad = None                 # (T_pad, Np) while FusedTrainer runs a padded (graph) step
         self._params = None
         self._params_ver = None
@@ -183,12 +231,6 @@ class MisaEngine:
         # model's text-encoder gradients by 5-15 % (measured round 1) and gained nothing once the
         # recurrence itself ran on tensor cores, so that mode was removed (DESIGN.md section 3.2).
         self.tc_kind = 0 if prec == "fp32" else 1
-        # the visual / acoustic encoders run on side streams next to the text encoder (whose
-        # recurrence occupies up to 120 of the 148 SMs)
-        self._side = None
-        self._text_stream = None
-        self._order_events = {}
-        self.fork_log = None
         # use_bert=True (SURVEY.md 8f N1): the BERT encoder runs on the hand-written kernels too
         # (mmda_b200/bert.py); its masked-mean output enters here as `utt_text` and backward()
         # returns the gradient wrt it.
@@ -260,7 +302,7 @@ class MisaEngine:
             raise MmdaError("lengths must stay on the CPU (reference src/solver.py:149)")
         ln = lengths_cpu.to(torch.int64)
         pad = self.pad
-        key = (ln.numel(), tuple(ln.tolist()), pad)
+        key = (ln.numel(), tuple(ln.tolist()), pad, self._dev)
         if key == self._pack_key:
             return self._pack_info
         if ln.numel() == 0 or int(ln.min()) <= 0:
@@ -298,81 +340,19 @@ class MisaEngine:
         return self._pack_info
 
     # ---------------------------------------------------------------- streams --------------
-    def _side_streams(self):
-        if self._side is None:
-            self._side = {m: torch.cuda.Stream(device=self._dev, priority=PRIO_SIDE) for m in ("v", "a")}
-        return self._side
-
-    def _wgrad_stream(self, m):
-        if not hasattr(self, "_wg"):
-            self._wg = {}
-        if m not in self._wg:
-            self._wg[m] = torch.cuda.Stream(device=self._dev, priority=PRIO_LEAF)
-        return self._wg[m]
-
-    def _mark(self, tag):
-        """profiling aid: timestamp on the current stream (tools/fork_timing.py)"""
-        if self.fork_log is not None:
-            ev = torch.cuda.Event(enable_timing=True)
-            ev.record(torch.cuda.current_stream())
-            self.fork_log.append((tag, ev))
-
     def _fork(self, fns, text_first=False):
-        """Run fns[m]() for m in v, a on side streams (after everything enqueued so far on the
-        current stream) and fns['t']() on the text stream; join before returning.  With
-        ``text_first`` the text function is enqueued first, so the side streams can wait on events
-        it recorded (`_order_events`).  The CPU dry run enqueues the same functions in that order
-        on one stream."""
-        if _DRYRUN:
-            for m in (("t", "v", "a") if text_first else ("v", "a", "t")):
+        """Run fns[m]() on modality m's stream, all after everything enqueued so far on the
+        current stream, in the order v, a, t (t, v, a with ``text_first``, so that the side
+        streams can wait on launch points the text function marked); join before returning.
+        The text encoder is the critical path: its stream's priority places its kernels ahead of
+        the visual / acoustic CTAs competing for SMs."""
+        k = self.k
+        start, done = k.mark(), []
+        for m in (("t", "v", "a") if text_first else ("v", "a", "t")):
+            with k.side(m, PRIO_TEXT if m == "t" else PRIO_SIDE, after=(start,)):
                 fns[m]()
-            return
-        main = torch.cuda.current_stream()
-        timing = self.fork_log is not None      # profiling aid (tools/fork_timing.py)
-        start = torch.cuda.Event(enable_timing=timing)
-        start.record(main)
-        done = []
-        if timing:
-            self.fork_log.append(("start", start))
-
-        def run_side():
-            for m, st in self._side_streams().items():
-                st.wait_event(start)
-                with torch.cuda.stream(st):
-                    self.k.bind_stream()
-                    fns[m]()
-                    ev = torch.cuda.Event(enable_timing=timing)
-                    ev.record(st)
-                    done.append(ev)
-                    if timing:
-                        self.fork_log.append((m, ev))
-
-        def run_text():
-            # the text encoder is the critical path: it runs on a high-priority stream so its
-            # kernels are placed ahead of the visual / acoustic CTAs competing for SMs
-            if self._text_stream is None:
-                self._text_stream = torch.cuda.Stream(device=self._dev, priority=PRIO_TEXT)
-            ts = self._text_stream
-            ts.wait_event(start)
-            with torch.cuda.stream(ts):
-                self.k.bind_stream()
-                fns["t"]()
-                ev = torch.cuda.Event(enable_timing=timing)
-                ev.record(ts)
-                done.append(ev)
-                if timing:
-                    self.fork_log.append(("t", ev))
-            self.k.bind_stream()
-
-        if text_first:
-            run_text()
-            run_side()
-            self.k.bind_stream()
-        else:
-            run_side()
-            run_text()
-        for ev in done:
-            main.wait_event(ev)
+            done.append(k.mark(m))
+        k.wait(*done)
 
     # ---------------------------------------------------------------- tensor-core operands --
     def pbuf(self, name, rows, cols):
@@ -503,9 +483,22 @@ class MisaEngine:
             if name.startswith("lstm_tc_ws_") and int(t[0]) != 0:
                 raise MmdaError(f"{name}: a tensor-core recurrence launch timed out waiting for a peer CTA")
 
+    def _launch_gate(self, gate, m, layer, tcws):
+        """The text recurrence launches cooperatively (every CTA resident at once): the small
+        visual / acoustic recurrences of a layer must not grab SMs just before it.  The text
+        stream (enqueued first) marks the point where it reaches its own launch of that layer in
+        ``gate``; the side streams wait for that point, so the launches become eligible together
+        and stream priority puts the text CTAs first."""
+        if m == "t":
+            if tcws is not None:
+                gate[layer] = self.k.mark()
+        else:
+            self.k.wait(gate.get(layer))
+
     # ---------------------------------------------------------------- forward --------------
-    def _encode(self, m, X, pk, train, P):
-        """reference src/models.py:163-180 + :203 for modality m on the packed rows X (N,I)."""
+    def _encode(self, m, X, pk, train, P, gate):
+        """reference src/models.py:163-180 + :203 for modality m on the packed rows X (N,I);
+        ``gate``: the launch points shared with the other modalities (`_launch_gate`)."""
         k, H = self.k, self.H[m]
         r1, r2, ln = ENC[m]
         N, B, Tmax = pk["N"], pk["B"], pk["Tmax"]
@@ -532,8 +525,6 @@ class MisaEngine:
             k.gemm_tc(0, 0, 0, N, 8 * H, I, Xp, Wst, G, bias=bst)
             Y, C = (Y1, C1) if r == r1 else (Y2, C2)
             o_f, o_r = (0, 2 * H) if r == r1 else (H, 3 * H)
-            if m == "t":
-                self._mark(f"  t.{r} in-proj GEMM enqueued-done")
             if self.gru:
                 k._c("mmda_gru_forward", _ptr(G), _ptr(P[f"{r}.weight_hh_l0"]),
                      _ptr(P[f"{r}.weight_hh_l0_reverse"]), _ptr(Y), _ptr(pk["lens"]),
@@ -541,20 +532,8 @@ class MisaEngine:
                      int(train))
                 continue
             tcws = self._lstm_tc_ws(m, B, H, Tmax)
-            if not _DRYRUN and r == r1 and self._fwd_order is not None:
-                # The text recurrence launches cooperatively (every CTA resident at once): the
-                # small visual / acoustic recurrences must not grab SMs just before it.  They
-                # wait for the point where the text stream reaches its own layer-1 launch; all
-                # three launches then become eligible together and stream priority puts the
-                # text CTAs first.
-                cur = torch.cuda.current_stream()
-                if m == "t" and tcws is not None:
-                    ev = torch.cuda.Event()
-                    ev.record(cur)
-                    self._fwd_order.append(ev)
-                elif m != "t":
-                    for ev in self._fwd_order:
-                        cur.wait_event(ev)
+            if r == r1:
+                self._launch_gate(gate, m, 1, tcws)
             if tcws is not None:
                 k._c("mmda_lstm_tc_forward", _ptr(G), _ptr(P[f"{r}.weight_hh_l0"]),
                      _ptr(P[f"{r}.weight_hh_l0_reverse"]), _ptr(Y), _ptr(C), _ptr(pk["lens"]),
@@ -565,8 +544,6 @@ class MisaEngine:
                      _ptr(P[f"{r}.weight_hh_l0_reverse"]), _ptr(Y), _ptr(C), _ptr(pk["lens"]),
                      _ptr(pk["sidx"]), _ptr(pk["off"]), _ptr(utt), 4 * H, o_f, o_r, B, H, Tmax,
                      int(train))
-            if m == "t":
-                self._mark(f"  t.{r} recurrence done")
         return utt
 
     def forward(self, sentences, visual, acoustic, lengths, train: bool, want_sp: bool = True,
@@ -619,20 +596,19 @@ class MisaEngine:
                 return
             k._c("mmda_embedding_forward", _ptr(P["embed.weight"]), _ptr(sent), _ptr(X["t"]),
                  _ptr(pk["row_t"]), _ptr(pk["row_j"]), _ptr(pk["sidx"]), N, B, self.H["t"], V)
-            utt["t"] = self._encode("t", X["t"], pk, train, P)
+            utt["t"] = self._encode("t", X["t"], pk, train, P, gate)
 
         def enc_side(m):
             def run():
                 k._c("mmda_gather_rows", _ptr(srcs[m]), _ptr(X[m]), X[m].stride(0), _ptr(pk["row_t"]),
                      _ptr(pk["row_j"]), _ptr(pk["sidx"]), N, B, self.H[m])
-                utt[m] = self._encode(m, X[m], pk, train, P)
+                utt[m] = self._encode(m, X[m], pk, train, P, gate)
             return run
 
         self.saved = dict(pk=pk, sent=sent, X=X, train=train, srcs=srcs)
-        self._fwd_order = [] if (not self.gru and not self.use_bert) else None
+        gate = {}
         self._fork({"t": enc_text, "v": enc_side("v"), "a": enc_side("a")},
-                   text_first=self._fwd_order is not None)
-        self._fwd_order = None
+                   text_first=not self.gru and not self.use_bert)
 
         # ---- heads: project -> private/shared -> recon (src/models.py:254-279) ----
         A = self.buf("A", 3, B, d)             # activation output (pre-LN)
@@ -807,7 +783,7 @@ class MisaEngine:
         # weight / bias gradients of the dense layers are leaves of the step's dependency graph:
         # they run on side streams (Kernels.leaf) so that only the dx products sit on the chain
         # to the BPTT launches; joined before a data-parallel all-reduce needs them, else at the end
-        k.leaf_on = not _DRYRUN
+        k.leaf_on = True
         k._leaf_used = {}
 
         # ---- classifier / confidence ----
@@ -979,7 +955,7 @@ class MisaEngine:
         def enc_bwd(m):
             def run():
                 if not (m == "t" and self.use_bert):
-                    self._encode_backward(m, dutt[m], G, pk, P, notify)
+                    self._encode_backward(m, dutt[m], G, pk, P, notify, gate)
                 notify(f"enc_{m}")       # on the stream that produced the gradients
             return run
 
@@ -991,18 +967,17 @@ class MisaEngine:
         # SMs the text kernel leaves free (measured 4.54 ms/step; waiting for the text launch to
         # complete 4.87, no gate 4.56).  The recurrence kernels clean their exchange flags
         # themselves, so no memset node sits between that point and the launch.
-        self._order_events = {}
+        gate = {}
         self._fork({m: enc_bwd(m) for m in MODS}, text_first=not self.gru)
-        self._order_events = {}
         k.join_leaves()
         k.leaf_on = False
         return dutt["t"] if self.use_bert else None
 
-    def _encode_backward(self, m, dutt, G, pk, P, notify=None):
+    def _encode_backward(self, m, dutt, G, pk, P, notify, gate):
         """BPTT of both layers of modality m + the hoisted weight-gradient GEMMs.  The recurrence
         and the dX GEMM form the critical path; the weight-gradient work of a layer (h_prev shift,
-        dW_ih, dW_hh, bias column sums) is pushed to a side stream so it overlaps the next BPTT
-        kernel (which leaves 36 of the 148 SMs free)."""
+        dW_ih, dW_hh, bias column sums) is pushed to side streams so it overlaps the next BPTT
+        kernel (which leaves 36 of the 148 SMs free).  ``gate``: as in `_encode`."""
         k, H = self.k, self.H[m]
         r1, r2, ln = ENC[m]
         N, B, Tmax = pk["N"], pk["B"], pk["Tmax"]
@@ -1018,9 +993,7 @@ class MisaEngine:
         scratch = self.buf(f"lstm_scratch_{m}", max(1, nbytes // 4))
         dY1n = self.pbuf(f"dY1n_{m}", N, 2 * H)
         dY1 = self.buf(f"dY1_{m}", N, 2 * H)
-        use_side = not _DRYRUN
-        cur = torch.cuda.current_stream() if use_side else None
-        side_used = []
+        wg_roles = []
         G_real = G
         if self.gru:
             P = {**P, **self._gru_overlay(m, P, "weights")}      # expanded by the forward
@@ -1031,13 +1004,7 @@ class MisaEngine:
                 k.layernorm_bwd(dY1n, Y1, None, P[f"{ln}.weight"], mu, rs, dY1, G[f"{ln}.weight"],
                                 G[f"{ln}.bias"])
             tcws = self._lstm_tc_ws(m, B, H, Tmax)
-            layer = 2 if r == r2 else 1
-            if use_side and m != "t" and layer in self._order_events:
-                cur.wait_event(self._order_events[layer])
-            if use_side and m == "t" and tcws is not None:
-                ev = torch.cuda.Event()
-                ev.record(cur)
-                self._order_events[layer] = ev
+            self._launch_gate(gate, m, 2 if r == r2 else 1, tcws)
             if tcws is not None:
                 k._c("mmda_lstm_tc_backward", _ptr(Gt), _ptr(P[f"{r}.weight_hh_l0"]),
                      _ptr(P[f"{r}.weight_hh_l0_reverse"]), _ptr(C), _ptr(dy), _ptr(dutt), 4 * H, o_f,
@@ -1053,8 +1020,6 @@ class MisaEngine:
                 # padding rows of d(gates) still hold the forward GEMM's values: zero them before
                 # the weight-gradient / dX GEMMs and bias column sums reduce over all N rows
                 k._c("mmda_zero_tail_rows", _ptr(Gt), 8 * H, _ptr(pk["n_dev"]), N)
-            if m == "t":
-                self._mark(f"  t.{r} BPTT done")
             I = Xin.shape[1]
             # 3xTF32 like the forward: weight / activation gradients are sums with heavy
             # cancellation, where bf16 operands cost several percent (measured 4-13 %)
@@ -1062,9 +1027,26 @@ class MisaEngine:
             Xp = self._prep(f"tcX_{r}", Xin, kind=0)          # the fp32 tensor itself
             Wst = self._prep_buf(f"tcW_{r}", 8 * H, I, 0, split=True)   # packed by the forward
 
-            hp_box = {}
+            def wgrad_dir(di):
+                # dG columns are gate-interleaved (u*4+g): c_ilv=H stores row u*4+g at g*H+u
+                suf = ("", "_reverse")[di]
+                dG = Gt[:, di * 4 * H:(di + 1) * 4 * H]
+                # contract over tokens: both operands MN-major, auto split-K
+                dGd = self._cols(dGp, di * 4 * H, (di + 1) * 4 * H)
+                k.gemm_tc(0, 1, 1, 4 * H, I, N, dGd, Xp, G[f"{r}.weight_ih_l0{suf}"], mode=1,
+                          split_k=0, c_ilv=H)
+                k.gemm_tc(0, 1, 1, 4 * H, H, N, dGd, HPp[di], G[f"{r}.weight_hh_l0{suf}"], mode=1,
+                          split_k=0, c_ilv=H)
+                k.colsum(dG, G[f"{r}.bias_ih_l0{suf}"], G[f"{r}.bias_hh_l0{suf}"], ilv=H)
+                if self.gru:     # 4-slot gradients -> the (3H, .) parameters' gradients
+                    k._c("mmda_gru_fold_grads", *[_ptr(G[f"{r}.{kk}{suf}"]) for kk in self._RNN_KEYS],
+                         H, I, *[_ptr(G_real[f"{r}.{kk}{suf}"]) for kk in self._RNN_KEYS])
 
-            def wgrad_common(r=r, Y=Y):
+            # one side stream per (layer, direction): the weight-gradient GEMMs of the second
+            # layer must not queue in front of the first layer's (they overlap the next BPTT
+            # launch and only get the SMs it leaves free)
+            wA, wB = ("wg", m, r, 0), ("wg", m, r, 1)
+            with k.side(wA, PRIO_LEAF):
                 if self.gru:
                     for suf in ("", "_reverse"):
                         for kk in self._RNN_KEYS:
@@ -1073,77 +1055,32 @@ class MisaEngine:
                 HP = self.buf(f"HP_{r}", N, 2 * Hp)
                 k._c("mmda_lstm_shift_h", _ptr(Y), _ptr(HP), _ptr(pk["row_t"]), _ptr(pk["row_j"]),
                      _ptr(pk["lens"]), _ptr(pk["off"]), N, H, Hp)
-                hp_box["HPp"] = [self._prep(f"tcHP_{r}_{di}", HP[:, di * Hp:di * Hp + H], kind=0)
-                                 for di in (0, 1)]
-
-            def wgrad_dir(di, r=r, Gt=Gt, I=I):
-                # dG columns are gate-interleaved (u*4+g): c_ilv=H stores row u*4+g at g*H+u
-                suf = ("", "_reverse")[di]
-                dG = Gt[:, di * 4 * H:(di + 1) * 4 * H]
-                # contract over tokens: both operands MN-major, auto split-K
-                dGd = self._cols(dGp, di * 4 * H, (di + 1) * 4 * H)
-                k.gemm_tc(0, 1, 1, 4 * H, I, N, dGd, Xp, G[f"{r}.weight_ih_l0{suf}"], mode=1,
-                          split_k=0, c_ilv=H)
-                k.gemm_tc(0, 1, 1, 4 * H, H, N, dGd, hp_box["HPp"][di],
-                          G[f"{r}.weight_hh_l0{suf}"], mode=1, split_k=0, c_ilv=H)
-                k.colsum(dG, G[f"{r}.bias_ih_l0{suf}"], G[f"{r}.bias_hh_l0{suf}"], ilv=H)
-                if self.gru:     # 4-slot gradients -> the (3H, .) parameters' gradients
-                    k._c("mmda_gru_fold_grads", *[_ptr(G[f"{r}.{kk}{suf}"]) for kk in self._RNN_KEYS],
-                         H, I, *[_ptr(G_real[f"{r}.{kk}{suf}"]) for kk in self._RNN_KEYS])
-
-            if use_side:
-                # one side stream per (layer, direction): the weight-gradient GEMMs of the second
-                # layer must not queue in front of the first layer's (they overlap the next BPTT
-                # launch and only get the SMs it leaves free)
-                sA, sB = self._wgrad_stream((m, r, 0)), self._wgrad_stream((m, r, 1))
-                ev = torch.cuda.Event()
-                ev.record(cur)
-                sA.wait_event(ev)
-                with torch.cuda.stream(sA):
-                    k.bind_stream()
-                    wgrad_common()
-                    evc = torch.cuda.Event()
-                    evc.record(sA)
-                    wgrad_dir(0)
-                sB.wait_event(evc)
-                with torch.cuda.stream(sB):
-                    k.bind_stream()
-                    wgrad_dir(1)
-                    if m == "t":
-                        self._mark(f"  t.{r} wgrad (side stream) done")
-                    if m == "t" and r == r2 and notify is not None:
-                        # rnn2's gradients are complete once both directions' streams are: let the
-                        # data-parallel trainer reduce them under the layer-1 BPTT
-                        eva = torch.cuda.Event()
-                        eva.record(sA)
-                        sB.wait_event(eva)
-                        notify("enc_t_l2")
-                k.bind_stream()
-                side_used += [sA, sB]
-            else:
-                wgrad_common()
+                HPp = [self._prep(f"tcHP_{r}_{di}", HP[:, di * Hp:di * Hp + H], kind=0)
+                       for di in (0, 1)]
+                common = k.mark()
                 wgrad_dir(0)
+            with k.side(wB, PRIO_LEAF, after=(common,)):
                 wgrad_dir(1)
+                if m == "t" and r == r2:
+                    # rnn2's gradients are complete once both directions' streams are: let the
+                    # data-parallel trainer reduce them under the layer-1 BPTT
+                    k.wait(k.mark(wA))
+                    notify("enc_t_l2")
+            wg_roles += [wA, wB]
             if r == r2 or m == "t":
                 dX = dY1n if r == r2 else self.buf("dX_t", N, H)
                 # dX = dG [N x 8H] * [W_ih ; W_ih_reverse] (stored [8H][I]: MN-major B)
                 k.gemm_tc(0, 0, 1, N, I, 8 * H, dGp, Wst, dX)
-                if m == "t":
-                    self._mark(f"  t.{r} dX GEMM done")
                 if r == r1:
                     V = P["embed.weight"].shape[0]
                     k._c("mmda_embedding_backward", _ptr(G["embed.weight"]),
                          _ptr(self.saved["sent"]), _ptr(dX), _ptr(pk["row_t"]), _ptr(pk["row_j"]),
                          _ptr(pk["sidx"]), N, B, H, V)
-                    if notify is not None:
-                        # the dense embedding gradient (the largest bucket) is complete here, a
-                        # millisecond of weight-gradient GEMMs before the rest of the encoder:
-                        # its all-reduce runs under them
-                        notify("embed")
-        for st in side_used:
-            done = torch.cuda.Event()
-            done.record(st)
-            cur.wait_event(done)
+                    # the dense embedding gradient (the largest bucket) is complete here, a
+                    # millisecond of weight-gradient GEMMs before the rest of the encoder: its
+                    # all-reduce runs under them
+                    notify("embed")
+        k.wait(*[k.mark(role) for role in wg_roles])
 
 
 # ------------------------------------------------------------------------------------------

@@ -169,14 +169,13 @@ class FusedTrainer:
         self._reduced = set()
         self._defer_ready = None
         self._equal_B = None            # local batch size last verified equal on every rank
-        self.trace_ready = None         # profiling aid: {tag: timed event} of the last step
+        self._early_ran = False         # _loss_early enqueued the token-only part of the losses
         # device-resident step state (step counter = dropout seed offset, Adam bias corrections,
         # learning rate: csrc/adam.cu StepState, 40 bytes)
         self.state = torch.zeros(5, dtype=torch.float64, device=self.p_arena.device)
         self._lr_dev = None             # learning rate last written into self.state
-        if not _engine._DRYRUN:
-            self.eng.k.bind_stream()
-            self.eng.k._c("mmda_step_state_init", _ptr(self.state), 0, 0.9, 0.999)
+        self.eng.k.bind_stream()
+        self.eng.k._c("mmda_step_state_init", _ptr(self.state), 0, 0.9, 0.999)
         # CUDA-graph replay of the whole step (single GPU and data parallel)
         self.use_graph = use_graph if use_graph is not None else True
         self._graphs = {}               # key -> captured step (see step())
@@ -225,6 +224,7 @@ class FusedTrainer:
             else:
                 self.m, self.v = torch.zeros_like(self.p_arena), torch.zeros_like(self.p_arena)
             self.step_count = step
+            self.state = self.state.to(self.p_arena.device)     # the step kernels read it by pointer
 
     def attach_grads(self):
         """Expose the arena gradients as ``param.grad`` (views; for inspection and tests).
@@ -282,24 +282,14 @@ class FusedTrainer:
         sync = self.global_stats and self.world > 1
         st, segA, segB, segC, losses, coef = self._loss_buffers(B)
         X0 = eng.buf("X0", B, 6, d)
-        main = torch.cuda.current_stream()
-        if not hasattr(self, "_loss_stream"):
-            self._loss_stream = torch.cuda.Stream(device=self.g_arena.device)
-        s = self._loss_stream
-        ev0 = torch.cuda.Event()
-        ev0.record(main)
-        s.wait_event(ev0)
-        with torch.cuda.stream(s):
-            k.bind_stream()
+        with k.side("loss"):
             st.zero_()
             k._c("mmda_loss_phase1", _ptr(X0), None, None, None, None, None, _ptr(segA), B, d, NC, 1)
             if sync:
                 self._allreduce(segA[:6 * d])
             self._loss_tokens(X0, segA, segB, segC, losses, coef, B, Bg, sync, mode=1)
-            ev = torch.cuda.Event()
-            ev.record(s)
-        k.bind_stream()
-        return ev
+        self._early_ran = True
+        return k.mark("loss")
 
     def _loss_tokens(self, X0, segA, segB, segC, losses, coef, B, Bg, sync, mode):
         """phase 2 .. 4b: centred / normalised tokens, moments, Grams, diff + CMD values and the
@@ -331,8 +321,9 @@ class FusedTrainer:
         return dZ
 
     def loss_and_grads(self, out, labels, B, early_ev=None):
-        """Fused losses forward + backward wrt the model outputs (csrc/loss.cu).  ``early_ev``:
-        the token-only part already ran (`_loss_early`); wait for it and do the rest."""
+        """Fused losses forward + backward wrt the model outputs (csrc/loss.cu).  When
+        `_loss_early` has enqueued the token-only part, wait for its event ``early_ev`` and do
+        the rest."""
         eng, k = self.eng, self.eng.k
         d, NC, cfg = eng.d, eng.NC, self.cfg
         Bg = float(B * self.world) if self.global_stats else float(B)
@@ -343,12 +334,13 @@ class FusedTrainer:
         y = labels
         w_conf = float(cfg.conf_weight) if self.use_confid else 0.0
         adv = eng.adversarial
-        if early_ev is None:
+        early, self._early_ran = self._early_ran, False
+        if not early:
             st.zero_()
             k._c("mmda_loss_phase1", _ptr(X0), _ptr(O), _ptr(R), _ptr(SC), _ptr(TCP), _ptr(y),
                  _ptr(segA), B, d, NC, 3)
         else:
-            torch.cuda.current_stream().wait_event(early_ev)
+            k.wait(early_ev)
             k._c("mmda_loss_phase1", _ptr(X0), _ptr(O), _ptr(R), _ptr(SC), _ptr(TCP), _ptr(y),
                  _ptr(segA), B, d, NC, 2)
         dDL = None
@@ -356,7 +348,7 @@ class FusedTrainer:
             dDL = eng.buf("dDL", 3, B, 3)
             k._c("mmda_loss_domain", _ptr(out["domain"]), _ptr(dDL), _ptr(segA), B, d, NC, Bg,
                  float(cfg.sim_weight))
-        if early_ev is None:
+        if not early:
             if sync:
                 self._allreduce(segA)
             dZ = self._loss_tokens(X0, segA, segB, segC, losses, coef, B, Bg, sync, mode=3)
@@ -389,12 +381,8 @@ class FusedTrainer:
     def _on_ready(self, tag):
         if self.world == 1 or (tag == "enc_t" and self.use_bert and not self._bert_done):
             return
-        if tag in self._ISSUE_ORDER and not _engine._DRYRUN and self._defer_ready is not None:
-            ev = torch.cuda.Event(enable_timing=self.trace_ready is not None)
-            ev.record(torch.cuda.current_stream())
-            self._defer_ready[tag] = ev
-            if self.trace_ready is not None:
-                self.trace_ready[tag] = ev
+        if tag in self._ISSUE_ORDER and self._defer_ready is not None:
+            self._defer_ready[tag] = self.eng.k.mark()
             return
         self._issue(tag)
 
@@ -416,18 +404,13 @@ class FusedTrainer:
         evs, self._defer_ready = self._defer_ready, None
         if not evs:
             return
-        main = torch.cuda.current_stream()
-        if not hasattr(self, "_ar_stream"):
-            self._ar_stream = torch.cuda.Stream(device=self.g_arena.device)
-        h = self._ar_stream
-        with torch.cuda.stream(h):
+        k = self.eng.k
+        with k.side("allreduce", after=()):
             for tag in self._ISSUE_ORDER:
                 if tag in evs:
-                    h.wait_event(evs[tag])
+                    k.wait(evs[tag])
                     self._issue(tag)
-            done = torch.cuda.Event()
-            done.record(h)
-        main.wait_event(done)
+        k.wait(k.mark("allreduce"))
 
     def forward_backward(self, sentences, visual, acoustic, lengths, labels, bert=None):
         """zero_grad + forward + losses + backward (+ gradient all-reduce).  Returns the device
@@ -447,35 +430,22 @@ class FusedTrainer:
                                         drop=self.model.training, seed=eng.seed ^ 0xB347,
                                         seed_dev=self.state)
         # the gradient arena (43 MB with a 20k-word embedding) is cleared on a side stream under
-        # the forward instead of on the chain between the classifier and the losses
-        zero_ev = None
-        if not _engine._DRYRUN:
-            cur = torch.cuda.current_stream()
-            if not hasattr(self, "_zero_stream"):
-                self._zero_stream = torch.cuda.Stream(device=self.g_arena.device)
-            ev0 = torch.cuda.Event()
-            ev0.record(cur)                       # after the previous step's Adam read the arena
-            self._zero_stream.wait_event(ev0)
-            with torch.cuda.stream(self._zero_stream):
-                self.g_arena[:self.n_active].zero_()
-                zero_ev = torch.cuda.Event()
-                zero_ev.record(self._zero_stream)
+        # the forward instead of on the chain between the classifier and the losses, after the
+        # previous step's optimizer read it
+        with eng.k.side("zero"):
+            self.g_arena[:self.n_active].zero_()
         early = {}
-        hook = None
-        if not _engine._DRYRUN:
-            def hook():
-                early["ev"] = self._loss_early(int(lengths.numel()))
+
+        def hook():
+            early["ev"] = self._loss_early(int(lengths.numel()))
         out = eng.forward(sentences, visual, acoustic, lengths, train=True, want_sp=False,
                           seed_dev=self.state, utt_text=utt_text, after_heads=hook)
         B = out["scores"].shape[0]
         if labels.shape != (B, eng.NC) or labels.dtype != torch.float32 or \
                 not (labels.is_cuda or _engine._DRYRUN):
             raise MmdaError("labels must be a CUDA float32 (B, num_classes) tensor")
-        if zero_ev is not None:
-            torch.cuda.current_stream().wait_event(zero_ev)
-        else:
-            self.g_arena[:self.n_active].zero_()
-        losses, grads = self.loss_and_grads(out, labels.contiguous(), B, early_ev=early.get("ev"))
+        eng.k.wait(eng.k.mark("zero"))
+        losses, grads = self.loss_and_grads(out, labels.contiguous(), B, early_ev=early["ev"])
         self._pending = []
         self._reduced = set()
         self._bert_done = False
@@ -500,8 +470,7 @@ class FusedTrainer:
         lr = float(self.lr)
         if lr == self._lr_dev:
             return
-        if not _engine._DRYRUN:
-            self.eng.k.bind_stream()
+        self.eng.k.bind_stream()
         LIB.call("mmda_step_state_set_lr", _ptr(self.state), lr, self.eng.k.stream)
         self._lr_dev = lr
 
@@ -623,8 +592,7 @@ class FusedTrainer:
                             "fused step count only")
         self.step_count = steps.pop() if steps else 0
         self.lr = float(g["lr"])
-        if not _engine._DRYRUN:
-            self.eng.k.bind_stream()
+        self.eng.k.bind_stream()
         # rewrites the step counter and beta products in place: a captured step reads them by
         # pointer, so it stays valid
         self.eng.k._c("mmda_step_state_init", _ptr(self.state), self.step_count, 0.9, 0.999)
@@ -781,10 +749,10 @@ class FusedTrainer:
         dev = device or self.p_arena.device
         fields = ("sentences", "visual", "acoustic", "labels") + \
             (("bert_sent", "bert_sent_type", "bert_sent_mask") if self.use_bert else ())
-        main = torch.cuda.current_stream()
+        k = self.eng.k
         staged = getattr(self, "_staged", None)
         if staged is not None and staged[0] is batch:
-            main.wait_event(staged[2])
+            k.wait(staged[2])
             t = staged[1]
         else:
             t = {f: getattr(batch, f).to(dev, non_blocking=True) for f in fields}
@@ -794,13 +762,10 @@ class FusedTrainer:
         if fetch:
             out = LossFuture(self, out)
         if prefetch is not None:
-            if not hasattr(self, "_copy_stream"):
-                self._copy_stream = torch.cuda.Stream(device=dev)
-            with torch.cuda.stream(self._copy_stream):
+            with k.side("copy", after=()):
                 nt = {f: getattr(prefetch, f).to(dev, non_blocking=True) for f in fields}
-                ev = torch.cuda.Event()
-                ev.record(self._copy_stream)
+            main = torch.cuda.current_stream()
             for v in nt.values():
                 v.record_stream(main)
-            self._staged = (prefetch, nt, ev)
+            self._staged = (prefetch, nt, k.mark("copy"))
         return out

@@ -108,11 +108,13 @@ def test_arena_plan_buckets_are_contiguous_and_ordered():
 
 
 class _StubLib:
-    """Records the C-ABI call sequence; lets the engine's host orchestration run on CPU."""
+    """Records the C-ABI call sequence (names; arguments in `args`, the stream last); lets the
+    engine's host orchestration run on CPU."""
     def __init__(self):
-        self.calls = []
+        self.calls, self.args = [], []
     def __call__(self, name, *args):
         self.calls.append(name)
+        self.args.append(args)
         return 0
 
 
@@ -126,7 +128,9 @@ def dryrun(monkeypatch):
     return stub
 
 
-def test_engine_kernel_sequence_level1_and_level2(dryrun):
+def test_engine_kernel_sequence_level1_and_level2_early_loss(dryrun):
+    """Level-1 gradient contract, then the C-ABI order of a fused step as the GPU runs it: the
+    token-only loss chain forked behind the heads, the rest of the losses before the backward."""
     from mmda_b200.synthetic import batch_for
     from mmda_b200.trainer import FusedTrainer
     cfg = mosei_config(vocab_size=80, batch_size=12, use_confidNet=True)
@@ -146,17 +150,29 @@ def test_engine_kernel_sequence_level1_and_level2(dryrun):
     # text layers (the embedding needs it) / of layer 2 only (visual, acoustic): 12 + 11 + 11
     assert fwd["mmda_gemm_tc"] == 34
     dryrun.calls.clear()
+    dryrun.args.clear()
     tr = FusedTrainer(model)
     tr.step(b.sentences, b.visual, b.acoustic, b.lengths, b.labels)
     seq = dryrun.calls
     assert seq[-1] == "mmda_adam_clip_step"
-    order = [seq.index(n) for n in ("mmda_embedding_forward", "mmda_lstm_forward",
-                                    "mmda_attention_forward", "mmda_loss_phase1", "mmda_loss_finalize",
-                                    "mmda_attention_backward", "mmda_lstm_backward",
-                                    "mmda_embedding_backward", "mmda_adam_clip_step")]
+    mode = lambda name: [a[-2] for n, a in zip(seq, dryrun.args) if n == name]    # last arg: stream
+    assert mode("mmda_loss_phase1") == [1, 2] and mode("mmda_loss_finalize") == [1, 2]
+    # the token-only part of the losses (DiffLoss / CMD) is enqueued right behind the heads (the
+    # last one ends with utt = private + shared and the recon linear), before the fusion layer
+    i1 = seq.index("mmda_loss_phase1")
+    assert seq[i1 - 2:i1] == ["mmda_add2d", "mmda_sgemm"]
+    assert seq[i1:i1 + 9] == ["mmda_loss_phase1", "mmda_loss_phase2", "mmda_loss_gram",
+                              "mmda_loss_finalize", "mmda_loss_dxn", "mmda_loss_phase4a",
+                              "mmda_loss_phase4b", "mmda_sgemm", "mmda_attention_forward"]
+    late = lambda name: len(seq) - 1 - seq[::-1].index(name)       # last call of that name
+    order = [seq.index("mmda_embedding_forward"), seq.index("mmda_lstm_forward"),
+             seq.index("mmda_attention_forward"), late("mmda_loss_phase1"),
+             late("mmda_loss_finalize"), seq.index("mmda_loss_grad_misc"),
+             seq.index("mmda_attention_backward"), seq.index("mmda_lstm_backward"),
+             seq.index("mmda_embedding_backward"), seq.index("mmda_adam_clip_step")]
     assert order == sorted(order)
     c2 = collections.Counter(seq)
-    assert c2["mmda_loss_phase1"] == c2["mmda_loss_phase2"] == c2["mmda_loss_phase4a"] == 1
+    assert c2["mmda_loss_phase1"] == 2 and c2["mmda_loss_phase2"] == c2["mmda_loss_phase4a"] == 1
     # parameters alias the arena; untouched-by-contract params sit past the active range
     for n, p in model.named_parameters():
         off, sz = tr.layout[n]

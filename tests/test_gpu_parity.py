@@ -541,6 +541,41 @@ def test_cuda_graph_replay_equals_eager(dev, rnncell):
     C.finish()
 
 
+def test_graph_step_follows_the_model_to_another_gpu(dev):
+    """The step's side streams belong to a device: after ``model.to('cuda:1')`` a trainer that
+    replayed a graph on cuda:0 steps on cuda:1 (eager warm-up, new capture, replays) and trains
+    exactly as a trainer built there with the same parameters and optimizer state."""
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs two GPUs")
+    from mmda_b200 import MISA, mosei_config
+    from mmda_b200.synthetic import batch_for
+    from mmda_b200.trainer import FusedTrainer
+    cfg = mosei_config(vocab_size=300, batch_size=48, use_confidNet=True)
+    b = batch_for(cfg, seed=7, lengths="full", seq_len=12)
+    d1 = torch.device("cuda:1")
+
+    def run(tr, d, n):
+        return torch.stack([tr.step(b.sentences.to(d), b.visual.to(d), b.acoustic.to(d), b.lengths,
+                                    b.labels.to(d))[:6].clone() for _ in range(n)]).cpu()
+    torch.manual_seed(5)
+    model = MISA(cfg).to(dev).eval()
+    tr = FusedTrainer(model)
+    run(tr, dev, 4)
+    assert tr._graph is not None
+    with torch.cuda.device(1):
+        model.to(d1)
+        ref = MISA(cfg)
+        ref.load_state_dict(model.state_dict())
+        fresh = FusedTrainer(ref.to(d1).eval())
+        tr._check_alias()                  # the moved trainer's optimizer state, on cuda:1
+        fresh.load_optimizer_state_dict(tr.optimizer_state_dict())
+        got, want = run(tr, d1, 5), run(fresh, d1, 5)
+        assert tr._graph is not None and tr.p_arena.device == d1
+        torch.cuda.synchronize()
+    err = float(((got - want).abs() / want.abs().clamp_min(1e-6)).max())
+    assert err < 1e-5, err
+
+
 def test_graph_replay_after_other_forwards(dev):
     """A captured step reads the packing buffers by pointer.  evaluate(), a level-1 forward or an
     eager step with other lengths overwrite them between two replays; the next replay must still
