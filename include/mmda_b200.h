@@ -29,12 +29,19 @@ typedef struct CUstream_st* mmda_stream_t; /* == cudaStream_t */
 #define MMDA_ERR_ARG (-2)
 #define MMDA_ERR_UNSUPPORTED (-3)
 
-/* activation ids for fused epilogues (config.activation, src/config.py:24-27) */
+/* activation ids for fused epilogues (config.activation, src/config.py:24-27), with torch's
+ * default arguments: ELU alpha 1, Hardshrink lambda 0.5, Hardtanh [-1, 1].  MMDA_ACT_RRELU is
+ * nn.RReLU in eval mode (fixed slope 11/48 = the mean of U(1/8, 1/3)); in training its random
+ * slopes come from mmda_rrelu_forward / mmda_rrelu_backward.  nn.PReLU has no id. */
 #define MMDA_ACT_NONE 0
 #define MMDA_ACT_LEAKYRELU 1
 #define MMDA_ACT_SIGMOID 2
 #define MMDA_ACT_RELU 3
 #define MMDA_ACT_TANH 4
+#define MMDA_ACT_ELU 5
+#define MMDA_ACT_HARDSHRINK 6
+#define MMDA_ACT_HARDTANH 7
+#define MMDA_ACT_RRELU 8
 
 const char* mmda_last_error(void);
 int mmda_abi_version(void);
@@ -235,6 +242,17 @@ int mmda_act_dropout_forward(float* x, long long n, int act, float p, unsigned l
 int mmda_dropout_act_backward(float* dy, const float* y, long long n, int act, float p,
                               unsigned long long seed, const unsigned long long* seed_dev,
                               unsigned stream_id, mmda_stream_t stream);
+/* nn.RReLU() in training mode, in place (y may alias x; dy is updated in place): the activation of
+ * project_{t,v,a} and discriminator_layer_1 (src/models.py:61-127) under --activation rrelu.
+ * y = x > 0 ? x : x * r, one slope r ~ U(1/8, 1/3) per element (x = 0 draws one as well), drawn
+ * from (seed [+ *seed_dev, the device step counter, if non-NULL], stream_id, row * cols + col)
+ * like mmda_dropout's mask, so the backward redraws exactly the forward's slopes and nothing per
+ * element is stored.  Backward: dy *= y > 0 ? 1 : r, with y the forward's output.  x / y / dy
+ * share the leading dimension ld. */
+int mmda_rrelu_forward(const float* x, float* y, int ld, int rows, int cols, unsigned long long seed,
+                       const unsigned long long* seed_dev, unsigned stream_id, mmda_stream_t stream);
+int mmda_rrelu_backward(float* dy, const float* y, int ld, int rows, int cols, unsigned long long seed,
+                        const unsigned long long* seed_dev, unsigned stream_id, mmda_stream_t stream);
 /* getBinaryTensor, src/utils/functions.py:112-115 */
 int mmda_threshold(const float* x, float* out, long long n, float thr, mmda_stream_t stream);
 

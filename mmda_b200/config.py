@@ -18,12 +18,27 @@ ACTIVATIONS = {
     "sigmoid": 2,
     "relu": 3,
     "tanh": 4,
+    "elu": 5,
+    "hardshrink": 6,
+    "hardtanh": 7,
+    "rrelu": 8,
+}
+
+# torch's defaults, which is what the kernels compute: the reference constructs
+# ``config.activation()`` with no arguments (src/models.py:61-127)
+ACTIVATION_DEFAULTS = {
+    "elu": dict(alpha=1.0),
+    "hardshrink": dict(lambd=0.5),
+    "hardtanh": dict(min_val=-1.0, max_val=1.0),
+    "rrelu": dict(lower=1.0 / 8, upper=1.0 / 3),
 }
 
 
 def activation_name(act: Any) -> str:
     """Map what the reference stores in ``config.activation`` (an ``nn.Module`` *class*,
-    reference ``src/config.py:24-27,78-79``) or a plain string onto a kernel epilogue name."""
+    reference ``src/config.py:24-27,78-79``), an instance of one, or a plain string onto a kernel
+    epilogue name.  An ELU / Hardshrink / Hardtanh / RReLU instance must carry torch's default
+    arguments (``inplace`` is free: it does not change the values)."""
     if isinstance(act, str):
         name = act.lower()
     else:
@@ -33,6 +48,12 @@ def activation_name(act: Any) -> str:
         raise ValueError(
             f"activation {act!r} has no sm_100a epilogue in this build "
             f"(supported: {sorted(k for k in ACTIVATIONS if k != 'none')})")
+    if not isinstance(act, (str, type)):
+        defaults = ACTIVATION_DEFAULTS.get(name, {})
+        bad = {k: getattr(act, k) for k, v in defaults.items() if getattr(act, k, v) != v}
+        if bad:
+            raise ValueError(f"activation {act!r}: only torch's defaults are implemented "
+                             f"({', '.join(f'{k}={v}' for k, v in defaults.items())})")
     return name
 
 

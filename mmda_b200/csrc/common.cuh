@@ -53,7 +53,15 @@ MmdaDeviceCtx* mmda_device_ctx();
   } while (0)
 
 // activation ids (keep in sync with mmda_b200/config.py::ACTIVATIONS and include/mmda_b200.h)
-enum : int { ACT_NONE = 0, ACT_LEAKYRELU = 1, ACT_SIGMOID = 2, ACT_RELU = 3, ACT_TANH = 4 };
+// torch's defaults (the reference constructs config.activation() with no arguments): ELU alpha 1,
+// Hardshrink lambda 0.5, Hardtanh [-1, 1], RReLU U(1/8, 1/3).  ACT_RRELU is RReLU's eval form, a
+// leaky slope of (1/8 + 1/3) / 2 = 11/48; its training form is mmda_rrelu_forward / _backward.
+enum : int {
+  ACT_NONE = 0, ACT_LEAKYRELU = 1, ACT_SIGMOID = 2, ACT_RELU = 3, ACT_TANH = 4, ACT_ELU = 5,
+  ACT_HARDSHRINK = 6, ACT_HARDTANH = 7, ACT_RRELU = 8
+};
+constexpr float RRELU_LOWER = 1.0f / 8.0f, RRELU_UPPER = 1.0f / 3.0f;
+constexpr float RRELU_EVAL_SLOPE = 11.0f / 48.0f;
 
 __device__ __forceinline__ float sigmoidf_acc(float x) { return 1.0f / (1.0f + expf(-x)); }
 
@@ -63,17 +71,27 @@ __device__ __forceinline__ float apply_act(float x, int act) {
     case ACT_SIGMOID: return sigmoidf_acc(x);
     case ACT_RELU: return x > 0.f ? x : 0.f;
     case ACT_TANH: return tanhf(x);
+    case ACT_ELU: return x > 0.f ? x : expm1f(x);
+    case ACT_HARDSHRINK: return (x > 0.5f || x < -0.5f) ? x : 0.f;
+    case ACT_HARDTANH: return x < -1.f ? -1.f : (x > 1.f ? 1.f : x);   // NaN passes, as in torch
+    case ACT_RRELU: return x > 0.f ? x : RRELU_EVAL_SLOPE * x;
     default: return x;
   }
 }
 
-// derivative expressed through the activation OUTPUT y (all supported activations allow it)
+// derivative expressed through the activation OUTPUT y (all supported activations allow it).  At
+// the kinks it is torch's: ELU' = 1 at 0 (y = 0 -> y + 1), Hardshrink' = 0 at +-0.5 (y = 0),
+// Hardtanh' = 0 at +-1 (|y| = 1)
 __device__ __forceinline__ float act_grad_from_output(float y, int act) {
   switch (act) {
     case ACT_LEAKYRELU: return y > 0.f ? 1.f : 0.01f;
     case ACT_SIGMOID: return y * (1.f - y);
     case ACT_RELU: return y > 0.f ? 1.f : 0.f;
     case ACT_TANH: return 1.f - y * y;
+    case ACT_ELU: return y > 0.f ? 1.f : y + 1.f;
+    case ACT_HARDSHRINK: return y != 0.f ? 1.f : 0.f;
+    case ACT_HARDTANH: return fabsf(y) < 1.f ? 1.f : 0.f;
+    case ACT_RRELU: return y > 0.f ? 1.f : RRELU_EVAL_SLOPE;
     default: return 1.f;
   }
 }
@@ -175,4 +193,9 @@ __device__ __forceinline__ float rng_uniform(uint64_t seed, uint32_t stream, uin
   uint32_t h = mix32((uint32_t)seed ^ mix32(idx + 0x9e3779b9U * (stream + 1)));
   h = mix32(h ^ (uint32_t)(seed >> 32) ^ (stream * 0x85ebca6bU));
   return (h >> 8) * (1.0f / 16777216.0f);
+}
+// training-mode RReLU slope of one element: U(1/8, 1/3) from the same counter-based stream, so the
+// backward redraws the forward's slope instead of storing it
+__device__ __forceinline__ float rrelu_slope(uint64_t seed, uint32_t stream, uint32_t idx) {
+  return fmaf(rng_uniform(seed, stream, idx), RRELU_UPPER - RRELU_LOWER, RRELU_LOWER);
 }

@@ -476,6 +476,33 @@ __global__ void dropout_act_bwd_kernel(float* __restrict__ dy, const float* __re
     dy[i] = d * act_grad_from_output(y[i], act);
   }
 }
+// training-mode RReLU (F.rrelu(training=True), torch's U(1/8, 1/3)): y = x > 0 ? x : x * r with one
+// slope r per element drawn from (seed, stream, r * cols + c) -- x = 0 draws one too, torch tests
+// x <= 0.  The backward redraws the same r; y > 0 exactly where x > 0 (r > 0), so it reads y.
+// y may alias x, and dy is updated in place.
+__global__ void rrelu_fwd_kernel(const float* x, float* y, int ld, int rows, int cols,
+                                 unsigned long long seed, const unsigned long long* __restrict__ seed_dev,
+                                 unsigned stream) {
+  if (seed_dev) seed += seed_dev[0] * 0x9E3779B97F4A7C15ULL;
+  const size_t n = (size_t)rows * cols;
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n;
+       i += (size_t)gridDim.x * blockDim.x) {
+    const size_t o = (i / cols) * ld + i % cols;
+    const float v = x[o];
+    y[o] = v > 0.f ? v : v * rrelu_slope(seed, stream, (uint32_t)i);
+  }
+}
+__global__ void rrelu_bwd_kernel(float* __restrict__ dy, const float* __restrict__ y, int ld, int rows,
+                                 int cols, unsigned long long seed,
+                                 const unsigned long long* __restrict__ seed_dev, unsigned stream) {
+  if (seed_dev) seed += seed_dev[0] * 0x9E3779B97F4A7C15ULL;
+  const size_t n = (size_t)rows * cols;
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n;
+       i += (size_t)gridDim.x * blockDim.x) {
+    const size_t o = (i / cols) * ld + i % cols;
+    if (!(y[o] > 0.f)) dy[o] *= rrelu_slope(seed, stream, (uint32_t)i);
+  }
+}
 __global__ void threshold_kernel(const float* __restrict__ x, float* __restrict__ out, size_t n,
                                  float thr) {
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n;
@@ -789,6 +816,28 @@ int mmda_dropout_act_backward(float* dy, const float* y, long long n, int act, f
   MMDA_REQUIRE(p >= 0.f && p < 1.f, "dropout_act_backward: p=%f", p);
   dropout_act_bwd_kernel<<<ew_grid((size_t)n), 256, 0, stream>>>(dy, y, (size_t)n, act, p, 1.f / (1.f - p),
                                                                  seed, seed_dev, stream_id);
+  MMDA_CHECK_LAUNCH();
+  return MMDA_OK;
+}
+
+int mmda_rrelu_forward(const float* x, float* y, int ld, int rows, int cols, unsigned long long seed,
+                       const unsigned long long* seed_dev, unsigned stream_id, cudaStream_t stream) {
+  if (rows <= 0 || cols <= 0) return MMDA_OK;
+  MMDA_REQUIRE(ld >= cols && (size_t)rows * cols <= 0xFFFFFFFFull,
+               "rrelu_forward: ld=%d < cols=%d or more than 2^32 elements", ld, cols);
+  rrelu_fwd_kernel<<<ew_grid((size_t)rows * cols), 256, 0, stream>>>(x, y, ld, rows, cols, seed, seed_dev,
+                                                                     stream_id);
+  MMDA_CHECK_LAUNCH();
+  return MMDA_OK;
+}
+
+int mmda_rrelu_backward(float* dy, const float* y, int ld, int rows, int cols, unsigned long long seed,
+                        const unsigned long long* seed_dev, unsigned stream_id, cudaStream_t stream) {
+  if (rows <= 0 || cols <= 0) return MMDA_OK;
+  MMDA_REQUIRE(ld >= cols && (size_t)rows * cols <= 0xFFFFFFFFull,
+               "rrelu_backward: ld=%d < cols=%d or more than 2^32 elements", ld, cols);
+  rrelu_bwd_kernel<<<ew_grid((size_t)rows * cols), 256, 0, stream>>>(dy, y, ld, rows, cols, seed, seed_dev,
+                                                                     stream_id);
   MMDA_CHECK_LAUNCH();
   return MMDA_OK;
 }

@@ -26,6 +26,10 @@ ENC = {"t": ("trnn1", "trnn2", "tlayer_norm"), "v": ("vrnn1", "vrnn2", "vlayer_n
        "a": ("arnn1", "arnn2", "alayer_norm")}
 PRIV_TAG = {"t": "1", "v": "1", "a": "3"}
 ACT_NONE, ACT_LEAKY, ACT_SIGMOID, ACT_RELU = 0, 1, 2, 3
+ACT_RRELU = ACTIVATIONS["rrelu"]
+# random-number stream ids of training-mode RReLU (+ modality index): project_m, then
+# discriminator_layer_1 on utt_shared_m.  The dropout sites use 1-8, BERT 200 and up.
+SID_RRELU_PROJECT, SID_RRELU_DISC = 9, 12
 LN_EPS = 1e-5
 ATT_P = 0.1            # nn.TransformerEncoderLayer default dropout (reference src/models.py:160)
 NHEAD = 2
@@ -192,6 +196,16 @@ class Kernels:
     def act_bwd(self, dy, y, act):
         self._c("mmda_act_backward", _ptr(dy), dy.stride(0), _ptr(y), y.stride(0), dy.shape[0],
                 dy.shape[1], act)
+
+    def rrelu(self, x, seed, sid, seed_dev=None):
+        """training-mode RReLU in place on the 2-D view x"""
+        self._c("mmda_rrelu_forward", _ptr(x), _ptr(x), x.stride(0), x.shape[0], x.shape[1], seed,
+                _ptr(seed_dev), sid)
+
+    def rrelu_bwd(self, dy, y, seed, sid, seed_dev=None):
+        assert dy.shape == y.shape and dy.stride(0) == y.stride(0)
+        self._c("mmda_rrelu_backward", _ptr(dy), _ptr(y), y.stride(0), y.shape[0], y.shape[1], seed,
+                _ptr(seed_dev), sid)
 
     def add(self, out, x, y=None, ax=1.0, ay=1.0):
         self._c("mmda_add2d", _ptr(out), out.stride(0), _ptr(x), x.stride(0), ax, _ptr(y),
@@ -576,6 +590,10 @@ class MisaEngine:
         p_cls = float(cfg.dropout) if drop else 0.0
         p_att = ATT_P if drop else 0.0
         self.p_cls, self.p_att = p_cls, p_att
+        # nn.RReLU draws its slopes where dropout is on and uses the mean slope otherwise: the
+        # linear then runs without an epilogue and the RReLU pass follows in place
+        self.rrelu_train = bool(drop) and self.act_id == ACT_RRELU
+        act_fwd = ACT_NONE if self.rrelu_train else self.act_id
 
         # ---- encoders on packed rows (three modalities concurrently) ----
         sent = None if self.use_bert else sentences.contiguous()
@@ -622,7 +640,9 @@ class MisaEngine:
         def head_fwd(i, m):
             def run():
                 k.linear(utt[m], P[f"project_{m}.project_{m}.weight"],
-                         P[f"project_{m}.project_{m}.bias"], A[i], act=self.act_id)
+                         P[f"project_{m}.project_{m}.bias"], A[i], act=act_fwd)
+                if self.rrelu_train:
+                    k.rrelu(A[i], seed, SID_RRELU_PROJECT + i, seed_dev)
                 k.layernorm(A[i], None, P[f"project_{m}.project_{m}_layer_norm.weight"],
                             P[f"project_{m}.project_{m}_layer_norm.bias"], O[i], pmu[i], prs[i])
                 tag = PRIV_TAG[m]
@@ -651,7 +671,9 @@ class MisaEngine:
             for i, m in enumerate(MODS):
                 k.linear(X0f[:, (3 + i) * d:(4 + i) * d],
                          P["discriminator.discriminator_layer_1.weight"],
-                         P["discriminator.discriminator_layer_1.bias"], DHp[i], act=self.act_id)
+                         P["discriminator.discriminator_layer_1.bias"], DHp[i], act=act_fwd)
+                if self.rrelu_train:
+                    k.rrelu(DHp[i], seed, SID_RRELU_DISC + i, seed_dev)
                 if p_cls > 0:
                     k.dropout(DHp[i], DH[i], p_cls, seed, 6 + i, seed_dev)
                 else:
@@ -883,7 +905,7 @@ class MisaEngine:
                              G["discriminator.discriminator_layer_2.bias"], dDH, 0.0)
                 if p_cls > 0:
                     k.dropout(dDH, dDH, p_cls, seed, 6 + i, seed_dev)
-                k.act_bwd(dDH, DHp[i], self.act_id)
+                self._act_bwd(dDH, DHp[i], SID_RRELU_DISC + i)
                 dS = self.buf("dSdom", B, d)
                 k.linear_bwd(dDH, X0f[:, (3 + i) * d:(4 + i) * d], w1,
                              G["discriminator.discriminator_layer_1.weight"],
@@ -940,7 +962,7 @@ class MisaEngine:
                                 pmu[i], prs[i], dA[i],
                                 G[f"project_{m}.project_{m}_layer_norm.weight"],
                                 G[f"project_{m}.project_{m}_layer_norm.bias"])
-                k.act_bwd(dA[i], A[i], self.act_id)
+                self._act_bwd(dA[i], A[i], SID_RRELU_PROJECT + i)
                 k.linear_bwd(dA[i], sv["utt"][m], P[f"project_{m}.project_{m}.weight"],
                              G[f"project_{m}.project_{m}.weight"],
                              G[f"project_{m}.project_{m}.bias"], dutt[m], 0.0)
@@ -972,6 +994,14 @@ class MisaEngine:
         k.join_leaves()
         k.leaf_on = False
         return dutt["t"] if self.use_bert else None
+
+    def _act_bwd(self, dy, y, sid):
+        """dy *= act'(y) for config.activation; training-mode RReLU redraws the forward's slopes
+        of random-number stream sid"""
+        if self.rrelu_train:
+            self.k.rrelu_bwd(dy, y, self.cur_seed, sid, self.seed_dev)
+        else:
+            self.k.act_bwd(dy, y, self.act_id)
 
     def _encode_backward(self, m, dutt, G, pk, P, notify, gate):
         """BPTT of both layers of modality m + the hoisted weight-gradient GEMMs.  The recurrence

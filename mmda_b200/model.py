@@ -20,7 +20,8 @@ import torch.nn as nn
 from .config import activation_name
 
 MODS = ("t", "v", "a")
-_TORCH_ACT = {"leakyrelu": nn.LeakyReLU, "relu": nn.ReLU, "tanh": nn.Tanh, "sigmoid": nn.Sigmoid}
+_TORCH_ACT = {"leakyrelu": nn.LeakyReLU, "relu": nn.ReLU, "tanh": nn.Tanh, "sigmoid": nn.Sigmoid,
+              "elu": nn.ELU, "hardshrink": nn.Hardshrink, "hardtanh": nn.Hardtanh, "rrelu": nn.RReLU}
 
 
 class BiLSTMParams(nn.Module):
