@@ -311,6 +311,84 @@ int mmda_loss_grad_misc(const float* scores, const float* tcp, const float* y, c
                         float* dO, int B, int d, int NC, float Bg, float w_recon, float w_conf,
                         mmda_stream_t stream);
 
+/* ---- fixed-order (bit-reproducible) counterparts of the reductions above.  The engine uses
+ * them while torch.are_deterministic_algorithms_enabled() is true; the plain entries keep their
+ * float atomics.  Each takes a device workspace of at least the bytes its *_workspace_bytes query
+ * returns for the same shape (16-byte aligned; contents need no initialisation: every byte read is
+ * written first by the same call).  The result is a function of the inputs, shape and device
+ * model only: independent of CTA timing, of other work on other streams, and of the run. ---- */
+/* out[c] += s[c] over `nparts` partial rows (row pitch ldp), s summed in a fixed order.  split = 0:
+ * out2 (optional) receives the same sums; split > 0: columns c >= split go to out2[c - split]
+ * instead.  The engine sums the three head streams' shared-encoder gradient partials with it
+ * (shared.shared_1, src/models.py:78-80, written by each modality's head, src/models.py:257-259). */
+int mmda_fixed_order_sum(const float* parts, int nparts, long long ldp, int cols, float* out,
+                         float* out2, int split, mmda_stream_t stream);
+/* mmda_colsum with per-CTA partials (a fixed number of rows each) and a fixed-order second pass:
+ * bias gradients of every nn.Linear / nn.LSTM of src/models.py:48-161.  As for every fixed-order
+ * entry whose rows may be padded (LayerNorm, split-K, embedding), zero rows appended at the end
+ * change no bit of the result. */
+long long mmda_colsum_det_workspace_bytes(int rows, int cols);
+int mmda_colsum_det(const float* x, int ld, int rows, int cols, float* out, float* out2,
+                    int out_interleave, float* workspace, mmda_stream_t stream);
+/* mmda_layernorm_backward with per-CTA dgamma / dbeta partials (a fixed number of rows per CTA)
+ * and a fixed-order second pass: the LayerNorms of src/models.py:70,164,160 (project_m, the
+ * encoders' layer norms, the fusion layer's norm1 / norm2); the _dropout form is
+ * mmda_layernorm_backward_dropout's (the BERT encoder's LayerNorms, src/models.py:41-45,186-198)
+ * with the same workspace size. */
+long long mmda_layernorm_backward_det_workspace_bytes(int rows, int width);
+int mmda_layernorm_backward_det(const float* dy, int lddy, const float* x, int ldx, const float* res,
+                                int ldr, const float* gamma, const float* mean, const float* rstd,
+                                float* dx, int lddx, float* dgamma, float* dbeta, int rows, int width,
+                                float* workspace, mmda_stream_t stream);
+int mmda_layernorm_backward_dropout_det(const float* dy, int lddy, const float* x, int ldx,
+                                        const float* res, int ldr, const float* gamma,
+                                        const float* mean, const float* rstd, float* dx, int lddx,
+                                        float* dgamma, float* dbeta, int rows, int width, float* ddrop,
+                                        void* ddrop_bf16, float p, unsigned long long seed,
+                                        const unsigned long long* seed_dev, unsigned stream_id,
+                                        float* workspace, mmda_stream_t stream);
+/* mmda_gemm_tc with mode 1 (C +=): the product is split over K into slices of a fixed number of
+ * K blocks (chosen from M and N only, never from K: split_k is ignored), each slice stored in the
+ * workspace and the slices added in slice order by a second kernel, instead of red.global.add: the
+ * hoisted LSTM weight gradients (src/models.py:48-55,164-175), the fusion FFN's and BERT's.  Zero
+ * rows appended to K change no bit.  mode 0 runs as mmda_gemm_tc with split_k = 1 (no workspace). */
+long long mmda_gemm_tc_det_workspace_bytes(int kind, int M, int N, int K, int mode, int split_k);
+int mmda_gemm_tc_det(int kind, int a_mn, int b_mn, int M, int N, int K, const void* A_hi,
+                     const void* A_lo, int lda, const void* B_hi, const void* B_lo, int ldb,
+                     float alpha, float* C, int ldc, const float* bias, const float* bias2, int mode,
+                     int split_k, int c_row_interleave, float* workspace, mmda_stream_t stream);
+/* mmda_embedding_backward (nn.Embedding, src/models.py:45) as a bucketing of the rows by token id
+ * (integer atomics: order-free counts), each bucket ordered by row index and summed in that order. */
+long long mmda_embedding_backward_det_workspace_bytes(int N, int V);
+int mmda_embedding_backward_det(float* dE, const long long* sentences, const float* dX,
+                                const int* row_t, const int* row_j, const int* sorted_idx, int N,
+                                int B, int D, int V, int* workspace, mmda_stream_t stream);
+/* DiffLoss / CMD chain (src/utils/functions.py:49-78,81-109): mmda_loss_phase2 / _phase4a with
+ * per-CTA partial sums reduced in a fixed order (one workspace size serves both), and
+ * mmda_loss_dxn with each output token's pair terms added in pair order (no atomics). */
+/* mmda_bert_embed_backward (BertEmbeddings, src/models.py:41-45) with the word rows bucketed and
+ * summed as above, the position rows summed over the batch in order, and the token-type rows
+ * through fixed-order chunk partials. */
+long long mmda_bert_embed_backward_det_workspace_bytes(int B, int S, int H, int V);
+int mmda_bert_embed_backward_det(const float* d, const long long* ids, const long long* types, int B,
+                                 int S, int H, int V, float* dword, float* dpos, float* dtyp,
+                                 void* workspace, mmda_stream_t stream);
+/* mmda_sgemm that runs the in-CTA split-K wherever mmda_sgemm would split K over CTAs with
+ * atomics (split_k >= 2, or the auto split of an accumulating product): the dense weight
+ * gradients of src/models.py:61-161.  Every other product runs exactly as in mmda_sgemm. */
+int mmda_sgemm_det(int transA, int transB, int M, int N, int K, float alpha, const float* A, int lda,
+                   const float* B, int ldb, float beta, float* C, int ldc, const float* bias,
+                   const float* bias2, int act, int split_k, int c_row_interleave,
+                   mmda_stream_t stream);
+long long mmda_loss_det_workspace_bytes(int B, int d);
+int mmda_loss_phase2_det(const float* X0, const float* segA, float* XN, float* inv_norm,
+                         float* moments, int B, int d, float Bg, float* workspace,
+                         mmda_stream_t stream);
+int mmda_loss_phase4a_det(float* DXN, const float* inv_norm, float* colsum2, int B, int d,
+                          float* workspace, mmda_stream_t stream);
+int mmda_loss_dxn_det(const float* XN, const float* Gm, float* DXN, int B, int d, float alpha,
+                      mmda_stream_t stream);
+
 /* ---- evaluation metrics on the device: Solver.eval + get_accuracy / get_metrics,
  * src/solver.py:311-370, src/utils/eval.py:14-65.  stats (4 + 3*NC floats, zero before a pass):
  * [0] sum of per-sample |y&p|/max(|y|p|,1), [1] samples, [2] sum of per-batch cls losses,

@@ -164,6 +164,13 @@ class BertEngine:
 
     def _ln_bwd_drop(self, dy, x, res, g, mean, rstd, dx, dg, db, ddrop, ddrop_bf, p, seed, seed_dev,
                      stream_id):
+        if self.k.det:
+            ws = self.k.det_ws("mmda_layernorm_backward_det_workspace_bytes", x.shape[0], x.shape[1])
+            self.k._c("mmda_layernorm_backward_dropout_det", _ptr(dy), dy.stride(0), _ptr(x),
+                      x.stride(0), _ptr(res), res.stride(0), _ptr(g), _ptr(mean), _ptr(rstd), _ptr(dx),
+                      dx.stride(0), _ptr(dg), _ptr(db), x.shape[0], x.shape[1], _ptr(ddrop),
+                      _ptr(ddrop_bf), p, seed, _ptr(seed_dev), stream_id, _ptr(ws))
+            return
         self.k._c("mmda_layernorm_backward_dropout", _ptr(dy), dy.stride(0), _ptr(x), x.stride(0),
                   _ptr(res), res.stride(0), _ptr(g), _ptr(mean), _ptr(rstd), _ptr(dx), dx.stride(0),
                   _ptr(dg), _ptr(db), x.shape[0], x.shape[1], _ptr(ddrop), _ptr(ddrop_bf), p, seed,
@@ -284,6 +291,7 @@ class BertEngine:
         eng, k, H, I, nh = self.eng, self.k, self.H, self.I, self.nh
         P = self.params()
         k.bind_stream()
+        k.det = torch.are_deterministic_algorithms_enabled()
         B, S, mask = sv["B"], sv["S"], sv["mask"]
         M = B * S
         p_h, p_a, seed, seed_dev = sv["p_h"], sv["p_a"], sv["seed"], sv["seed_dev"]
@@ -434,7 +442,12 @@ class BertEngine:
             demb = other
             k.layernorm_bwd(dx, emb, None, P[E + "LayerNorm.weight"], stats[0, 0], stats[0, 1], demb,
                             gw_or(E + "LayerNorm.weight", scr_g), gw_or(E + "LayerNorm.bias", scr_b))
-            k._c("mmda_bert_embed_backward", _ptr(demb), _ptr(sv["ids"]), _ptr(sv["types"]), B, S, H,
-                 self.V, _ptr(gw(E + "word_embeddings.weight")),
-                 _ptr(gw(E + "position_embeddings.weight")),
-                 _ptr(gw(E + "token_type_embeddings.weight")))
+            grads = (_ptr(gw(E + "word_embeddings.weight")), _ptr(gw(E + "position_embeddings.weight")),
+                     _ptr(gw(E + "token_type_embeddings.weight")))
+            if k.det:
+                ws = k.det_ws("mmda_bert_embed_backward_det_workspace_bytes", B, S, H, self.V)
+                k._c("mmda_bert_embed_backward_det", _ptr(demb), _ptr(sv["ids"]), _ptr(sv["types"]), B,
+                     S, H, self.V, *grads, _ptr(ws))
+            else:
+                k._c("mmda_bert_embed_backward", _ptr(demb), _ptr(sv["ids"]), _ptr(sv["types"]), B, S,
+                     H, self.V, *grads)

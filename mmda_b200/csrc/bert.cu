@@ -49,6 +49,50 @@ __global__ void bert_embed_bwd_kernel(const float* __restrict__ d, const long lo
   }
 }
 
+// Fixed-order counterpart (mmda_bert_embed_backward_det).  word: the rows bucketed by token id and
+// each bucket summed in row order (pack.cu); position: dpos[s] += sum over b ascending; token type:
+// per-chunk partials of BERT_DET_ROWS rows, added in chunk order.
+constexpr int BERT_DET_ROWS = 128;
+int embedding_rows_det(float* dE, const float* dX, int N, int D, int V, int* workspace, cudaStream_t stream);
+extern "C" int mmda_fixed_order_sum(const float* parts, int nparts, long long ldp, int cols, float* out,
+                                    float* out2, int split, cudaStream_t stream);
+
+__global__ void bert_word_ids_kernel(const long long* __restrict__ ids, int M, int V, int* __restrict__ out) {
+  const int m = blockIdx.x * blockDim.x + threadIdx.x;
+  if (m < M) out[m] = ids[m] > 0 && ids[m] < V ? (int)ids[m] : -1;     // padding_idx 0: no gradient
+}
+
+__global__ void bert_pos_bwd_det_kernel(const float* __restrict__ d, int B, int S, int H, float* __restrict__ dpos) {
+  const size_t n = (size_t)S * H;
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+    float acc = 0.f;
+    for (int b = 0; b < B; ++b) acc += d[(size_t)b * n + i];
+    dpos[i] += acc;
+  }
+}
+
+// part[chunk][0:H] = sum of the chunk's type-0 rows, part[chunk][H:2H] = type-1 rows
+__global__ void bert_type_partial_kernel(const float* __restrict__ d, const long long* __restrict__ types, int M,
+                                         int H, float* __restrict__ part) {
+  __shared__ float red[2][8][33];
+  const int c = blockIdx.x * 32 + threadIdx.x;
+  const int r_beg = blockIdx.y * BERT_DET_ROWS, r_end = min(M, r_beg + BERT_DET_ROWS);
+  float s0 = 0.f, s1 = 0.f;
+  if (c < H)
+    for (int r = r_beg + threadIdx.y; r < r_end; r += 8) {
+      const float v = d[(size_t)r * H + c];
+      if (types[r] != 0) s1 += v; else s0 += v;
+    }
+  red[0][threadIdx.y][threadIdx.x] = s0;
+  red[1][threadIdx.y][threadIdx.x] = s1;
+  __syncthreads();
+  if (threadIdx.y != 0 || c >= H) return;
+  float t0 = 0.f, t1 = 0.f;
+  for (int w = 0; w < 8; ++w) { t0 += red[0][w][threadIdx.x]; t1 += red[1][w][threadIdx.x]; }
+  part[(size_t)blockIdx.y * 2 * H + c] = t0;
+  part[(size_t)blockIdx.y * 2 * H + H + c] = t1;
+}
+
 // ---------------------------------------------------------------- GELU (erf form) ----------
 __device__ __forceinline__ float gelu_f(float v) {
   return 0.5f * v * (1.f + erff(v * 0.70710678118654752f));
@@ -1325,6 +1369,40 @@ int mmda_bert_embed_backward(const float* d, const long long* ids, const long lo
   MMDA_REQUIRE(B > 0 && S > 0 && H > 0, "bert_embed_backward: bad sizes B=%d S=%d H=%d", B, S, H);
   bert_embed_bwd_kernel<<<B * S, 256, 0, stream>>>(d, ids, types, B * S, S, H, V, dword, dpos, dtyp);
   MMDA_CHECK_LAUNCH();
+  return MMDA_OK;
+}
+
+long long mmda_bert_embed_backward_det_workspace_bytes(int B, int S, int H, int V) {
+  if (B <= 0 || S <= 0 || H <= 0 || V <= 0) return 0;
+  const long long M = (long long)B * S, ints = (2LL * V + 4 * M + 3) / 4 * 4;
+  return ints * (long long)sizeof(int) + (M + BERT_DET_ROWS - 1) / BERT_DET_ROWS * 2 * H * (long long)sizeof(float);
+}
+
+int mmda_bert_embed_backward_det(const float* d, const long long* ids, const long long* types, int B, int S,
+                                 int H, int V, float* dword, float* dpos, float* dtyp, void* workspace,
+                                 cudaStream_t stream) {
+  MMDA_REQUIRE(B > 0 && S > 0 && H > 0 && V > 0 && workspace && (reinterpret_cast<uintptr_t>(workspace) & 15) == 0,
+               "bert_embed_backward_det: bad sizes B=%d S=%d H=%d / workspace", B, S, H);
+  const int M = B * S;
+  int* iws = reinterpret_cast<int*>(workspace);
+  if (dword) {
+    bert_word_ids_kernel<<<(M + 255) / 256, 256, 0, stream>>>(ids, M, V, iws + 2 * V);
+    MMDA_CHECK_LAUNCH();
+    const int rc = embedding_rows_det(dword, d, M, H, V, iws, stream);
+    if (rc != MMDA_OK) return rc;
+  }
+  if (dpos) {
+    size_t g = ((size_t)S * H + 255) / 256;
+    bert_pos_bwd_det_kernel<<<(int)(g > 148 * 8 ? 148 * 8 : g), 256, 0, stream>>>(d, B, S, H, dpos);
+    MMDA_CHECK_LAUNCH();
+  }
+  if (dtyp) {
+    float* part = reinterpret_cast<float*>(iws + (2LL * V + 4LL * M + 3) / 4 * 4);
+    const int chunks = (M + BERT_DET_ROWS - 1) / BERT_DET_ROWS;
+    bert_type_partial_kernel<<<dim3((H + 31) / 32, chunks), dim3(32, 8), 0, stream>>>(d, types, M, H, part);
+    MMDA_CHECK_LAUNCH();
+    return mmda_fixed_order_sum(part, chunks, 2LL * H, 2 * H, dtyp, dtyp + H, H, stream);
+  }
   return MMDA_OK;
 }
 

@@ -112,13 +112,16 @@ dropout_layernorm_fwd_kernel(float* __restrict__ x, int ldx, const float* __rest
 
 // dx = rstd * (dy*g - mean(dy*g) - xhat * mean(dy*g*xhat));  dgamma += sum_r dy*xhat;  dbeta += sum_r dy
 constexpr int LN_MAXC = 20;   // width <= 640 (every MISA norm); 32 -> width <= 1024 (BERT's 768)
-template <int LN_MAXC>
+template <int LN_MAXC, bool PART = false>
 __global__ void __launch_bounds__(256)
 layernorm_bwd_kernel(const float* __restrict__ dy, int lddy, const float* __restrict__ x, int ldx,
                      const float* __restrict__ res, int ldr, const float* __restrict__ gamma,
                      const float* __restrict__ mean, const float* __restrict__ rstd,
                      float* __restrict__ dx, int lddx, float* __restrict__ dgamma,
-                     float* __restrict__ dbeta, int rows, int width, int rows_per_block) {
+                     float* __restrict__ dbeta, int rows, int width, int rows_per_block,
+                     float* __restrict__ part = nullptr) {
+  // part (optional, [gridDim.x][2][width]): this CTA's dgamma | dbeta partials are stored there
+  // instead of added with atomics -- the fixed-order reduction of mmda_layernorm_backward_det
   __shared__ float red[8][33];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int r_beg = blockIdx.x * rows_per_block;
@@ -168,7 +171,10 @@ layernorm_bwd_kernel(const float* __restrict__ dy, int lddy, const float* __rest
         float t = 0.f;
         for (int w = 0; w < 8; ++w) t += red[w][lane];
         const int c = lane + 32 * i;
-        if (c < width) atomicAdd(dgamma + c, t);
+        if (c < width) {
+          if (PART) part[(size_t)blockIdx.x * 2 * width + c] = t;
+          else atomicAdd(dgamma + c, t);
+        }
       }
       __syncthreads();
       red[warp][lane] = ab[i];
@@ -177,7 +183,10 @@ layernorm_bwd_kernel(const float* __restrict__ dy, int lddy, const float* __rest
         float t = 0.f;
         for (int w = 0; w < 8; ++w) t += red[w][lane];
         const int c = lane + 32 * i;
-        if (c < width) atomicAdd(dbeta + c, t);
+        if (c < width) {
+          if (PART) part[(size_t)blockIdx.x * 2 * width + width + c] = t;
+          else atomicAdd(dbeta + c, t);
+        }
       }
     }
   }
@@ -187,7 +196,7 @@ layernorm_bwd_kernel(const float* __restrict__ dy, int lddy, const float* __rest
 // xhat and dy*gamma in registers between the two row reductions and the dx store, so dy / x / res
 // are read once and dx written once (4 x rows x width x 4 B of traffic in all).  Needs width % 4
 // == 0 and 16-byte aligned rows; NV = float4 chunks per lane (width <= 128 * NV).
-template <int NV>
+template <int NV, bool PART = false>
 __global__ void __launch_bounds__(256)
 layernorm_bwd_v4_kernel(const float* __restrict__ dy, int lddy, const float* __restrict__ x, int ldx,
                         const float* __restrict__ res, int ldr, const float* __restrict__ gamma,
@@ -196,7 +205,8 @@ layernorm_bwd_v4_kernel(const float* __restrict__ dy, int lddy, const float* __r
                         float* __restrict__ dbeta, int rows, int width, int rows_per_block,
                         float* __restrict__ ddrop = nullptr, __nv_bfloat16* __restrict__ ddrop_bf16 = nullptr,
                         float p = 0.f, float keep_scale = 1.f, unsigned long long seed = 0,
-                        const unsigned long long* __restrict__ seed_dev = nullptr, unsigned stream = 0) {
+                        const unsigned long long* __restrict__ seed_dev = nullptr, unsigned stream = 0,
+                        float* __restrict__ part = nullptr) {
   // ddrop / ddrop_bf16 (optional, contiguous [rows][width]): dropout(dx) on the stream of the
   // forward's dropout of the tensor this gradient belongs to (element index row * width + col)
   __shared__ float4 red[8][32];
@@ -280,7 +290,10 @@ layernorm_bwd_v4_kernel(const float* __restrict__ dy, int lddy, const float* __r
           float t = 0.f;
 #pragma unroll
           for (int w = 0; w < 8; ++w) t += reinterpret_cast<const float*>(&red[w][lane])[warp];
-          if (c < w4) atomicAdd((which ? dbeta : dgamma) + 4 * c + warp, t);
+          if (c < w4) {
+            if (PART) part[(size_t)blockIdx.x * 2 * width + which * width + 4 * c + warp] = t;
+            else atomicAdd((which ? dbeta : dgamma) + 4 * c + warp, t);
+          }
         }
       }
     }
@@ -293,6 +306,7 @@ layernorm_bwd_v4_kernel(const float* __restrict__ dy, int lddy, const float* __r
 // at a time -- one float4 per thread, the next row's loads in flight while this row's two sums go
 // through a warp shuffle + one shared-memory exchange -- at ~60 registers, so several CTAs share an
 // SM and the loads of a dozen rows overlap.  Same arithmetic, same optional dropped outputs.
+template <bool PART>
 __global__ void __launch_bounds__(256)
 layernorm_bwd_row_kernel(const float* __restrict__ dy, int lddy, const float* __restrict__ x, int ldx,
                          const float* __restrict__ res, int ldr, const float* __restrict__ gamma,
@@ -301,7 +315,8 @@ layernorm_bwd_row_kernel(const float* __restrict__ dy, int lddy, const float* __
                          float* __restrict__ dbeta, int rows, int width, int rows_per_block,
                          float* __restrict__ ddrop, __nv_bfloat16* __restrict__ ddrop_bf16, float p,
                          float keep_scale, unsigned long long seed,
-                         const unsigned long long* __restrict__ seed_dev, unsigned stream) {
+                         const unsigned long long* __restrict__ seed_dev, unsigned stream,
+                         float* __restrict__ part) {
   __shared__ float red[2][8][2];
   if (seed_dev) seed += seed_dev[0] * 0x9E3779B97F4A7C15ULL;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nwarp = blockDim.x >> 5;
@@ -369,7 +384,11 @@ layernorm_bwd_row_kernel(const float* __restrict__ dy, int lddy, const float* __
       }
     }
   }
-  if (act) {     // one atomic per column per CTA
+  if (act && PART) {
+    float* pg = part + (size_t)blockIdx.x * 2 * width + 4 * tid;
+    *reinterpret_cast<float4*>(pg) = ag;
+    *reinterpret_cast<float4*>(pg + width) = ab;
+  } else if (act) {     // one atomic per column per CTA
     atomicAdd(dgamma + 4 * tid + 0, ag.x); atomicAdd(dgamma + 4 * tid + 1, ag.y);
     atomicAdd(dgamma + 4 * tid + 2, ag.z); atomicAdd(dgamma + 4 * tid + 3, ag.w);
     atomicAdd(dbeta + 4 * tid + 0, ab.x); atomicAdd(dbeta + 4 * tid + 1, ab.y);
@@ -381,15 +400,23 @@ static void launch_ln_bwd_row(const float* dy, int lddy, const float* x, int ldx
                               const float* gamma, const float* mean, const float* rstd, float* dx, int lddx,
                               float* dgamma, float* dbeta, int rows, int width, float* ddrop,
                               __nv_bfloat16* ddrop_bf16, float p, unsigned long long seed,
-                              const unsigned long long* seed_dev, unsigned stream_id, cudaStream_t stream) {
+                              const unsigned long long* seed_dev, unsigned stream_id, cudaStream_t stream,
+                              float* part = nullptr, int fixed_rpb = 0) {
   const int threads = ((width / 4) + 31) / 32 * 32;
   int rpb = (rows + 148 * 6 - 1) / (148 * 6);        // ~6 CTAs per SM, each a contiguous run of rows
   if (rpb < 4) rpb = 4;
+  if (fixed_rpb) rpb = fixed_rpb;
   const int grid = (rows + rpb - 1) / rpb;
-  layernorm_bwd_row_kernel<<<grid, threads, 0, stream>>>(dy, lddy, x, ldx, res, ldr, gamma, mean, rstd, dx,
-                                                         lddx, dgamma, dbeta, rows, width, rpb, ddrop,
-                                                         ddrop_bf16, p, 1.f / (1.f - p), seed, seed_dev,
-                                                         stream_id);
+  if (part)
+    layernorm_bwd_row_kernel<true><<<grid, threads, 0, stream>>>(dy, lddy, x, ldx, res, ldr, gamma, mean, rstd,
+                                                                 dx, lddx, dgamma, dbeta, rows, width, rpb, ddrop,
+                                                                 ddrop_bf16, p, 1.f / (1.f - p), seed, seed_dev,
+                                                                 stream_id, part);
+  else
+    layernorm_bwd_row_kernel<false><<<grid, threads, 0, stream>>>(dy, lddy, x, ldx, res, ldr, gamma, mean, rstd,
+                                                                  dx, lddx, dgamma, dbeta, rows, width, rpb, ddrop,
+                                                                  ddrop_bf16, p, 1.f / (1.f - p), seed, seed_dev,
+                                                                  stream_id, nullptr);
 }
 
 // ---------------------------------------------------------------- elementwise ---------------
@@ -424,9 +451,12 @@ __global__ void add2d_kernel(float* __restrict__ out, int ldo, const float* x, i
   }
 }
 // out[c] += sum_r x[r][c]  (and out2 if given): bias gradients
+template <bool PART = false>
 __global__ void colsum_kernel(const float* __restrict__ x, int ld, int rows, int cols,
                               float* __restrict__ out, float* __restrict__ out2,
-                              int rows_per_block, int ilv) {
+                              int rows_per_block, int ilv, float* __restrict__ part = nullptr) {
+  // part (optional, [gridDim.y][cols]): the CTA's column sums are stored there instead of added
+  // with atomics -- the fixed-order reduction of mmda_colsum_det
   __shared__ float red[8][33];
   const int c = blockIdx.x * 32 + threadIdx.x;
   const int r_beg = blockIdx.y * rows_per_block, r_end = min(rows, r_beg + rows_per_block);
@@ -438,10 +468,48 @@ __global__ void colsum_kernel(const float* __restrict__ x, int ld, int rows, int
   if (threadIdx.y == 0 && c < cols) {
     float t = 0.f;
     for (int w = 0; w < 8; ++w) t += red[w][threadIdx.x];
+    if (PART) {
+      part[(size_t)blockIdx.y * cols + c] = t;
+      return;
+    }
     const int co = ilv ? (c & 3) * ilv + (c >> 2) : c;   // gate-interleaved column -> g*H+u
     atomicAdd(out + co, t);
     if (out2) atomicAdd(out2 + co, t);
   }
+}
+
+// Fixed-order sum of per-CTA partial rows: s[c] = sum_y part[y][c], y ascending in eight interleaved
+// lanes that are then added in lane order.  out[co] += s (and out2[co] += s), co = c or the
+// gate-interleaved column; with split > 0, columns c >= split go to out2[c - split] instead.
+__global__ void fixed_order_sum_kernel(const float* __restrict__ part, int nparts, long long ldp, int cols,
+                                       float* __restrict__ out, float* __restrict__ out2, int split,
+                                       int ilv) {
+  __shared__ float red[8][33];
+  const int c = blockIdx.x * 32 + threadIdx.x;
+  float s = 0.f;
+  if (c < cols)
+    for (int y = threadIdx.y; y < nparts; y += 8) s += part[(size_t)y * ldp + c];
+  red[threadIdx.y][threadIdx.x] = s;
+  __syncthreads();
+  if (threadIdx.y != 0 || c >= cols) return;
+  float t = 0.f;
+  for (int w = 0; w < 8; ++w) t += red[w][threadIdx.x];
+  if (split > 0) {
+    if (c < split) out[c] += t;
+    else out2[c - split] += t;
+    return;
+  }
+  const int co = ilv ? (c & 3) * ilv + (c >> 2) : c;
+  out[co] += t;
+  if (out2) out2[co] += t;
+}
+
+static int launch_fixed_order_sum(const float* part, int nparts, long long ldp, int cols, float* out,
+                                  float* out2, int split, int ilv, cudaStream_t stream) {
+  fixed_order_sum_kernel<<<(cols + 31) / 32, dim3(32, 8), 0, stream>>>(part, nparts, ldp, cols, out, out2,
+                                                                      split, ilv);
+  MMDA_CHECK_LAUNCH();
+  return MMDA_OK;
 }
 // inverted dropout; the keep mask is a pure function of (seed, stream, index) so the backward
 // regenerates it instead of storing it
@@ -720,6 +788,14 @@ int mmda_layernorm_backward_dropout(const float* dy, int lddy, const float* x, i
   return MMDA_OK;
 }
 
+static bool ln_bwd_v4(const float* dy, int lddy, const float* x, int ldx, const float* res, int ldr,
+                      const float* gamma, const float* dx, int lddx, int width) {
+  return width % 4 == 0 && lddy % 4 == 0 && ldx % 4 == 0 && lddx % 4 == 0 && (!res || ldr % 4 == 0) &&
+         ((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(x) |
+           reinterpret_cast<uintptr_t>(res) | reinterpret_cast<uintptr_t>(dx) |
+           reinterpret_cast<uintptr_t>(gamma)) & 15) == 0;
+}
+
 int mmda_layernorm_backward(const float* dy, int lddy, const float* x, int ldx, const float* res,
                             int ldr, const float* gamma, const float* mean, const float* rstd,
                             float* dx, int lddx, float* dgamma, float* dbeta, int rows, int width,
@@ -729,11 +805,7 @@ int mmda_layernorm_backward(const float* dy, int lddy, const float* x, int ldx, 
   int rpb = (rows + 295) / 296;
   rpb = (rpb + 7) / 8 * 8;
   const int grid = (rows + rpb - 1) / rpb;
-  const bool v4 = width % 4 == 0 && lddy % 4 == 0 && ldx % 4 == 0 && lddx % 4 == 0 &&
-                  (!res || ldr % 4 == 0) &&
-                  ((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(x) |
-                    reinterpret_cast<uintptr_t>(res) | reinterpret_cast<uintptr_t>(dx) |
-                    reinterpret_cast<uintptr_t>(gamma)) & 15) == 0;
+  const bool v4 = ln_bwd_v4(dy, lddy, x, ldx, res, ldr, gamma, dx, lddx, width);
   if (v4 && width <= 256)
     layernorm_bwd_v4_kernel<2><<<grid, 256, 0, stream>>>(dy, lddy, x, ldx, res, ldr, gamma, mean, rstd,
                                                          dx, lddx, dgamma, dbeta, rows, width, rpb);
@@ -749,6 +821,74 @@ int mmda_layernorm_backward(const float* dy, int lddy, const float* x, int ldx, 
                                                        dx, lddx, dgamma, dbeta, rows, width, rpb);
   MMDA_CHECK_LAUNCH();
   return MMDA_OK;
+}
+
+// Fixed-order plans: a reduction's partition depends on the row index only -- LN_DET_ROWS rows per
+// LayerNorm CTA, COLSUM_DET_ROWS rows per column-sum chunk -- never on the row count.  Rows appended
+// at the end (the zero rows of a padded launch) therefore only append +0 terms: the bits do not
+// depend on how far a batch was padded.
+constexpr int LN_DET_ROWS = 64, COLSUM_DET_ROWS = 128;
+
+long long mmda_layernorm_backward_det_workspace_bytes(int rows, int width) {
+  if (rows <= 0 || width <= 0) return 0;
+  return (long long)((rows + LN_DET_ROWS - 1) / LN_DET_ROWS) * 2 * width * sizeof(float);
+}
+
+// dgamma / dbeta through per-CTA partials (LN_DET_ROWS rows each) and the fixed-order sum; with
+// ddrop / ddrop_bf16 also dropout(dx) as mmda_layernorm_backward_dropout
+static int ln_bwd_det(const float* dy, int lddy, const float* x, int ldx, const float* res, int ldr,
+                      const float* gamma, const float* mean, const float* rstd, float* dx, int lddx,
+                      float* dgamma, float* dbeta, int rows, int width, float* ddrop, __nv_bfloat16* ddrop_bf16,
+                      float p, unsigned long long seed, const unsigned long long* seed_dev, unsigned stream_id,
+                      float* part, cudaStream_t stream) {
+  MMDA_REQUIRE(part && (reinterpret_cast<uintptr_t>(part) & 15) == 0,
+               "layernorm_backward_det: workspace must be 16-byte aligned");
+  const bool v4 = ln_bwd_v4(dy, lddy, x, ldx, res, ldr, gamma, dx, lddx, width);
+  MMDA_REQUIRE(v4 || (!ddrop && !ddrop_bf16), "layernorm_backward_dropout_det: needs 16-byte rows");
+  const int rpb = LN_DET_ROWS, grid = (rows + rpb - 1) / rpb;
+  if (v4 && width <= 256)
+    layernorm_bwd_v4_kernel<2, true><<<grid, 256, 0, stream>>>(dy, lddy, x, ldx, res, ldr, gamma, mean, rstd,
+                                                               dx, lddx, dgamma, dbeta, rows, width, rpb, ddrop,
+                                                               ddrop_bf16, p, 1.f / (1.f - p), seed, seed_dev,
+                                                               stream_id, part);
+  else if (v4)
+    launch_ln_bwd_row(dy, lddy, x, ldx, res, ldr, gamma, mean, rstd, dx, lddx, dgamma, dbeta, rows, width,
+                      ddrop, ddrop_bf16, p, seed, seed_dev, stream_id, stream, part, rpb);
+  else if (width <= 32 * LN_MAXC)
+    layernorm_bwd_kernel<LN_MAXC, true><<<grid, 256, 0, stream>>>(dy, lddy, x, ldx, res, ldr, gamma, mean,
+                                                                  rstd, dx, lddx, dgamma, dbeta, rows,
+                                                                  width, rpb, part);
+  else
+    layernorm_bwd_kernel<32, true><<<grid, 256, 0, stream>>>(dy, lddy, x, ldx, res, ldr, gamma, mean, rstd,
+                                                             dx, lddx, dgamma, dbeta, rows, width, rpb, part);
+  MMDA_CHECK_LAUNCH();
+  return launch_fixed_order_sum(part, grid, 2 * width, 2 * width, dgamma, dbeta, width, 0, stream);
+}
+
+int mmda_layernorm_backward_det(const float* dy, int lddy, const float* x, int ldx, const float* res,
+                                int ldr, const float* gamma, const float* mean, const float* rstd,
+                                float* dx, int lddx, float* dgamma, float* dbeta, int rows, int width,
+                                float* workspace, cudaStream_t stream) {
+  if (rows <= 0) return MMDA_OK;
+  MMDA_REQUIRE(width > 0 && width <= 1024, "layernorm_backward_det: width=%d (max 1024)", width);
+  return ln_bwd_det(dy, lddy, x, ldx, res, ldr, gamma, mean, rstd, dx, lddx, dgamma, dbeta, rows, width,
+                    nullptr, nullptr, 0.f, 0, nullptr, 0, workspace, stream);
+}
+
+int mmda_layernorm_backward_dropout_det(const float* dy, int lddy, const float* x, int ldx, const float* res,
+                                        int ldr, const float* gamma, const float* mean, const float* rstd,
+                                        float* dx, int lddx, float* dgamma, float* dbeta, int rows, int width,
+                                        float* ddrop, void* ddrop_bf16, float p, unsigned long long seed,
+                                        const unsigned long long* seed_dev, unsigned stream_id,
+                                        float* workspace, cudaStream_t stream) {
+  if (rows <= 0) return MMDA_OK;
+  MMDA_REQUIRE(width > 0 && width <= 1024 && width % 4 == 0 && p >= 0.f && p < 1.f,
+               "layernorm_backward_dropout_det: width=%d p=%f", width, p);
+  MMDA_REQUIRE(((reinterpret_cast<uintptr_t>(ddrop)) & 15) == 0 && (reinterpret_cast<uintptr_t>(ddrop_bf16) & 7) == 0,
+               "layernorm_backward_dropout_det: outputs must be aligned");
+  return ln_bwd_det(dy, lddy, x, ldx, res, ldr, gamma, mean, rstd, dx, lddx, dgamma, dbeta, rows, width,
+                    ddrop, reinterpret_cast<__nv_bfloat16*>(ddrop_bf16), p, seed, seed_dev, stream_id,
+                    workspace, stream);
 }
 
 int mmda_act_forward(float* x, int ld, int rows, int cols, int act, cudaStream_t stream) {
@@ -775,18 +915,50 @@ int mmda_add2d(float* out, int ldo, const float* x, int ldx, float ax, const flo
   return MMDA_OK;
 }
 
-int mmda_colsum(const float* x, int ld, int rows, int cols, float* out, float* out2,
-                int out_interleave, cudaStream_t stream) {
-  if (rows <= 0 || cols <= 0) return MMDA_OK;
+static int colsum_plan(int rows, int cols, int* gy_out) {
   const int gx = (cols + 31) / 32;
   int gy = (296 + gx - 1) / gx;
   if (gy > (rows + 7) / 8) gy = (rows + 7) / 8;
   if (gy < 1) gy = 1;
   int rpb = (rows + gy - 1) / gy;
-  gy = (rows + rpb - 1) / rpb;
-  colsum_kernel<<<dim3(gx, gy), dim3(32, 8), 0, stream>>>(x, ld, rows, cols, out, out2, rpb, out_interleave);
+  *gy_out = (rows + rpb - 1) / rpb;
+  return rpb;
+}
+
+int mmda_colsum(const float* x, int ld, int rows, int cols, float* out, float* out2,
+                int out_interleave, cudaStream_t stream) {
+  if (rows <= 0 || cols <= 0) return MMDA_OK;
+  int gy;
+  const int rpb = colsum_plan(rows, cols, &gy);
+  colsum_kernel<<<dim3((cols + 31) / 32, gy), dim3(32, 8), 0, stream>>>(x, ld, rows, cols, out, out2, rpb,
+                                                                        out_interleave);
   MMDA_CHECK_LAUNCH();
   return MMDA_OK;
+}
+
+long long mmda_colsum_det_workspace_bytes(int rows, int cols) {
+  if (rows <= 0 || cols <= 0) return 0;
+  return (long long)((rows + COLSUM_DET_ROWS - 1) / COLSUM_DET_ROWS) * cols * sizeof(float);
+}
+
+int mmda_colsum_det(const float* x, int ld, int rows, int cols, float* out, float* out2,
+                    int out_interleave, float* workspace, cudaStream_t stream) {
+  if (rows <= 0 || cols <= 0) return MMDA_OK;
+  MMDA_REQUIRE(workspace != nullptr, "colsum_det: no workspace");
+  const int gy = (rows + COLSUM_DET_ROWS - 1) / COLSUM_DET_ROWS;
+  colsum_kernel<true><<<dim3((cols + 31) / 32, gy), dim3(32, 8), 0, stream>>>(x, ld, rows, cols, out, out2,
+                                                                              COLSUM_DET_ROWS, out_interleave,
+                                                                              workspace);
+  MMDA_CHECK_LAUNCH();
+  return launch_fixed_order_sum(workspace, gy, cols, cols, out, out2, 0, out_interleave, stream);
+}
+
+int mmda_fixed_order_sum(const float* parts, int nparts, long long ldp, int cols, float* out, float* out2,
+                         int split, cudaStream_t stream) {
+  if (nparts <= 0 || cols <= 0) return MMDA_OK;
+  MMDA_REQUIRE(parts && out && ldp >= cols && split >= 0 && split < cols && (split == 0 || out2),
+               "fixed_order_sum: nparts=%d ldp=%lld cols=%d split=%d", nparts, ldp, cols, split);
+  return launch_fixed_order_sum(parts, nparts, ldp, cols, out, out2, split, 0, stream);
 }
 
 int mmda_dropout(const float* x, float* out, long long n, float p, unsigned long long seed,

@@ -292,6 +292,19 @@ __global__ void zero2d_kernel(float* __restrict__ c, int ldc, int rows, int cols
     c[(i / cols) * ldc + (i % cols)] = 0.f;
 }
 
+// split_k == 0 on an accumulating product (no activation, beta == 1): the auto planner's split count
+static int sgemm_auto_split(int M, int N, int K) {
+  const long big_tiles = (long)((M + 127) / 128) * ((N + 127) / 128);
+  const long med_tiles = (long)((M + 63) / 64) * ((N + 63) / 64);
+  const long small_tiles = (long)((M + 31) / 32) * ((N + 31) / 32);
+  const int cfg = big_tiles >= 120 ? 2 : (med_tiles >= 32 ? 1 : 0);
+  const long tiles = cfg == 2 ? big_tiles : cfg == 1 ? med_tiles : small_tiles;
+  const long want = cfg == 0 ? 592 : 148;       // small tiles: 64-thread CTAs, want several per SM
+  int split_k = 1;
+  while (tiles * split_k < want && K / (split_k * 2) >= 256 && split_k < 32) split_k *= 2;
+  return split_k;
+}
+
 extern "C" int mmda_sgemm(int transA, int transB, int M, int N, int K, float alpha,
                           const float* A, int lda, const float* B, int ldb, float beta, float* C,
                           int ldc, const float* bias, const float* bias2, int act, int split_k,
@@ -314,10 +327,7 @@ extern "C" int mmda_sgemm(int transA, int transB, int M, int N, int K, float alp
     // auto split only where the result is accumulated anyway (gradients); plain forward
     // products stay single-pass so the forward is bitwise reproducible run to run
     const bool can_split = act == ACT_NONE && beta == 1.f;
-    const long tiles = cfg == 2 ? big_tiles : cfg == 1 ? med_tiles : small_tiles;
-    const long want = cfg == 0 ? 592 : 148;       // small tiles: 64-thread CTAs, want several per SM
-    if (can_split)
-      while (tiles * split_k < want && K / (split_k * 2) >= 256 && split_k < 32) split_k *= 2;
+    if (can_split) split_k = sgemm_auto_split(M, N, K);
   }
   MMDA_REQUIRE(split_k == 1 || (act == ACT_NONE && (beta == 1.f || beta == 0.f)),
                "sgemm: split-K accumulates into C (needs beta 0/1, no activation)");
@@ -342,4 +352,22 @@ extern "C" int mmda_sgemm(int transA, int transB, int M, int N, int K, float alp
                                           alpha, beta, act, split_k, c_row_interleave, stream);
   return launch_sgemm<32, 32, 32, 4, 4>(transA, transB, A, B, C, bias, bias2, M, N, K, lda, ldb, ldc,
                                         alpha, beta, act, split_k, c_row_interleave, stream);
+}
+
+// mmda_sgemm where every product that mmda_sgemm would split over grid.z with atomics (split_k >= 2,
+// or the auto split of an accumulating product) runs the in-CTA split-K, whose four K groups are
+// added in a fixed order; every other product runs exactly as in mmda_sgemm.
+extern "C" int mmda_sgemm_det(int transA, int transB, int M, int N, int K, float alpha,
+                              const float* A, int lda, const float* B, int ldb, float beta, float* C,
+                              int ldc, const float* bias, const float* bias2, int act, int split_k,
+                              int c_row_interleave, cudaStream_t stream) {
+  if (M <= 0 || N <= 0) return MMDA_OK;
+  const bool atomic = split_k >= 2 ||
+                      (split_k == 0 && act == ACT_NONE && beta == 1.f && sgemm_auto_split(M, N, K) > 1);
+  if (atomic) {
+    MMDA_REQUIRE(c_row_interleave == 0, "sgemm_det: no fixed-order split-K with an interleaved store");
+    split_k = -1;
+  }
+  return mmda_sgemm(transA, transB, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, bias, bias2, act, split_k,
+                    c_row_interleave, stream);
 }

@@ -105,7 +105,7 @@ struct TcArgs {
   int M, N, K, ldc;
   int a_mn, b_mn;       // 1 = MN-major operand
   float alpha;
-  int mode;             // 0 store, 1 C += , 2 atomic add (split-K)
+  int mode;             // 0 store, 1 C += , 2 atomic add (split-K), 3 store slice z at C + z*M*ldc
   int kb_per_split;     // K blocks per split-K slice
   int c_ilv;            // H: logical C row u*4+g is stored at row g*H+u; 0: identity
 };
@@ -130,7 +130,7 @@ struct TcArgs2 {
   int* sched;          // [0] next tile, [1] finished CTAs (self-resetting)
 };
 
-template <int KIND, int RAW>
+template <int KIND, int RAW, bool SLICES = false>
 __global__ void __launch_bounds__(NUM_THREADS + (RAW ? 128 : 0), 1)
 gemm_tc2_kernel(const __grid_constant__ CUtensorMap mapAh, const __grid_constant__ CUtensorMap mapAl,
                 const __grid_constant__ CUtensorMap mapBh, const __grid_constant__ CUtensorMap mapBl,
@@ -417,7 +417,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap mapAh, const __grid_constant
         const int grow = m0 + q * 32 + lane;
         const bool row_ok = grow < p.M;
         const int row_out = p.c_ilv ? (grow & 3) * p.c_ilv + (grow >> 2) : grow;
-        float* crow = p.C + (size_t)row_out * p.ldc;
+        float* crow = SLICES ? p.C + ((size_t)z * p.M + row_out) * p.ldc : p.C + (size_t)row_out * p.ldc;
         const bool vec_ok = (p.ldc & 3) == 0 && ((uintptr_t)p.C & 15) == 0;
 #pragma unroll
         for (int cc = 0; cc < BN / 32; ++cc) {
@@ -438,7 +438,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap mapAh, const __grid_constant
                 v.x += b4.x; v.y += b4.y; v.z += b4.z; v.w += b4.w;
               }
               float* cp = crow + nb + j;
-              if (p.mode != 0) {
+              if (!SLICES && p.mode != 0) {
                 asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(cp), "f"(v.x),
                              "f"(v.y), "f"(v.z), "f"(v.w)
                              : "memory");
@@ -456,7 +456,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap mapAh, const __grid_constant
                   if (p.bias) v += p.bias[col];
                   if (p.bias2) v += p.bias2[col];
                 }
-                if (p.mode != 0) atomicAdd(crow + col, v);
+                if (!SLICES && p.mode != 0) atomicAdd(crow + col, v);
                 else crow[col] = v;
               }
             }
@@ -675,13 +675,67 @@ int mmda_cast_bf16(const float* x, int ldx, int rows, int cols, void* out, int l
   return MMDA_OK;
 }
 
+}  // extern "C"
+
+namespace {
+
+// split_k <= 0: auto -- fill the chip for long-K problems.  Depends on the shape and mode only.
+int plan_split_k(int esz, int M, int N, int K, int mode, int split_k) {
+  const int BK = 128 / esz;
+  const int kb_total = (K + BK - 1) / BK;
+  const int tiles = ((M + BM - 1) / BM) * ((N + BN - 1) / BN);
+  if (split_k <= 0) {
+    split_k = 1;
+    while (tiles * split_k < 148 && kb_total / (split_k * 2) >= 8 && split_k < 32) split_k *= 2;
+    // bound the per-accumulator chain (fp32 accumulation in the tensor core truncates)
+    while (mode == 1 && (long)kb_total * BK / split_k > 2048 && split_k < 64) split_k *= 2;
+  }
+  if (split_k > kb_total) split_k = kb_total;
+  return split_k;
+}
+
+// Fixed-order split-K plan: a fixed number of K blocks per slice, chosen from the output tiles (so
+// that a short output still spreads over the chip) and never from K.  K beyond the real rows (the
+// zero rows of a padded launch) then only adds +0 products and +0 slices: the bits do not depend on
+// how far the contraction was padded.
+int det_kb_per_split(int esz, int M, int N) {
+  const int tiles = ((M + BM - 1) / BM) * ((N + BN - 1) / BN);
+  const int chain = 2048 / (128 / esz);          // the per-accumulator chain bound of plan_split_k
+  const int kps = tiles < 74 ? 32 : 64;
+  return kps < chain ? kps : chain;
+}
+
+template <int KIND, int RAW, bool SLICES>
+int launch_tc2(const CUtensorMap& mAh, const CUtensorMap& mAl, const CUtensorMap& mBh, const CUtensorMap& mBl,
+               const TcArgs2& a2, int ctas, int smem, cudaStream_t stream) {
+  MMDA_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<KIND, RAW, SLICES>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  gemm_tc2_kernel<KIND, RAW, SLICES><<<ctas, NUM_THREADS + (RAW ? 128 : 0), smem, stream>>>(mAh, mAl, mBh, mBl, a2);
+  return MMDA_OK;
+}
+
+// C[row_out][c] (+)= sum_z slices[z][r][c], z ascending (the fixed-order split-K reduction)
+__global__ void splitk_reduce_kernel(const float* __restrict__ slices, int split, int M, int N, int ldw,
+                                     float* __restrict__ C, int ldc, int c_ilv, int accumulate) {
+  const size_t n = (size_t)M * N, zs = (size_t)M * ldw;
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+    const int r = (int)(i / N), c = (int)(i % N);
+    const float* sp = slices + (size_t)r * ldw + c;
+    float s = sp[0];
+    for (int z = 1; z < split; ++z) s += sp[z * zs];
+    const int ro = c_ilv ? (r & 3) * c_ilv + (r >> 2) : r;
+    float* cp = C + (size_t)ro * ldc + c;
+    *cp = accumulate ? *cp + s : s;
+  }
+}
+
 // kind 0: A_hi/A_lo/B_hi/B_lo are fp32 (tf32 split); kind 1: A_hi/B_hi are bf16, *_lo ignored.
 // a_mn / b_mn = 0: operand stored [MN][K] (K contiguous); 1: stored [K][MN] (MN contiguous).
 // mode 0: C = ..., 1: C += ...; split_k > 1 accumulates with atomics (C must be initialised).
-int mmda_gemm_tc(int kind, int a_mn, int b_mn, int M, int N, int K, const void* A_hi,
+// With slices (mode 1 only): det_kps K blocks per slice, slices stored and added in order.
+int gemm_tc_impl(int kind, int a_mn, int b_mn, int M, int N, int K, const void* A_hi,
                  const void* A_lo, int lda, const void* B_hi, const void* B_lo, int ldb, float alpha,
                  float* C, int ldc, const float* bias, const float* bias2, int mode, int split_k,
-                 int c_row_interleave, cudaStream_t stream) {
+                 int c_row_interleave, float* slices, int det_kps, cudaStream_t stream) {
   if (M <= 0 || N <= 0) return MMDA_OK;
   // kind 2: 3xTF32 from plain fp32 operands (A_hi / B_hi point at the fp32 data, the lo pointers
   // are ignored); the hi/lo split happens in shared memory inside the kernel
@@ -713,21 +767,19 @@ int mmda_gemm_tc(int kind, int a_mn, int b_mn, int M, int N, int K, const void* 
   if ((rc = enc(&mBl, kind == 0 ? B_lo : B_hi, b_mn, N, ldb)) != MMDA_OK) return rc;
 
   const int kb_total = (K + BK - 1) / BK;
-  const int tiles = ((M + BM - 1) / BM) * ((N + BN - 1) / BN);
-  if (split_k <= 0) {   // auto: fill the chip for long-K problems
-    split_k = 1;
-    while (tiles * split_k < 148 && kb_total / (split_k * 2) >= 8 && split_k < 32) split_k *= 2;
-    // bound the per-accumulator chain (fp32 accumulation in the tensor core truncates)
-    while (mode == 1 && (long)kb_total * BK / split_k > 2048 && split_k < 64) split_k *= 2;
-  }
-  if (split_k > kb_total) split_k = kb_total;
+  split_k = slices ? (kb_total + det_kps - 1) / det_kps : plan_split_k(esz, M, N, K, mode, split_k);
   MMDA_REQUIRE(split_k == 1 || mode == 1, "gemm_tc: split-K accumulates into C (mode must be 1)");
   TcArgs a;
   a.C = C; a.bias = bias; a.bias2 = bias2; a.M = M; a.N = N; a.K = K; a.ldc = ldc;
   a.a_mn = a_mn; a.b_mn = b_mn; a.alpha = alpha;
   a.mode = split_k > 1 ? 2 : mode;
-  a.kb_per_split = (kb_total + split_k - 1) / split_k;
+  a.kb_per_split = slices ? det_kps : (kb_total + split_k - 1) / split_k;
   a.c_ilv = c_row_interleave;
+  if (slices != nullptr) {
+    // fixed-order split-K: slice z of the product goes to slices[z] ([M][ldw], plain rows); the
+    // reduction kernel adds the slices in z order and applies the row interleave
+    a.C = slices; a.ldc = (N + 3) / 4 * 4; a.mode = 3; a.c_ilv = 0;
+  }
   TcArgs2 a2;
   a2.a = a;
   a2.tiles_m = (M + BM - 1) / BM; a2.tiles_n = (N + BN - 1) / BN; a2.split = split_k;
@@ -739,21 +791,70 @@ int mmda_gemm_tc(int kind, int a_mn, int b_mn, int M, int N, int K, const void* 
   const int n_sm = ctx->sm_count;
   const int ctas = a2.total < n_sm ? a2.total : n_sm;
   constexpr int smem2 = 12 * TILE_BYTES + 1024 + 512 + 4 * 32 * 33 * 4;
-  if (kind == 0 && raw_mode == 1) {
-    MMDA_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
-    gemm_tc2_kernel<0, 1><<<ctas, NUM_THREADS + 128, smem2, stream>>>(mAh, mAl, mBh, mBl, a2);
-  } else if (kind == 0 && raw_mode == 2) {
-    MMDA_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<0, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
-    gemm_tc2_kernel<0, 2><<<ctas, NUM_THREADS + 128, smem2, stream>>>(mAh, mAl, mBh, mBl, a2);
-  } else if (kind == 0) {
-    MMDA_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
-    gemm_tc2_kernel<0, 0><<<ctas, NUM_THREADS, smem2, stream>>>(mAh, mAl, mBh, mBl, a2);
-  } else {
-    MMDA_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
-    gemm_tc2_kernel<1, 0><<<ctas, NUM_THREADS, smem2, stream>>>(mAh, mAl, mBh, mBl, a2);
-  }
+  const bool sl = a.mode == 3;
+  if (kind == 0 && raw_mode == 1)
+    rc = sl ? launch_tc2<0, 1, true>(mAh, mAl, mBh, mBl, a2, ctas, smem2, stream)
+            : launch_tc2<0, 1, false>(mAh, mAl, mBh, mBl, a2, ctas, smem2, stream);
+  else if (kind == 0 && raw_mode == 2)
+    rc = sl ? launch_tc2<0, 2, true>(mAh, mAl, mBh, mBl, a2, ctas, smem2, stream)
+            : launch_tc2<0, 2, false>(mAh, mAl, mBh, mBl, a2, ctas, smem2, stream);
+  else if (kind == 0)
+    rc = sl ? launch_tc2<0, 0, true>(mAh, mAl, mBh, mBl, a2, ctas, smem2, stream)
+            : launch_tc2<0, 0, false>(mAh, mAl, mBh, mBl, a2, ctas, smem2, stream);
+  else
+    rc = sl ? launch_tc2<1, 0, true>(mAh, mAl, mBh, mBl, a2, ctas, smem2, stream)
+            : launch_tc2<1, 0, false>(mAh, mAl, mBh, mBl, a2, ctas, smem2, stream);
+  if (rc != MMDA_OK) return rc;
   MMDA_CHECK_LAUNCH();
+  if (slices != nullptr) {
+    const size_t n = (size_t)M * N;
+    size_t g = (n + 255) / 256;
+    if (g > 148 * 2) g = 148 * 2;
+    splitk_reduce_kernel<<<(int)g, 256, 0, stream>>>(slices, split_k, M, N, (N + 3) / 4 * 4, C, ldc,
+                                                     c_row_interleave, mode);
+    MMDA_CHECK_LAUNCH();
+  }
   return MMDA_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int mmda_gemm_tc(int kind, int a_mn, int b_mn, int M, int N, int K, const void* A_hi,
+                 const void* A_lo, int lda, const void* B_hi, const void* B_lo, int ldb, float alpha,
+                 float* C, int ldc, const float* bias, const float* bias2, int mode, int split_k,
+                 int c_row_interleave, cudaStream_t stream) {
+  return gemm_tc_impl(kind, a_mn, b_mn, M, N, K, A_hi, A_lo, lda, B_hi, B_lo, ldb, alpha, C, ldc, bias,
+                      bias2, mode, split_k, c_row_interleave, nullptr, 0, stream);
+}
+
+static int det_slices(int kind, int M, int N, int K) {
+  const int esz = kind == 1 ? 2 : 4, kb_total = (K + 128 / esz - 1) / (128 / esz);
+  const int kps = det_kb_per_split(esz, M, N);
+  return (kb_total + kps - 1) / kps;
+}
+
+long long mmda_gemm_tc_det_workspace_bytes(int kind, int M, int N, int K, int mode, int split_k) {
+  (void)split_k;
+  if (M <= 0 || N <= 0 || K <= 0 || mode != 1) return 0;
+  return (long long)det_slices(kind, M, N, K) * M * ((N + 3) / 4 * 4) * (long long)sizeof(float);
+}
+
+int mmda_gemm_tc_det(int kind, int a_mn, int b_mn, int M, int N, int K, const void* A_hi,
+                     const void* A_lo, int lda, const void* B_hi, const void* B_lo, int ldb, float alpha,
+                     float* C, int ldc, const float* bias, const float* bias2, int mode, int split_k,
+                     int c_row_interleave, float* workspace, cudaStream_t stream) {
+  if (M <= 0 || N <= 0) return MMDA_OK;
+  MMDA_REQUIRE(K > 0, "gemm_tc_det: K=%d", K);
+  if (mode != 1)      // a plain store: one pass over K, nothing to reduce
+    return gemm_tc_impl(kind, a_mn, b_mn, M, N, K, A_hi, A_lo, lda, B_hi, B_lo, ldb, alpha, C, ldc, bias,
+                        bias2, mode, 1, c_row_interleave, nullptr, 0, stream);
+  MMDA_REQUIRE(workspace && (reinterpret_cast<uintptr_t>(workspace) & 15) == 0,
+               "gemm_tc_det: needs a 16-byte aligned workspace");
+  return gemm_tc_impl(kind, a_mn, b_mn, M, N, K, A_hi, A_lo, lda, B_hi, B_lo, ldb, alpha, C, ldc, bias,
+                      bias2, mode, split_k, c_row_interleave, workspace,
+                      det_kb_per_split(kind == 1 ? 2 : 4, M, N), stream);
 }
 
 }  // extern "C"

@@ -22,6 +22,8 @@
 #include "common.cuh"
 
 constexpr int LOSS_MAXC = 8;   // d <= 256
+extern "C" int mmda_fixed_order_sum(const float* parts, int nparts, long long ldp, int cols, float* out,
+                                    float* out2, int split, cudaStream_t stream);
 constexpr int NTOK = 6;
 
 __device__ __forceinline__ float block_sum_256(float v, float* red) {
@@ -97,10 +99,14 @@ loss_phase1_kernel(const float* __restrict__ X0, const float* __restrict__ O,
   }
 }
 
+template <bool PART = false>
 __global__ void __launch_bounds__(256)
 loss_phase2_kernel(const float* __restrict__ X0, const float* __restrict__ segA,
                    float* __restrict__ XN, float* __restrict__ inv_norm,
-                   float* __restrict__ moments, int B, int d, float Bg, int rows_per_block) {
+                   float* __restrict__ moments, int B, int d, float Bg, int rows_per_block,
+                   float* __restrict__ part = nullptr) {
+  // part (optional, [gridDim.y][12][d]): the CTA's moment sums are stored there instead of added
+  // with atomics -- the fixed-order reduction of mmda_loss_phase2_det
   __shared__ float red[8][33];
   const int i = blockIdx.x;   // token
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -149,7 +155,11 @@ loss_phase2_kernel(const float* __restrict__ X0, const float* __restrict__ segA,
             float t = 0.f;
             for (int w = 0; w < 8; ++w) t += red[w][lane];
             const int c = lane + 32 * m;
-            if (c < d) atomicAdd(moments + ((size_t)(i - 3) * 4 + k) * d + c, t);
+            if (c < d) {
+              const size_t o = ((size_t)(i - 3) * 4 + k) * d + c;
+              if (PART) part[(size_t)blockIdx.y * 12 * d + o] = t;
+              else atomicAdd(moments + o, t);
+            }
           }
         }
       }
@@ -252,9 +262,11 @@ loss_finalize_kernel(const float* __restrict__ segA, const float* __restrict__ s
   }
 }
 
+template <bool PART = false>
 __global__ void __launch_bounds__(256)
 loss_phase4a_kernel(float* __restrict__ DXN, const float* __restrict__ inv_norm,
-                    float* __restrict__ colsum2, int B, int d, int rows_per_block) {
+                    float* __restrict__ colsum2, int B, int d, int rows_per_block,
+                    float* __restrict__ part = nullptr) {
   __shared__ float red[8][33];
   const int i = blockIdx.x;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -281,7 +293,10 @@ loss_phase4a_kernel(float* __restrict__ DXN, const float* __restrict__ inv_norm,
         float t = 0.f;
         for (int w = 0; w < 8; ++w) t += red[w][lane];
         const int c = lane + 32 * m;
-        if (c < d) atomicAdd(colsum2 + i * d + c, t);
+        if (c < d) {
+          if (PART) part[(size_t)blockIdx.y * NTOK * d + i * d + c] = t;
+          else atomicAdd(colsum2 + i * d + c, t);
+        }
       }
     }
   }
@@ -414,6 +429,30 @@ int mmda_loss_phase2(const float* X0, const float* segA, float* XN, float* inv_n
   return MMDA_OK;
 }
 
+static int loss_row_chunks(int B, int* rpb_out) {
+  int rpb = (B + 23) / 24;
+  rpb = (rpb + 7) / 8 * 8;
+  *rpb_out = rpb;
+  return (B + rpb - 1) / rpb;
+}
+
+long long mmda_loss_det_workspace_bytes(int B, int d) {
+  if (B <= 0 || d <= 0) return 0;
+  const long long chunks = (B + 7) / 8 < 24 ? (B + 7) / 8 : 24;     // >= loss_row_chunks(B), monotone in B
+  return chunks * 12 * d * (long long)sizeof(float);
+}
+
+int mmda_loss_phase2_det(const float* X0, const float* segA, float* XN, float* inv_norm,
+                         float* moments, int B, int d, float Bg, float* workspace, cudaStream_t stream) {
+  MMDA_REQUIRE(B > 0 && d > 0 && d <= 32 * LOSS_MAXC && workspace, "loss_phase2_det: B=%d d=%d", B, d);
+  int rpb;
+  const int gy = loss_row_chunks(B, &rpb);
+  loss_phase2_kernel<true><<<dim3(NTOK, gy), 256, 0, stream>>>(X0, segA, XN, inv_norm, moments, B, d, Bg,
+                                                                rpb, workspace);
+  MMDA_CHECK_LAUNCH();
+  return mmda_fixed_order_sum(workspace, gy, 12LL * d, 12 * d, moments, nullptr, 0, stream);
+}
+
 int mmda_loss_finalize(const float* segA, const float* segB, float* losses, float* coef, int d,
                        int NC, float Bg, float w_diff, float w_sim, float w_recon, float w_conf,
                        int adversarial, int mode, cudaStream_t stream) {
@@ -433,6 +472,16 @@ int mmda_loss_phase4a(float* DXN, const float* inv_norm, float* colsum2, int B, 
   loss_phase4a_kernel<<<grid, 256, 0, stream>>>(DXN, inv_norm, colsum2, B, d, rpb);
   MMDA_CHECK_LAUNCH();
   return MMDA_OK;
+}
+
+int mmda_loss_phase4a_det(float* DXN, const float* inv_norm, float* colsum2, int B, int d,
+                          float* workspace, cudaStream_t stream) {
+  MMDA_REQUIRE(B > 0 && d > 0 && d <= 32 * LOSS_MAXC && workspace, "loss_phase4a_det: B=%d d=%d", B, d);
+  int rpb;
+  const int gy = loss_row_chunks(B, &rpb);
+  loss_phase4a_kernel<true><<<dim3(NTOK, gy), 256, 0, stream>>>(DXN, inv_norm, colsum2, B, d, rpb, workspace);
+  MMDA_CHECK_LAUNCH();
+  return mmda_fixed_order_sum(workspace, gy, (long long)NTOK * d, NTOK * d, colsum2, nullptr, 0, stream);
 }
 
 int mmda_loss_phase4b(const float* X0, const float* DXN, const float* segA, const float* segB,
@@ -563,17 +612,11 @@ __global__ void __launch_bounds__(256) loss_gram_kernel(const float* __restrict_
   }
 }
 
-// One CTA per (output token x, pair p it takes part in, 32 x 32 output tile): 12 (x, p) slots, each a
-// K = d contraction, accumulated into the zeroed DXN with atomics (a private token sits in three
-// pairs; walking them inside one CTA tripled the length of the chain: 30 -> 12 us).
-__global__ void __launch_bounds__(256) loss_dxn_kernel(const float* __restrict__ XN, const float* __restrict__ Gm,
-                                                       float* __restrict__ DXN, int B, int d, float alpha) {
-  __shared__ float Xs[32][33], Gs[32][33];
-  const int p = blockIdx.z >> 1, is_a = (blockIdx.z & 1) == 0;
-  const int x = is_a ? c_pair_a[p] : c_pair_b[p];
-  const int b0 = blockIdx.y * 32, i0 = blockIdx.x * 32;
+// acc[r] = (slot's product)[b0 + ty*4 + r][i0 + tx] for slot (pair p, a side or b side)
+__device__ __forceinline__ void dxn_tile(const float* __restrict__ XN, const float* __restrict__ Gm, int B,
+                                         int d, int p, int is_a, int b0, int i0, float (&Xs)[32][33],
+                                         float (&Gs)[32][33], float (&acc)[4]) {
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
-  float acc[4] = {0.f, 0.f, 0.f, 0.f};
   const float* X = XN + (size_t)(is_a ? c_pair_b[p] : c_pair_a[p]) * B * d;
   const float* G = Gm + (size_t)p * d * d;
   for (int j0 = 0; j0 < d; j0 += 32) {
@@ -596,10 +639,49 @@ __global__ void __launch_bounds__(256) loss_dxn_kernel(const float* __restrict__
     }
     __syncthreads();
   }
+}
+
+// One CTA per (output token x, pair p it takes part in, 32 x 32 output tile): 12 (x, p) slots, each a
+// K = d contraction, accumulated into the zeroed DXN with atomics (a private token sits in three
+// pairs; walking them inside one CTA tripled the length of the chain: 30 -> 12 us).
+__global__ void __launch_bounds__(256) loss_dxn_kernel(const float* __restrict__ XN, const float* __restrict__ Gm,
+                                                       float* __restrict__ DXN, int B, int d, float alpha) {
+  __shared__ float Xs[32][33], Gs[32][33];
+  const int p = blockIdx.z >> 1, is_a = (blockIdx.z & 1) == 0;
+  const int x = is_a ? c_pair_a[p] : c_pair_b[p];
+  const int b0 = blockIdx.y * 32, i0 = blockIdx.x * 32;
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  float acc[4] = {0.f, 0.f, 0.f, 0.f};
+  dxn_tile(XN, Gm, B, d, p, is_a, b0, i0, Xs, Gs, acc);
 #pragma unroll
   for (int r = 0; r < 4; ++r) {
     const int b = b0 + ty * 4 + r, i = i0 + tx;
     if (b < B && i < d) atomicAdd(DXN + ((size_t)x * B + b) * d + i, alpha * acc[r]);
+  }
+}
+
+// Fixed-order variant: one CTA per (output token x, 32 x 32 tile) walks the slots x takes part in,
+// pair order, and stores the sum (no atomics, no zero-fill)
+__global__ void __launch_bounds__(256) loss_dxn_det_kernel(const float* __restrict__ XN,
+                                                           const float* __restrict__ Gm,
+                                                           float* __restrict__ DXN, int B, int d, float alpha) {
+  __shared__ float Xs[32][33], Gs[32][33];
+  const int x = blockIdx.z;
+  const int b0 = blockIdx.y * 32, i0 = blockIdx.x * 32;
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  float sum[4] = {0.f, 0.f, 0.f, 0.f};
+  for (int slot = 0; slot < 12; ++slot) {
+    const int p = slot >> 1, is_a = (slot & 1) == 0;
+    if ((is_a ? c_pair_a[p] : c_pair_b[p]) != x) continue;      // block-uniform
+    float acc[4] = {0.f, 0.f, 0.f, 0.f};
+    dxn_tile(XN, Gm, B, d, p, is_a, b0, i0, Xs, Gs, acc);
+#pragma unroll
+    for (int r = 0; r < 4; ++r) sum[r] += alpha * acc[r];
+  }
+#pragma unroll
+  for (int r = 0; r < 4; ++r) {
+    const int b = b0 + ty * 4 + r, i = i0 + tx;
+    if (b < B && i < d) DXN[((size_t)x * B + b) * d + i] = sum[r];
   }
 }
 
@@ -681,6 +763,15 @@ extern "C" int mmda_linear_skinny(const float* x, int ldx, const float* w, const
                                   int ldy, int M, int N, int K, int act, cudaStream_t stream) {
   MMDA_REQUIRE(M > 0 && K > 0 && N >= 1 && N <= 8, "linear_skinny: M=%d N=%d K=%d (N <= 8)", M, N, K);
   linear_skinny_kernel<8><<<(M + 7) / 8, 256, 0, stream>>>(x, ldx, w, bias, y, ldy, M, N, K, act);
+  MMDA_CHECK_LAUNCH();
+  return MMDA_OK;
+}
+
+extern "C" int mmda_loss_dxn_det(const float* XN, const float* Gm, float* DXN, int B, int d, float alpha,
+                                 cudaStream_t stream) {
+  MMDA_REQUIRE(B > 0 && d > 0, "loss_dxn_det: B=%d d=%d", B, d);
+  dim3 grid((d + 31) / 32, (B + 31) / 32, NTOK);
+  loss_dxn_det_kernel<<<grid, 256, 0, stream>>>(XN, Gm, DXN, B, d, alpha);
   MMDA_CHECK_LAUNCH();
   return MMDA_OK;
 }

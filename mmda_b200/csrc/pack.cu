@@ -101,6 +101,96 @@ __global__ void embedding_bwd_kernel(float* __restrict__ dE, const long long* __
   for (int c = threadIdx.x; c < D; c += blockDim.x) atomicAdd(d + c, s[c]);
 }
 
+// ---- fixed-order embedding backward: rows bucketed by token id, each bucket summed in row order ----
+// workspace (ints): count[V] | start[V] | id[N] | slot[N] | list[N] | sorted[N]
+__global__ void emb_det_ids_kernel(const long long* __restrict__ sent, const int* __restrict__ row_t,
+                                   const int* __restrict__ row_j, const int* __restrict__ sorted_idx,
+                                   int N, int B, int V, int* __restrict__ ids) {
+  const int row = blockIdx.x * blockDim.x + threadIdx.x;
+  if (row >= N) return;
+  const long long id = sent[(size_t)row_t[row] * B + sorted_idx[row_j[row]]];
+  ids[row] = id >= 0 && id < V ? (int)id : -1;
+}
+
+__global__ void emb_det_count_kernel(const int* __restrict__ ids, int N, int* __restrict__ count,
+                                     int* __restrict__ slot) {
+  const int row = blockIdx.x * blockDim.x + threadIdx.x;
+  if (row >= N) return;
+  const int id = ids[row];
+  slot[row] = id >= 0 ? atomicAdd(count + id, 1) : -1;     // integer: the counts are order-free
+}
+
+// exclusive scan of count[V] -> start[V]: one CTA, each thread a contiguous run
+__global__ void __launch_bounds__(1024) emb_det_scan_kernel(const int* __restrict__ count,
+                                                            int* __restrict__ start, int V) {
+  __shared__ int part[1024];
+  const int per = (V + 1023) / 1024, b = threadIdx.x * per, e = min(V, b + per);
+  int s = 0;
+  for (int v = b; v < e; ++v) s += count[v];
+  part[threadIdx.x] = s;
+  __syncthreads();
+  for (int off = 1; off < 1024; off <<= 1) {     // Hillis-Steele inclusive scan
+    const int t = threadIdx.x >= off ? part[threadIdx.x - off] : 0;
+    __syncthreads();
+    part[threadIdx.x] += t;
+    __syncthreads();
+  }
+  int run = threadIdx.x ? part[threadIdx.x - 1] : 0;
+  for (int v = b; v < e; ++v) { start[v] = run; run += count[v]; }
+}
+
+__global__ void emb_det_place_kernel(const int* __restrict__ ids, const int* __restrict__ slot,
+                                     const int* __restrict__ start, int N, int* __restrict__ list) {
+  const int row = blockIdx.x * blockDim.x + threadIdx.x;
+  if (row < N && ids[row] >= 0) list[start[ids[row]] + slot[row]] = row;
+}
+
+// one CTA per token id (grid-stride): order the bucket by row index (rank = number of smaller rows;
+// the bucket's rows are distinct), then dE[v][c] += sum of dX[row][c] over the bucket in row order
+__global__ void __launch_bounds__(256) emb_det_reduce_kernel(float* __restrict__ dE, const float* __restrict__ dX,
+                                                             const int* __restrict__ count,
+                                                             const int* __restrict__ start,
+                                                             const int* __restrict__ list,
+                                                             int* __restrict__ sorted, int V, int D) {
+  for (int v = blockIdx.x; v < V; v += gridDim.x) {
+    const int n = count[v];
+    if (n == 0) continue;
+    const int s0 = start[v];
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+      const int r = list[s0 + i];
+      int rank = 0;
+      for (int j = 0; j < n; ++j) rank += list[s0 + j] < r;
+      sorted[s0 + rank] = r;
+    }
+    __syncthreads();
+    for (int c = threadIdx.x; c < D; c += blockDim.x) {
+      float acc = 0.f;
+      for (int j = 0; j < n; ++j) acc += dX[(size_t)sorted[s0 + j] * D + c];
+      dE[(size_t)v * D + c] += acc;
+    }
+    __syncthreads();
+  }
+}
+
+// dE[ids[r]][:] += dX[r][:] (ids[r] < 0: skipped) with each id's rows summed in row order.  The
+// caller has written ids[N] at workspace + 2V (mmda_embedding_backward_det's layout); shared with
+// the BERT embedding backward (bert.cu).
+int embedding_rows_det(float* dE, const float* dX, int N, int D, int V, int* workspace, cudaStream_t stream) {
+  int *count = workspace, *start = count + V, *ids = start + V, *slot = ids + N, *list = slot + N,
+      *sorted = list + N;
+  MMDA_CUDA(cudaMemsetAsync(count, 0, (size_t)V * sizeof(int), stream));
+  emb_det_count_kernel<<<(N + 255) / 256, 256, 0, stream>>>(ids, N, count, slot);
+  MMDA_CHECK_LAUNCH();
+  emb_det_scan_kernel<<<1, 1024, 0, stream>>>(count, start, V);
+  MMDA_CHECK_LAUNCH();
+  emb_det_place_kernel<<<(N + 255) / 256, 256, 0, stream>>>(ids, slot, start, N, list);
+  MMDA_CHECK_LAUNCH();
+  emb_det_reduce_kernel<<<V < 148 * 8 ? V : 148 * 8, 256, 0, stream>>>(dE, dX, count, start, list, sorted,
+                                                                        V, D);
+  MMDA_CHECK_LAUNCH();
+  return MMDA_OK;
+}
+
 extern "C" {
 
 int mmda_pack_build(const int* lens_sorted, int B, int Tmax, int N, int* batch_sizes,
@@ -164,6 +254,22 @@ int mmda_embedding_backward(float* dE, const long long* sentences, const float* 
                                                           sorted_idx, N, B, D, V);
   MMDA_CHECK_LAUNCH();
   return MMDA_OK;
+}
+
+long long mmda_embedding_backward_det_workspace_bytes(int N, int V) {
+  if (N <= 0 || V <= 0) return 0;
+  return (2LL * V + 4LL * N) * (long long)sizeof(int);
+}
+
+int mmda_embedding_backward_det(float* dE, const long long* sentences, const float* dX,
+                                const int* row_t, const int* row_j, const int* sorted_idx, int N,
+                                int B, int D, int V, int* workspace, cudaStream_t stream) {
+  if (N <= 0) return MMDA_OK;
+  MMDA_REQUIRE(V > 0 && D > 0 && workspace, "embedding_backward_det: V=%d D=%d / no workspace", V, D);
+  emb_det_ids_kernel<<<(N + 255) / 256, 256, 0, stream>>>(sentences, row_t, row_j, sorted_idx, N, B, V,
+                                                          workspace + 2 * V);
+  MMDA_CHECK_LAUNCH();
+  return embedding_rows_det(dE, dX, N, D, V, workspace, stream);
 }
 
 }  // extern "C"

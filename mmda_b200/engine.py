@@ -59,6 +59,10 @@ class Kernels:
         self._leaf_used = {}            # leaf role -> None, in first-use order since the last join
         self._role = None               # role of the stream `side` runs on; None: the caller's
         self._streams = {}
+        # torch.are_deterministic_algorithms_enabled() as the engine read it at its last forward /
+        # backward: route every cross-CTA reduction to its fixed-order entry
+        self.det = False
+        self.buf_fn = None              # the engine's workspace allocator (MisaEngine.buf)
 
     def bind_stream(self):
         # the CPU dry run binds the role name, so that a stubbed library sees where launches go
@@ -70,6 +74,14 @@ class Kernels:
     def _c(self, name, *args):
         self.launches += 1
         LIB.call(name, *args, self.stream)
+
+    def det_ws(self, query, *args):
+        """Scratch of a fixed-order reduction, sized by the entry's ``*_workspace_bytes`` query:
+        one buffer per stream role, since the launches of one stream run in order."""
+        nbytes = int(LIB.raw(query)(*args))
+        if nbytes < 0:
+            raise MmdaError(LIB.raw("mmda_last_error")().decode())
+        return self.buf_fn(f"det_ws_{self._role}", max(4, (nbytes + 15) // 16 * 4))
 
     def _stream(self, role, priority=0, device=None):
         key = (torch.cuda.current_device() if device is None else device, role)
@@ -129,8 +141,10 @@ class Kernels:
         assert (A.shape[1] if ta else A.shape[0]) == M, (A.shape, C.shape, ta)
         assert (B.shape[0] if tb else B.shape[1]) == N and (B.shape[1] if tb else B.shape[0]) == K, \
             (A.shape, B.shape, C.shape, ta, tb)
-        self._c("mmda_sgemm", int(ta), int(tb), M, N, K, alpha, _ptr(A), A.stride(0), _ptr(B),
-                B.stride(0), beta, _ptr(C), C.stride(0), _ptr(bias), _ptr(bias2), act, split_k, c_ilv)
+        # deterministic: the entry that swaps every atomic split-K for the in-CTA one
+        self._c("mmda_sgemm_det" if self.det else "mmda_sgemm", int(ta), int(tb), M, N, K, alpha,
+                _ptr(A), A.stride(0), _ptr(B), B.stride(0), beta, _ptr(C), C.stride(0), _ptr(bias),
+                _ptr(bias2), act, split_k, c_ilv)
 
     def gemm_tc(self, kind, a_mn, b_mn, M, N, K, A, B, C, alpha=1.0, bias=None, mode=0, split_k=1,
                 c_ilv=0):
@@ -140,6 +154,12 @@ class Kernels:
             kind = 2     # A plain fp32 (split in shared memory); B plain (Bl None) or pre-split
         elif kind == 0 and Bl is None:
             raise MmdaError("gemm_tc: a pre-split A operand needs a pre-split B operand")
+        if self.det and mode == 1 and split_k != 1:
+            ws = self.det_ws("mmda_gemm_tc_det_workspace_bytes", kind, M, N, K, mode, split_k)
+            self._c("mmda_gemm_tc_det", kind, int(a_mn), int(b_mn), M, N, K, _ptr(Ah), _ptr(Al),
+                    Ah.stride(0), _ptr(Bh), _ptr(Bl), Bh.stride(0), alpha, _ptr(C), C.stride(0),
+                    _ptr(bias), None, mode, split_k, c_ilv, _ptr(ws))
+            return
         self._c("mmda_gemm_tc", kind, int(a_mn), int(b_mn), M, N, K, _ptr(Ah), _ptr(Al), Ah.stride(0),
                 _ptr(Bh), _ptr(Bl), Bh.stride(0), alpha, _ptr(C), C.stride(0), _ptr(bias), None, mode,
                 split_k, c_ilv)
@@ -177,6 +197,11 @@ class Kernels:
             self.gemm(dy, w, dx, beta=dx_beta, split_k=1 if dx_beta not in (0.0, 1.0) else 0)
 
     def colsum(self, x, out, out2=None, ilv=0):
+        if self.det:
+            ws = self.det_ws("mmda_colsum_det_workspace_bytes", x.shape[0], x.shape[1])
+            self._c("mmda_colsum_det", _ptr(x), x.stride(0), x.shape[0], x.shape[1], _ptr(out),
+                    _ptr(out2), ilv, _ptr(ws))
+            return
         self._c("mmda_colsum", _ptr(x), x.stride(0), x.shape[0], x.shape[1], _ptr(out), _ptr(out2),
                 ilv)
 
@@ -186,6 +211,12 @@ class Kernels:
                 _ptr(mean), _ptr(rstd), x.shape[0], x.shape[1], LN_EPS)
 
     def layernorm_bwd(self, dy, x, res, g, mean, rstd, dx, dg, db):
+        if self.det:
+            ws = self.det_ws("mmda_layernorm_backward_det_workspace_bytes", x.shape[0], x.shape[1])
+            self._c("mmda_layernorm_backward_det", _ptr(dy), dy.stride(0), _ptr(x), x.stride(0),
+                    _ptr(res), 0 if res is None else res.stride(0), _ptr(g), _ptr(mean), _ptr(rstd),
+                    _ptr(dx), dx.stride(0), _ptr(dg), _ptr(db), x.shape[0], x.shape[1], _ptr(ws))
+            return
         self._c("mmda_layernorm_backward", _ptr(dy), dy.stride(0), _ptr(x), x.stride(0), _ptr(res),
                 0 if res is None else res.stride(0), _ptr(g), _ptr(mean), _ptr(rstd), _ptr(dx),
                 dx.stride(0), _ptr(dg), _ptr(db), x.shape[0], x.shape[1])
@@ -224,6 +255,7 @@ class MisaEngine:
         self.model = model
         self.cfg = model.config
         self.k = Kernels()
+        self.k.buf_fn = self.buf
         self.ws: Dict[str, torch.Tensor] = {}
         self.ws_version = 0
         self.act_id = ACTIVATIONS[model.act_name]
@@ -569,6 +601,7 @@ class MisaEngine:
         k, cfg, d, NC = self.k, self.cfg, self.d, self.NC
         P = self.params()
         k.bind_stream()
+        k.det = torch.are_deterministic_algorithms_enabled()
         if self.use_bert != (utt_text is not None):
             raise MmdaError("utt_text (masked-mean BERT output) is required iff config.use_bert")
         for name, t in (("sentences", sentences), ("visual", visual), ("acoustic", acoustic)):
@@ -784,6 +817,7 @@ class MisaEngine:
         k, d, NC = self.k, self.d, self.NC
         P = self.params()
         k.bind_stream()
+        k.det = det = torch.are_deterministic_algorithms_enabled()
         sv = self.saved
         if not sv.get("train"):
             raise MmdaError("backward() needs a forward(train=True)")
@@ -934,6 +968,9 @@ class MisaEngine:
         dA = self.buf("dA", 3, B, d)
         dutt = {m: self.buf(f"dutt_{m}", B, self.utt_dim[m]) for m in MODS}
         pmu, prs = self.buf("proj_mu", 3, B), self.buf("proj_rs", 3, B)
+        # the shared encoder's gradient gets a term from each modality's stream: atomically
+        # accumulated into one tensor, or (deterministic) one partial per stream, summed below
+        sh_part = self.buf("shared_1_part", 3, d * d + d) if det else None
 
         def head_bwd(i, m):
             def run():
@@ -955,9 +992,13 @@ class MisaEngine:
                              G[f"private_{m}.private_{m}_{tag}.weight"],
                              G[f"private_{m}.private_{m}_{tag}.bias"], dO[i],
                              1.0 if has_do else 0.0)
-                # the shared encoder's gradient is accumulated by all three modality streams
-                k.linear_bwd(ss, O[i], P["shared.shared_1.weight"], G["shared.shared_1.weight"],
-                             G["shared.shared_1.bias"], dO[i], 1.0, dw_split=2)
+                if det:
+                    sh_part[i].zero_()
+                    k.linear_bwd(ss, O[i], P["shared.shared_1.weight"], sh_part[i, :d * d].view(d, d),
+                                 sh_part[i, d * d:], dO[i], 1.0)
+                else:
+                    k.linear_bwd(ss, O[i], P["shared.shared_1.weight"], G["shared.shared_1.weight"],
+                                 G["shared.shared_1.bias"], dO[i], 1.0, dw_split=2)
                 k.layernorm_bwd(dO[i], A[i], None, P[f"project_{m}.project_{m}_layer_norm.weight"],
                                 pmu[i], prs[i], dA[i],
                                 G[f"project_{m}.project_{m}_layer_norm.weight"],
@@ -969,6 +1010,10 @@ class MisaEngine:
             return run
 
         self._fork({m: head_bwd(i, m) for i, m in enumerate(MODS)})
+        if det:
+            k.join_leaves()
+            k._c("mmda_fixed_order_sum", _ptr(sh_part), 3, d * d + d, d * d + d,
+                 _ptr(G["shared.shared_1.weight"]), _ptr(G["shared.shared_1.bias"]), d * d)
         if on_ready is not None:
             k.join_leaves()
         notify("heads")
@@ -1103,9 +1148,15 @@ class MisaEngine:
                 k.gemm_tc(0, 0, 1, N, I, 8 * H, dGp, Wst, dX)
                 if r == r1:
                     V = P["embed.weight"].shape[0]
-                    k._c("mmda_embedding_backward", _ptr(G["embed.weight"]),
-                         _ptr(self.saved["sent"]), _ptr(dX), _ptr(pk["row_t"]), _ptr(pk["row_j"]),
-                         _ptr(pk["sidx"]), N, B, H, V)
+                    if k.det:
+                        ws = k.det_ws("mmda_embedding_backward_det_workspace_bytes", N, V)
+                        k._c("mmda_embedding_backward_det", _ptr(G["embed.weight"]),
+                             _ptr(self.saved["sent"]), _ptr(dX), _ptr(pk["row_t"]),
+                             _ptr(pk["row_j"]), _ptr(pk["sidx"]), N, B, H, V, _ptr(ws))
+                    else:
+                        k._c("mmda_embedding_backward", _ptr(G["embed.weight"]),
+                             _ptr(self.saved["sent"]), _ptr(dX), _ptr(pk["row_t"]),
+                             _ptr(pk["row_j"]), _ptr(pk["sidx"]), N, B, H, V)
                     # the dense embedding gradient (the largest bucket) is complete here, a
                     # millisecond of weight-gradient GEMMs before the rest of the encoder: its
                     # all-reduce runs under them

@@ -301,7 +301,13 @@ class FusedTrainer:
         w_conf = float(cfg.conf_weight) if self.use_confid else 0.0
         XN = eng.buf("XN", 6, B, d)
         inv = eng.buf("inv_norm", 6, B)
-        k._c("mmda_loss_phase2", _ptr(X0), _ptr(segA), _ptr(XN), _ptr(inv), _ptr(segB), B, d, Bg)
+        det = k.det         # torch.are_deterministic_algorithms_enabled() at this step's forward
+        if det:
+            ws = k.det_ws("mmda_loss_det_workspace_bytes", B, d)
+            k._c("mmda_loss_phase2_det", _ptr(X0), _ptr(segA), _ptr(XN), _ptr(inv), _ptr(segB), B, d,
+                 Bg, _ptr(ws))
+        else:
+            k._c("mmda_loss_phase2", _ptr(X0), _ptr(segA), _ptr(XN), _ptr(inv), _ptr(segB), B, d, Bg)
         Gm = segB[12 * d:].view(6, d, d)
         k._c("mmda_loss_gram", _ptr(XN), _ptr(Gm), B, d)     # the six pairs in one launch
         if sync:
@@ -311,8 +317,12 @@ class FusedTrainer:
              int(adv), mode)
         DXN = eng.buf("DXN", 6, B, d)
         alpha = float(cfg.diff_weight) * 2.0 / float(d * d)
-        k._c("mmda_loss_dxn", _ptr(XN), _ptr(Gm), _ptr(DXN), B, d, alpha)
-        k._c("mmda_loss_phase4a", _ptr(DXN), _ptr(inv), _ptr(segC), B, d)
+        if det:
+            k._c("mmda_loss_dxn_det", _ptr(XN), _ptr(Gm), _ptr(DXN), B, d, alpha)
+            k._c("mmda_loss_phase4a_det", _ptr(DXN), _ptr(inv), _ptr(segC), B, d, _ptr(ws))
+        else:
+            k._c("mmda_loss_dxn", _ptr(XN), _ptr(Gm), _ptr(DXN), B, d, alpha)
+            k._c("mmda_loss_phase4a", _ptr(DXN), _ptr(inv), _ptr(segC), B, d)
         if sync:
             self._allreduce(segC)
         dZ = eng.buf("dZ", B, 6, d)
@@ -633,8 +643,9 @@ class FusedTrainer:
         Np = padded_rows(N, B, T)
         if visual.shape[0] != T or acoustic.shape[0] != T or int(lengths.max()) > T:
             return self._eager_step(sentences, visual, acoustic, lengths, labels)
+        # a graph holds the launches of one reduction mode: the deterministic flag is part of the key
         key = (tuple(sentences.shape), tuple(visual.shape), tuple(acoustic.shape), Np, N == Np,
-               self.model.training)
+               self.model.training, torch.are_deterministic_algorithms_enabled())
         alias = tuple(p.data_ptr() for p in self.model.parameters()) + \
             tuple(p.requires_grad for p in self.model.parameters())
         if self._graphs and (self._graphs_ws != self.eng.ws_version or self._graphs_alias != alias):
