@@ -61,16 +61,14 @@ int mmda_ctx_info(int* out6);
 
 /* ---- packing: pack_padded_sequence(enforce_sorted=False), src/models.py:164,173 -------------
  * lens_sorted: lengths after the host's descending torch.sort (device int32, B entries).
- * Writes batch_sizes[Tmax], offsets[Tmax+1] and the (t, j) coordinates of each of the N rows. */
-int mmda_pack_build(const int* lens_sorted, int B, int Tmax, int N, int* batch_sizes, int* offsets,
-                    int* row_t, int* row_j, mmda_stream_t stream);
-/* Same, for a launch padded to Np >= N packed rows (one captured CUDA graph serves every length
- * pattern whose row count rounds to the same Np; Tmax is then the padded time extent of the input
- * tensors, batch_sizes[t] = 0 past the longest sequence): rows [N, Np) of the row maps point at
- * token (0, 0), so row-wise kernels launched over Np rows read valid memory.  The reference packs
- * exactly (pack_padded_sequence, src/models.py:164); the padding rows never reach a valid row's
- * result -- GEMM rows are independent and the backward zeroes them (mmda_zero_tail_rows) before
- * any reduction over rows. */
+ * Writes batch_sizes[Tmax], offsets[Tmax+1] and the (t, j) coordinates of each of the N rows, for
+ * a launch padded to Np >= N packed rows (Np == N packs exactly; one captured CUDA graph serves
+ * every length pattern whose row count rounds to the same Np; Tmax is then the padded time extent
+ * of the input tensors, batch_sizes[t] = 0 past the longest sequence): rows [N, Np) of the row
+ * maps point at token (0, 0), so row-wise kernels launched over Np rows read valid memory.  The
+ * reference packs exactly (pack_padded_sequence, src/models.py:164); the padding rows never reach
+ * a valid row's result -- GEMM rows are independent and the backward zeroes them
+ * (mmda_zero_tail_rows) before any reduction over rows. */
 int mmda_pack_build_padded(const int* lens_sorted, int B, int Tmax, int N, int Np, int* batch_sizes,
                            int* offsets, int* row_t, int* row_j, mmda_stream_t stream);
 /* rows [*n_rows_dev, Np) of the fp32 matrix A (row pitch ld floats, ld % 4 == 0) := 0; the row
@@ -149,16 +147,12 @@ long long mmda_lstm_scratch_bytes(int B, int H);
 /* out6 = {cluster size, units per CTA, batch tile, n batch tiles, smem fwd, smem bwd}; the
  * contraction split of the backward is 16 lanes for H > 128, else 4 */
 int mmda_lstm_plan(int B, int H, int* out6);
-/* stacked gate-interleaved copy of W_ih (both directions) + bias stack for the hoisted GEMMs:
- * row dir*4H+u*4+g <- row g*H+u.  mode 0 fp32 (out_a), 1 tf32 hi/lo (out_a,out_b), 2 bf16 (out_a). */
+/* stacked gate-interleaved copy of W_ih (both directions) + bias stack for the hoisted 3xTF32
+ * GEMMs: row dir*4H+u*4+g <- row g*H+u, split into tf32 hi (out_a) and lo (out_b), both [8H][ld];
+ * bias_out (nullable) [8H] = b_ih + b_hh in the same row order. */
 int mmda_lstm_pack_weights(const float* w_ih_f, const float* w_ih_r, const float* b_ih_f,
                            const float* b_hh_f, const float* b_ih_r, const float* b_hh_r, int H, int I,
-                           int mode, void* out_a, float* out_b, int ld, float* bias_out,
-                           mmda_stream_t stream);
-/* diagnostic: per-step phase timestamps of CTA 0 of subsequent forward launches (NULL = off) */
-int mmda_lstm_set_debug_buffer(long long* dev_buf);
-/* diagnostic: co-resident clusters of the recurrent kernel for cluster sizes {1,2,4,8,16} */
-int mmda_lstm_probe_clusters(int smem_bytes, int threads, int* out5);
+                           float* out_a, float* out_b, int ld, float* bias_out, mmda_stream_t stream);
 /* h_{prev} operand for the hoisted dW_hh GEMM: [N][2][Hp] (Hp >= H: direction pitch) */
 int mmda_lstm_shift_h(const float* y, float* hprev, const int* row_t, const int* row_j,
                       const int* lens_sorted, const int* offsets, int N, int H, int Hp,
@@ -187,8 +181,6 @@ int mmda_lstm_tc_backward(float* gates, const float* whh_f, const float* whh_r, 
                           int utt_off_r, const int* lens_sorted, const int* sorted_idx,
                           const int* offsets, int B, int H, int Tmax, void* ws,
                           mmda_stream_t stream);
-/* diagnostic: per-step phase timestamps of CTA 0 (NULL = off) */
-int mmda_lstm_tc_set_debug_buffer(long long* dev_buf);
 
 /* ---- nn.LayerNorm, src/models.py:65-80,155-157,172 and the two norms of the fusion layer ----
  * y = LN(x + res) (res may be NULL); mean/rstd saved per row for the backward. */

@@ -68,7 +68,7 @@ int mmda_ctx_info(int* out6) {
   return MMDA_OK;
 }
 
-int mmda_abi_version(void) { return 1; }
+int mmda_abi_version(void) { return 2; }
 
 // out[0]=SM count, out[1]=max opt-in smem/block, out[2]=cc major, out[3]=cc minor, out[4]=L2 bytes
 int mmda_device_info(int* out5) {

@@ -24,7 +24,6 @@
 // per step.  The backward kernel keeps the same slice, produces partial dh_{t-1} over all H
 // columns, exchanges the partials through an L2-resident scratch and reduces its own columns.
 #include "common.cuh"
-#include <cuda_bf16.h>
 
 constexpr int kMatvecUnroll = 4;   // inner-loop unroll of the one-unit mat-vec (3 and 5 measured equal)
 
@@ -43,7 +42,6 @@ struct LstmArgs {
   float* scratch;         // bwd: partial-sum exchange [2][n_clusters][C][BT][Kpad]
   int utt_ld, utt_off0, utt_off1;
   int B, H, Hs, Kpad, C, n_tiles, save;
-  long long* dbg;         // optional per-step phase timestamps (profiling builds of the bench)
 };
 
 template <int N, int BITLO>
@@ -133,11 +131,8 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_fwd_kernel(const
   const uint32_t slice_bytes = (uint32_t)(Hs * BTP * 4);
   const uint32_t slice_addr = (uint32_t)__cvta_generic_to_shared(h_s + rank * Hs * BTP);
 
-  const bool dbg_on = p.dbg != nullptr && blockIdx.x == 0 && blockIdx.y == 0 && tid == 0;
-#define LSTM_TS(i) if (dbg_on) p.dbg[s * 8 + (i)] = clock64();
   for (int s = 0; s < Lmax; ++s) {
     const int t = dir == 0 ? s : Lmax - 1 - s;
-    LSTM_TS(0)
     if (C > 1 && tid == 0) mbar_arrive_expect_tx(mbar, (C - 1) * slice_bytes);   // arm for h_t
     const bool a0 = u_ok && t < len0, a1 = u_ok && t < len1;
     const int off_t = __ldg(p.offsets + t);
@@ -174,7 +169,6 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_fwd_kernel(const
       }
       reduce_scatter<32, 8>(acc, lane);  // lane q now owns batch rows 2q, 2q+1 -> acc[0..8)
     }
-    LSTM_TS(1)
     cluster_arrive_relaxed();  // A: this CTA is done reading h_{t-1}
 
     float hn0 = 0.f, hn1 = 0.f, s0[5], s1[5];
@@ -212,9 +206,7 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_fwd_kernel(const
       }
     }
 
-    LSTM_TS(2)
     cluster_wait();  // A: every CTA of the cluster is done reading h_{t-1}
-    LSTM_TS(3)
     if (a0 || a1) *reinterpret_cast<float2*>(h_slot) = make_float2(hn0, hn1);
     if (C > 1) {
       fence_proxy_async_smem();
@@ -229,7 +221,6 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_fwd_kernel(const
     } else {
       __syncthreads();
     }
-    LSTM_TS(4)
     // global stores drain while the barrier completes
     if (a0) {
       if (p.save) {
@@ -249,11 +240,8 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_fwd_kernel(const
       const bool fin = dir == 0 ? (t == len1 - 1) : (t == 0);
       if (fin && p.utt) p.utt[(size_t)orig1 * p.utt_ld + utt_off + u_glob] = hn1;
     }
-    LSTM_TS(5)
     if (C > 1) mbar_wait_parity(mbar, s & 1);   // the 7 peer slices of h_t have landed
-    LSTM_TS(6)
   }
-#undef LSTM_TS
   cluster_sync_all();   // no CTA may exit while a peer's bulk copy still reads its shared memory
 }
 
@@ -328,12 +316,9 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_bwd_kernel(const
   const size_t slab = (size_t)BT * Kpad;   // one CTA's partial block
   float dc0 = 0.f, dc1 = 0.f;
 
-  const bool dbg_on = p.dbg != nullptr && blockIdx.x == 0 && blockIdx.y == 0 && tid == 0;
-#define LSTM_TS(i) if (dbg_on) p.dbg[s * 8 + (i)] = clock64();
   for (int s = 0; s < Lmax; ++s) {
     const int t = dir == 0 ? Lmax - 1 - s : s;
     const int par = s & 1;
-    LSTM_TS(0)
     float* scr = p.scratch + ((size_t)(par * 2 * p.n_tiles + cl_id) * C) * slab;
 
     // ---- partial dh over all H columns from this CTA's gate rows of the successor step ----
@@ -372,7 +357,6 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_bwd_kernel(const
         }
       }
     }
-    LSTM_TS(2)
     cluster_arrive();   // release: this CTA's partials are published
     // ---- fetch everything the cell update needs while the cluster barrier completes ----
     const bool a0 = u_ok && t < len0, a1 = u_ok && t < len1;
@@ -412,9 +396,7 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_bwd_kernel(const
       rec1 = dir == 0 ? (t + 1 < len1) : (t >= 1);
     }
 
-    LSTM_TS(1)
     cluster_wait();     // acquire: partials of every CTA visible
-    LSTM_TS(3)
     // all 2*C partial loads in flight at once (they are L2 round trips), then summed
     float rdh0 = 0.f, rdh1 = 0.f;
     {
@@ -483,11 +465,8 @@ __global__ void __launch_bounds__(BT == 40 ? 800 : 640, 1) lstm_bwd_kernel(const
       float* sp = dG_s + (u * 4) * BTP + ebl0 + 1;
       sp[0] = dig; sp[BTP] = dfg; sp[2 * BTP] = dgg; sp[3 * BTP] = dog;
     }
-    LSTM_TS(4)
     __syncthreads();  // dG_s complete before the next step's matvec
-    LSTM_TS(5)
   }
-#undef LSTM_TS
   cluster_sync_all();
 }
 
@@ -512,13 +491,13 @@ __global__ void lstm_shift_kernel(const float* __restrict__ y, float* __restrict
 
 // Stacked, gate-interleaved copy of the two directions' W_ih for the hoisted GEMMs:
 //   row (dir*4H + u*4 + g) of the copy = row (g*H + u) of weight_ih_l0{,_reverse}
-// so the GEMM writes / reads the [N][2][H][4] gate layout directly.  mode 0: fp32 copy (out_a);
-// mode 1: tf32 hi/lo split (out_a, out_b); mode 2: bf16 (out_a).  Also writes the matching bias
-// stack b_ih + b_hh (bias_out, nullable).
+// so the GEMM writes / reads the [N][2][H][4] gate layout directly, split into tf32 hi (out_a) and
+// the fp32 remainder lo (out_b) for the 3xTF32 GEMMs.  Also writes the matching bias stack
+// b_ih + b_hh (bias_out, nullable).
 __global__ void lstm_pack_weights_kernel(const float* __restrict__ wf, const float* __restrict__ wr,
                                          const float* __restrict__ bif, const float* __restrict__ bhf,
                                          const float* __restrict__ bir, const float* __restrict__ bhr,
-                                         int H, int I, int mode, void* __restrict__ out_a,
+                                         int H, int I, float* __restrict__ out_a,
                                          float* __restrict__ out_b, int ld, float* __restrict__ bias_out) {
   const int H4 = 4 * H;
   const size_t n = (size_t)2 * H4 * I;
@@ -529,17 +508,11 @@ __global__ void lstm_pack_weights_kernel(const float* __restrict__ wf, const flo
     const int dir = r / H4, rr = r % H4, g = rr / H, u = rr % H;
     const float v = (dir ? wr : wf)[(size_t)rr * I + c];
     const size_t o = (size_t)(dir * H4 + u * 4 + g) * ld + c;
-    if (mode == 0) {
-      reinterpret_cast<float*>(out_a)[o] = v;
-    } else if (mode == 1) {
-      uint32_t hb;
-      asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(v));
-      const float h = __uint_as_float(hb);
-      reinterpret_cast<float*>(out_a)[o] = h;
-      out_b[o] = v - h;
-    } else {
-      reinterpret_cast<__nv_bfloat16*>(out_a)[o] = __float2bfloat16(v);
-    }
+    uint32_t hb;
+    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(v));
+    const float h = __uint_as_float(hb);
+    out_a[o] = h;
+    out_b[o] = v - h;
     if (bias_out != nullptr && c == 0)
       bias_out[dir * H4 + u * 4 + g] = (dir ? bir : bif)[rr] + (dir ? bhr : bhf)[rr];
   }
@@ -692,16 +665,7 @@ static int launch_cluster(K kern, const LstmArgs& a, const LstmPlan& pl, int thr
   return MMDA_OK;
 }
 
-static long long* g_lstm_dbg = nullptr;
-
 extern "C" {
-
-// profiling aid: when set (device buffer of >= 8*Tmax int64), CTA 0 of the NEXT forward launches
-// records clock64() at the phase boundaries of every step
-int mmda_lstm_set_debug_buffer(long long* dev_buf) {
-  g_lstm_dbg = dev_buf;
-  return MMDA_OK;
-}
 
 long long mmda_lstm_scratch_bytes(int B, int H) {
   LstmPlan pl;
@@ -716,33 +680,6 @@ int mmda_lstm_plan(int B, int H, int* out6) {
   if (rc != MMDA_OK) return rc;
   out6[0] = pl.C; out6[1] = pl.Hs; out6[2] = pl.BT; out6[3] = pl.n_tiles;
   out6[4] = (int)pl.smem_fwd; out6[5] = (int)pl.smem_bwd;
-  return MMDA_OK;
-}
-
-// probe: how many clusters of the text-size forward kernel can be co-resident (out[i] for
-// cluster sizes 1,2,4,8,16 with the given dynamic smem bytes and block size); -1 = not launchable
-int mmda_lstm_probe_clusters(int smem_bytes, int threads, int* out5) {
-  const int sizes[5] = {1, 2, 4, 8, 16};
-  auto kern = lstm_fwd_kernel<32, 0>;
-  MMDA_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
-  cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-  for (int i = 0; i < 5; ++i) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(sizes[i] * 64, 2, 1);
-    cfg.blockDim = dim3(threads, 1, 1);
-    cfg.dynamicSmemBytes = smem_bytes;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = sizes[i];
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    int n = -1;
-    cudaError_t e = cudaOccupancyMaxActiveClusters(&n, kern, &cfg);
-    out5[i] = e == cudaSuccess ? n : -1;
-    if (e != cudaSuccess) cudaGetLastError();
-  }
   return MMDA_OK;
 }
 
@@ -762,7 +699,6 @@ static int rnn_forward(int cell, float* gates, const float* whh_f, const float* 
   a.utt = utt; a.utt_ld = utt_ld; a.utt_off0 = utt_off_f; a.utt_off1 = utt_off_r;
   a.B = B; a.H = H; a.Hs = pl.Hs; a.Kpad = pl.Kpad; a.C = pl.C; a.n_tiles = pl.n_tiles;
   a.save = save_for_backward;
-  a.dbg = g_lstm_dbg;
   if (cell != 0) {
     if (pl.BT == 40) return launch_cluster(lstm_fwd_kernel<40, 1>, a, pl, pl.threads_fwd, pl.smem_fwd, stream);
     if (pl.BT == 32) return launch_cluster(lstm_fwd_kernel<32, 1>, a, pl, pl.threads_fwd, pl.smem_fwd, stream);
@@ -788,7 +724,6 @@ static int rnn_backward(int cell, float* gates, const float* whh_f, const float*
   a.gates = gates; a.whh[0] = whh_f; a.whh[1] = whh_r; a.c = const_cast<float*>(c);
   a.dy = dy; a.dutt = dutt; a.utt_ld = utt_ld; a.utt_off0 = utt_off_f; a.utt_off1 = utt_off_r;
   a.lens = lens_sorted; a.sorted_idx = sorted_idx; a.offsets = offsets; a.scratch = scratch;
-  a.dbg = g_lstm_dbg;
   a.B = B; a.H = H; a.Hs = pl.Hs; a.Kpad = pl.Kpad; a.C = pl.C; a.n_tiles = pl.n_tiles;
   if (cell != 0) {
     if (pl.BT == 40 && pl.KS == 16)
@@ -872,14 +807,19 @@ int mmda_gru_fold_grads(const float* dw4_ih, const float* dw4_hh, const float* d
 
 int mmda_lstm_pack_weights(const float* w_ih_f, const float* w_ih_r, const float* b_ih_f,
                            const float* b_hh_f, const float* b_ih_r, const float* b_hh_r, int H, int I,
-                           int mode, void* out_a, float* out_b, int ld, float* bias_out,
+                           float* out_a, float* out_b, int ld, float* bias_out,
                            cudaStream_t stream) {
-  MMDA_REQUIRE(mode >= 0 && mode <= 2 && H > 0 && I > 0 && ld >= I, "lstm_pack_weights: bad arguments");
-  MMDA_REQUIRE(mode != 1 || out_b != nullptr, "lstm_pack_weights: tf32 split needs out_b");
+  MMDA_REQUIRE(H > 0 && I > 0 && ld >= I, "lstm_pack_weights: bad arguments");
+  MMDA_REQUIRE(out_a != nullptr && out_b != nullptr, "lstm_pack_weights: out_a and out_b required");
+  // every output is a float array: a value that is not 4-byte aligned (such as the 0 / 1 / 2 pack
+  // mode a caller of ABI version 1 passes where out_a now stands) is refused before any launch
+  MMDA_REQUIRE(((uintptr_t)out_a | (uintptr_t)out_b | (uintptr_t)bias_out) % 4 == 0,
+               "lstm_pack_weights: out_a / out_b / bias_out not 4-byte aligned (ABI version 2 has "
+               "no mode argument)");
   size_t n = (size_t)8 * H * I, g = (n + 255) / 256;
   if (g > 1184) g = 1184;
   lstm_pack_weights_kernel<<<(int)g, 256, 0, stream>>>(w_ih_f, w_ih_r, b_ih_f, b_hh_f, b_ih_r, b_hh_r,
-                                                       H, I, mode, out_a, out_b, ld, bias_out);
+                                                       H, I, out_a, out_b, ld, bias_out);
   MMDA_CHECK_LAUNCH();
   return MMDA_OK;
 }

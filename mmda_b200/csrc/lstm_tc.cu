@@ -64,7 +64,6 @@ struct TclArgs {
   uint8_t* xch;           // fwd: h operand images [2][NT][2][2*KA*B_ATOM]; bwd: partials [2][NT][2][S][48][S*32] f32
   unsigned* flags;        // [2][NT] counters (zeroed before the launch): one tick per cell warp and step
   int* err;               // set to 1 when a peer never showed up
-  long long* dbg;
 };
 
 // wait until *flag >= target (one thread); returns false after SPIN_LIMIT ticks or when another
@@ -220,8 +219,6 @@ __global__ void __launch_bounds__(TCL_FWD_THREADS4, 1) lstm_tc_fwd_kernel(const 
   const int ycol = dir * H + u;
   const int utt_off = dir == 0 ? p.utt_off0 : p.utt_off1;
   uint32_t n_done[MAXSUB] = {0, 0, 0, 0};  // completed phases of "my" barrier of each sub-tile
-  const bool dbg_on = p.dbg != nullptr && blockIdx.x == 0;
-#define TCL_TS(i) if (dbg_on && tile == grp && k == 0) p.dbg[s * 16 + (i)] = clock64();
 
   for (int tile = grp; tile < p.NT; tile += p.G) {
     const int b_base = tile * p.BT;
@@ -250,7 +247,6 @@ __global__ void __launch_bounds__(TCL_FWD_THREADS4, 1) lstm_tc_fwd_kernel(const 
           for (int k = 0; k < MAXSUB; ++k) {
             if (s >= Lk[k]) continue;
             if (!aborted && !spin_until(flags + k, (unsigned)(S * s), p.err)) aborted = true;
-            TCL_TS(1)
             fence_proxy_async_global();
             mbar_expect_tx(copy_bar(k), IMGS);
             bulk_g2s(sbase + (uint32_t)k * IMGS, img_g + ((size_t)k * 2 + ((s - 1) & 1)) * IMGS, IMGS,
@@ -269,7 +265,6 @@ __global__ void __launch_bounds__(TCL_FWD_THREADS4, 1) lstm_tc_fwd_kernel(const 
           mbar_wait(copy_bar(k), n_done[k] & 1);
           ++n_done[k];
           fence_after();
-          if (lane == 0) { TCL_TS(2) }
           const uint32_t idesc = idesc_f16(128, SUB);
           const uint32_t d_m0 = tmD + (uint32_t)k * 3 * SUB, d_m1 = d_m0 + SUB, d_x = d_m0 + 2 * SUB;
           const uint64_t b1_0 = make_desc(sbase + (uint32_t)k * IMGS, 16, 1024);
@@ -291,7 +286,6 @@ __global__ void __launch_bounds__(TCL_FWD_THREADS4, 1) lstm_tc_fwd_kernel(const 
             commit(mma_bar(k));
           }
           __syncwarp();
-          if (lane == 0) { TCL_TS(3) }
         }
       continue;
     }
@@ -303,7 +297,6 @@ __global__ void __launch_bounds__(TCL_FWD_THREADS4, 1) lstm_tc_fwd_kernel(const 
           if (s + 1 >= Lk[k]) continue;
           mbar_wait(stage_bar(k), n_done[k] & 1);
           ++n_done[k];
-          if (lane == 0) { TCL_TS(7) }
           uint8_t* dst = img_g + ((size_t)k * 2 + (s & 1)) * IMGS;
           const uint8_t* st = sptr + stage_off + k * STAGE_BYTES;
 #pragma unroll
@@ -313,11 +306,9 @@ __global__ void __launch_bounds__(TCL_FWD_THREADS4, 1) lstm_tc_fwd_kernel(const 
             const uint4 v = *reinterpret_cast<const uint4*>(st + sp * (SUB * 64) + n * 64 + c * 16);
             *reinterpret_cast<uint4*>(dst + sp * SPLS + swz_chunk(n, 4 * r + c, SUB_ATOM)) = v;
           }
-          if (lane == 0) { TCL_TS(9) }
           fence_proxy_async_global();     // my generic-proxy writes vs the peers' bulk copies
           __syncwarp();                   // orders the 32 lanes' stores before lane 0's release (cumulative)
           if (lane == 0) red_release_add(flags + k, 1u);
-          if (lane == 0) { TCL_TS(8) }
         }
       continue;
     }
@@ -346,7 +337,6 @@ __global__ void __launch_bounds__(TCL_FWD_THREADS4, 1) lstm_tc_fwd_kernel(const 
       for (int k = 0; k < MAXSUB; ++k) {
         if (s >= Lk[k]) continue;
         const int t = dir == 0 ? s : Lk[k] - 1 - s;
-        if (tid == 0) { TCL_TS(0) }
         const int off_t = __ldg(p.offsets + t);
         const float4 xg0 = xg[k][0], xg1 = xg[k][1];
         if (s + 1 < Lk[k]) {   // next step's x-projection of these two cells
@@ -368,7 +358,6 @@ __global__ void __launch_bounds__(TCL_FWD_THREADS4, 1) lstm_tc_fwd_kernel(const 
           mbar_wait(mma_bar(k), n_done[k] & 1);
           ++n_done[k];
           fence_after();
-          if (tid == 0) { TCL_TS(4) }
           uint32_t m0[8], m1[8], xx[8];
           const uint32_t col = (uint32_t)(k * 3 * SUB + 8 * hc);
           tmem_ld8(tmD + lane_sel + col, m0);
@@ -414,7 +403,6 @@ __global__ void __launch_bounds__(TCL_FWD_THREADS4, 1) lstm_tc_fwd_kernel(const 
           __syncwarp();
           if (lane == 0) mbar_arrive(stage_bar(k));
         }
-        if (tid == 0) { TCL_TS(5) }
         // ---- outputs nobody waits for inside this launch ----
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
@@ -430,10 +418,8 @@ __global__ void __launch_bounds__(TCL_FWD_THREADS4, 1) lstm_tc_fwd_kernel(const 
             if (fin && p.utt) p.utt[(size_t)orig_c[k][i] * p.utt_ld + utt_off + u] = hn[i];
           }
         }
-        if (tid == 0) { TCL_TS(6) }
       }
   }
-#undef TCL_TS
   fence_before();
   __syncthreads();
   if (warp == 0) tmem_dealloc512(tm);
@@ -569,8 +555,6 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
 
   const int H2 = 2 * H, H8 = 8 * H;
   uint32_t n_done[BMAXSUB] = {0, 0, 0};      // completed phases of "my" barrier of each sub-tile
-  const bool dbg_on = p.dbg != nullptr && blockIdx.x == 0;
-#define TCL_TS(i) if (dbg_on && tile == grp && k == 0) p.dbg[s * 16 + (i)] = clock64();
 
   for (int tile = grp; tile < p.NT; tile += p.G) {
     const int b_base = tile * p.BT;
@@ -606,7 +590,6 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
           for (int k = 0; k < BMAXSUB; ++k) {
             if (s >= Lk[k]) continue;
             if (!aborted && !spin_until(flags + k, (unsigned)(S * BWD_WRITERS * s), p.err)) aborted = true;
-            TCL_TS(1)
             mbar_arrive(part_bar(k));
           }
       }
@@ -622,7 +605,6 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
           mbar_wait(dg_bar(k), n_done[k] & 1);       // all eight cell warps staged d(gates) of (k, s)
           ++n_done[k];
           fence_after();
-          if (lane == 0) { TCL_TS(2) }
           const uint32_t idesc = idesc_f16(128, BSUB);
           const uint64_t b1_0 = make_desc(sbase + (uint32_t)k * BWD_SUB_BYTES, 16, 1024);
           const uint64_t B1_0 = b1_0 + (uint64_t)(BWD_PLANE >> 4), b2_0 = B1_0 + (uint64_t)(BWD_PLANE >> 4);
@@ -645,7 +627,6 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
             commit(mma_bar(k));
           }
           __syncwarp();
-          if (lane == 0) { TCL_TS(3) }
         }
       continue;
     }
@@ -663,13 +644,12 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
           mbar_wait(mma_bar(k), n_done[k] & 1);
           ++n_done[k];
           fence_after();
-          if (lane == 0 && q == 0) { TCL_TS(4) }
           // undo 2^11 * s of the block of step s-1 (same exponent arithmetic as the cell warps)
           const unsigned mxb = *reinterpret_cast<volatile unsigned*>(smax + ((s - 1) & 1) * BMAXSUB + k);
           const int e = mxb == 0u ? 0 : min(120, max(-120, 129 - (int)((mxb >> 23) & 0xffu)));
           const float unscale = ldexpf(1.f, -11 - e);
           float* dst = part + (((size_t)k * 2 + (s & 1)) * S + r) * slab;
-          // not unrolled: keeps the kernel at 120 registers
+          // not unrolled: keeps the kernel at 124 registers
 #pragma unroll 1
           for (int mt = 0; mt < MT; ++mt) {
             const int j = mt * 128 + q * 32 + lane;
@@ -687,11 +667,9 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
               if (ok && jj + 8 < n_prev) dj[(size_t)(jj + 8) * XLD] = __uint_as_float(v1[jj]) * unscale;
             }
           }
-          if (lane == 0 && q == 0) { TCL_TS(8) }
           fence_before();
           __syncwarp();
           if (lane == 0) red_release_add(flags + k, 1u);
-          if (lane == 0 && q == 0) { TCL_TS(5) }
         }
       continue;
     }
@@ -739,7 +717,6 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
       for (int k = 0; k < BMAXSUB; ++k) {
         if (s >= Lk[k]) continue;
         const int t = dir == 0 ? Lk[k] - 1 - s : s;
-        if (tid == 0) { TCL_TS(0) }
         // ---- everything the cell backward needs that does not depend on the exchange: staged in
         // shared memory by this thread's own cp.async of the previous step (or the tile prologue) ----
         const int off_t = offs_s[t];
@@ -769,7 +746,6 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
         if (s > 0) {
           mbar_wait(part_bar(k), n_done[k] & 1);   // every CTA's partials of (k, s) are in L2
           ++n_done[k];
-          if (tid == 0) { TCL_TS(6) }
           // ---- reduce my columns over the S partial blocks (all loads in flight at once) ----
           const float* src = part + ((size_t)k * 2 + (s & 1)) * S * slab + u;
           float v[2][12];
@@ -788,7 +764,6 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
             dh[i] += sum;
           }
         }
-        if (tid == 0) { TCL_TS(10) }
         // every cell warp is past item (k, s-1): the slot of the NEXT step can be cleared
         if (tid == 0) smax[((s + 1) & 1) * BMAXSUB + k] = 0u;
         // ---- cell backward ----
@@ -816,9 +791,7 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
           mx = warp_max(mx);
           if (!(mx < 3.0e38f)) mx = 3.0e38f;                    // inf / nan guard: keep the exponent finite
           if (lane == 0) atomicMax(smax + (s & 1) * BMAXSUB + k, __float_as_uint(mx));
-          if (tid == 0) { TCL_TS(11) }
           asm volatile("bar.sync 1, 256;" ::: "memory");
-          if (tid == 0) { TCL_TS(12) }
           const unsigned mxb = *reinterpret_cast<volatile unsigned*>(smax + (s & 1) * BMAXSUB + k);
           const int e = mxb == 0u ? 0 : min(120, max(-120, 129 - (int)((mxb >> 23) & 0xffu)));
           const float sc = ldexpf(1.f, e);
@@ -845,7 +818,6 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
           __syncwarp();
           if (lane == 0) mbar_arrive(dg_bar(k));
         }
-        if (tid == 0) { TCL_TS(7) }
         // the GEMM operand copy of d(gates): nobody inside this launch waits for it
 #pragma unroll
         for (int i = 0; i < 2; ++i)
@@ -853,7 +825,6 @@ __global__ void __launch_bounds__(TCL_BWD_THREADS4, 1) lstm_tc_bwd_kernel(const 
             *reinterpret_cast<float4*>(p.gates + (size_t)(off_t + b_base + k * BSUB + warp + 8 * i) * H8 + gcol) = dgv[i];
       }
   }
-#undef TCL_TS
   fence_before();
   __syncthreads();
   if (warp == 0) tmem_dealloc512(tm);
@@ -928,7 +899,6 @@ int tcl_make_plan(int B, int H, int Tmax, TclPlan* pl) {
   return MMDA_OK;
 }
 
-long long* g_tcl_dbg = nullptr;
 int g_tcl_plan_bwd = 0;     // mmda_lstm_tc_plan reports the backward decomposition when set
 
 }  // namespace
@@ -967,11 +937,6 @@ int mmda_lstm_tc_plan_select(int backward) {
   return MMDA_OK;
 }
 
-int mmda_lstm_tc_set_debug_buffer(long long* dev_buf) {
-  g_tcl_dbg = dev_buf;
-  return MMDA_OK;
-}
-
 static int tcl_launch(bool bwd, TclArgs& a, int B, int H, int Tmax, void* ws, cudaStream_t stream) {
   MMDA_REQUIRE(B > 0 && H > 0 && Tmax > 0, "lstm_tc: bad sizes B=%d H=%d Tmax=%d", B, H, Tmax);
   MMDA_REQUIRE(ws != nullptr, "lstm_tc: workspace required (mmda_lstm_tc_workspace_bytes)");
@@ -989,7 +954,6 @@ static int tcl_launch(bool bwd, TclArgs& a, int B, int H, int Tmax, void* ws, cu
   if (bwd) { a.S = pl.Sb; a.G = pl.Gb; a.BT = pl.BTb; a.NT = pl.NTb; a.U = pl.Ub; }
   else { a.S = pl.S; a.G = pl.G; a.BT = pl.BT; a.NT = pl.NT; a.U = TCL_UNITS; }
   a.Tmax = Tmax;
-  a.dbg = g_tcl_dbg;
   // flags: zero from the caller's initial fill, then left clean by every launch (kernel epilogue)
   const size_t smem = bwd ? pl.smem_bwd : pl.smem_fwd;
   auto kern = bwd ? lstm_tc_bwd_kernel : lstm_tc_fwd_kernel;

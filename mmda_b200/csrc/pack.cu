@@ -191,10 +191,9 @@ int embedding_rows_det(float* dE, const float* dX, int N, int D, int V, int* wor
   return MMDA_OK;
 }
 
-extern "C" {
-
-int mmda_pack_build(const int* lens_sorted, int B, int Tmax, int N, int* batch_sizes,
-                    int* offsets, int* row_t, int* row_j, cudaStream_t stream) {
+// batch_sizes, offsets and the (t, j) coordinates of the N packed rows
+static int pack_build(const int* lens_sorted, int B, int Tmax, int N, int* batch_sizes,
+                      int* offsets, int* row_t, int* row_j, cudaStream_t stream) {
   MMDA_REQUIRE(B > 0 && Tmax > 0 && N > 0, "pack_build: empty batch (B=%d Tmax=%d N=%d)", B, Tmax, N);
   MMDA_REQUIRE(Tmax <= 8192, "pack_build: Tmax=%d too large", Tmax);
   pack_build_kernel<<<1, 256, (Tmax + 1) * sizeof(int), stream>>>(lens_sorted, B, Tmax,
@@ -205,10 +204,12 @@ int mmda_pack_build(const int* lens_sorted, int B, int Tmax, int N, int* batch_s
   return MMDA_OK;
 }
 
+extern "C" {
+
 int mmda_pack_build_padded(const int* lens_sorted, int B, int Tmax, int N, int Np, int* batch_sizes,
                            int* offsets, int* row_t, int* row_j, cudaStream_t stream) {
   MMDA_REQUIRE(Np >= N, "pack_build_padded: Np=%d < N=%d", Np, N);
-  int rc = mmda_pack_build(lens_sorted, B, Tmax, N, batch_sizes, offsets, row_t, row_j, stream);
+  int rc = pack_build(lens_sorted, B, Tmax, N, batch_sizes, offsets, row_t, row_j, stream);
   if (rc != MMDA_OK || Np == N) return rc;
   pack_tail_kernel<<<(Np - N + 255) / 256, 256, 0, stream>>>(N, Np, row_t, row_j);
   MMDA_CHECK_LAUNCH();

@@ -446,13 +446,13 @@ class MisaEngine:
 
     def _pack_weights(self, r, P, H, I):
         """Stacked gate-interleaved copy of layer r's W_ih (both directions), split into tf32
-        hi/lo for the 3xTF32 GEMMs (pack mode 1), + the bias stack."""
+        hi/lo for the 3xTF32 GEMMs, + the bias stack."""
         W = self._prep_buf(f"tcW_{r}", 8 * H, I, 0, split=True)
         bst = self.buf(f"bst_{r}", 8 * H)
         self.k._c("mmda_lstm_pack_weights", _ptr(P[f"{r}.weight_ih_l0"]),
                   _ptr(P[f"{r}.weight_ih_l0_reverse"]), _ptr(P[f"{r}.bias_ih_l0"]),
                   _ptr(P[f"{r}.bias_hh_l0"]), _ptr(P[f"{r}.bias_ih_l0_reverse"]),
-                  _ptr(P[f"{r}.bias_hh_l0_reverse"]), H, I, 1, _ptr(W[0]), _ptr(W[1]),
+                  _ptr(P[f"{r}.bias_hh_l0_reverse"]), H, I, _ptr(W[0]), _ptr(W[1]),
                   W[0].stride(0), _ptr(bst))
         return W, bst
 
@@ -753,13 +753,9 @@ class MisaEngine:
         ffn_tc = self._tc_lin_ok(rows, FF, d)
         if ffn_tc:
             self.tc_linear("ffn1", X1, P[TL + "linear1.weight"], P[TL + "linear1.bias"], F1)
-            if F1.is_contiguous():       # ReLU + dropout in one pass
-                k._c("mmda_act_dropout_forward", _ptr(F1), F1.numel(), ACT_RELU, p_att, seed,
-                     _ptr(seed_dev), 3)
-            else:
-                k.act(F1, ACT_RELU)
-                if p_att > 0:
-                    k.dropout(F1, F1, p_att, seed, 3, seed_dev)
+            # ReLU + dropout in one pass
+            k._c("mmda_act_dropout_forward", _ptr(F1), F1.numel(), ACT_RELU, p_att, seed,
+                 _ptr(seed_dev), 3)
         else:
             k.linear(X1, P[TL + "linear1.weight"], P[TL + "linear1.bias"], F1, act=ACT_RELU)
             if p_att > 0:
@@ -882,13 +878,9 @@ class MisaEngine:
             else:
                 k.linear_bwd(dF2, F1, P[TL + "linear2.weight"], G[TL + "linear2.weight"],
                              G[TL + "linear2.bias"], dF1, 0.0)
-            if dF1.is_contiguous() and F1.is_contiguous():      # dropout' + ReLU' in one pass
-                k._c("mmda_dropout_act_backward", _ptr(dF1), _ptr(F1), dF1.numel(), ACT_RELU, p_att,
-                     seed, _ptr(seed_dev), 3)
-            else:
-                if p_att > 0:
-                    k.dropout(dF1, dF1, p_att, seed, 3, seed_dev)
-                k.act_bwd(dF1, F1, ACT_RELU)
+            # dropout' + ReLU' in one pass
+            k._c("mmda_dropout_act_backward", _ptr(dF1), _ptr(F1), dF1.numel(), ACT_RELU, p_att,
+                 seed, _ptr(seed_dev), 3)
             # dX1 = dS2 + dF1 W1   (accumulate in place into dS2)
             if dF2 is dS2:
                 k.join_leaves()      # no dropout: dS2 is still being read as linear2's d(output)

@@ -19,8 +19,19 @@ def test_library_exports_every_declared_symbol():
     assert len(protos) >= 30
     for name in protos:
         assert hasattr(dll, name), f"{name} declared in include/mmda_b200.h but not exported"
-    assert LIB.load().mmda_abi_version() == 1
+    assert LIB.load().mmda_abi_version() == 2
     assert LIB.load().mmda_last_error() is not None
+
+
+def test_pack_weights_refuses_misaligned_outputs():
+    """A pack mode (0 / 1 / 2) in out_a's place, or any output that is no float array, is an
+    argument error before anything is launched (no GPU needed to see it)."""
+    pack = LIB.raw("mmda_lstm_pack_weights")
+    p = 1 << 40                                    # 16-byte aligned stand-in, never dereferenced
+    for out_a, out_b, bias in ((1, p, p), (2, p, p), (p, p + 2, p), (p, p, p + 1)):
+        rc = pack(p, p, p, p, p, p, 37, 23, out_a, out_b, 29, bias, None)
+        assert rc == -2, (out_a, out_b, bias, rc)    # MMDA_ERR_ARG
+        assert b"aligned" in LIB.load().mmda_last_error()
 
 
 def test_header_cites_reference_sites():

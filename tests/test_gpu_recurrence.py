@@ -218,26 +218,23 @@ def P(t):
 
 
 def spread(*shape, g):
-    """fp32 values over many binades (rounding of the tf32 / bf16 conversions is exercised)."""
+    """fp32 values over many binades (rounding of the tf32 conversion is exercised)."""
     return torch.randn(*shape, generator=g) * torch.pow(10.0, torch.randint(-6, 6, shape, generator=g).float())
 
 
-@pytest.mark.parametrize("mode", [0, 1, 2])
-def test_lstm_pack_weights(mode):
+def test_lstm_pack_weights_tf32_split():
     dev = torch.device("cuda:0")
-    g = torch.Generator().manual_seed(21 + mode)
+    g = torch.Generator().manual_seed(22)
     H, I, ld = 37, 23, 29
     w = [spread(4 * H, I, g=g) for _ in range(2)]
     b = [spread(4 * H, g=g) for _ in range(4)]       # b_ih_f, b_hh_f, b_ih_r, b_hh_r
     wd, bd = [x.to(dev) for x in w], [x.to(dev) for x in b]
     sentinel = -3.0
     out_a = torch.full((8 * H, ld), sentinel, device=dev)
-    if mode == 2:
-        out_a = torch.full((8 * H, ld), sentinel, dtype=torch.bfloat16, device=dev)
-    out_b = torch.full((8 * H, ld), sentinel, device=dev) if mode == 1 else None
+    out_b = torch.full((8 * H, ld), sentinel, device=dev)
     bias = torch.full((8 * H,), sentinel, device=dev)
     lib().call("mmda_lstm_pack_weights", P(wd[0]), P(wd[1]), P(bd[0]), P(bd[1]), P(bd[2]), P(bd[3]),
-               H, I, mode, P(out_a), P(out_b), ld, P(bias), torch.cuda.current_stream().cuda_stream)
+               H, I, P(out_a), P(out_b), ld, P(bias), torch.cuda.current_stream().cuda_stream)
     torch.cuda.synchronize()
     # row dir*4H + u*4 + g of the copy = row g*H + u of weight_ih_l0{,_reverse}
     W = torch.stack(w).view(2, 4, H, I).transpose(1, 2).reshape(8 * H, I)
@@ -246,19 +243,14 @@ def test_lstm_pack_weights(mode):
     got = out_a.cpu()
     assert torch.all(got[:, I:] == sentinel), "pitch columns past I were written"
     got = got[:, :I]
-    if mode == 0:
-        assert same_bits(got, W)
-    elif mode == 1:
-        lo = out_b.cpu()
-        assert torch.all(lo[:, I:] == sentinel)
-        lo = lo[:, :I]
-        bits = got.view(torch.int32)
-        assert torch.all(bits & 0x1FFF == 0), "hi is not tf32-representable"
-        rna = ((W.view(torch.int32) + 0x1000) & ~0x1FFF).view(torch.float32)   # round to nearest, ties away
-        assert same_bits(got, rna)
-        assert same_bits(got + lo, W), "hi + lo != w"
-    else:
-        assert torch.equal(got.view(torch.int16), W.to(torch.bfloat16).view(torch.int16))
+    lo = out_b.cpu()
+    assert torch.all(lo[:, I:] == sentinel)
+    lo = lo[:, :I]
+    bits = got.view(torch.int32)
+    assert torch.all(bits & 0x1FFF == 0), "hi is not tf32-representable"
+    rna = ((W.view(torch.int32) + 0x1000) & ~0x1FFF).view(torch.float32)   # round to nearest, ties away
+    assert same_bits(got, rna)
+    assert same_bits(got + lo, W), "hi + lo != w"
 
 
 def test_gru_expand_and_fold():

@@ -129,7 +129,7 @@ def rel(a, b):
 SENTINEL = -7.0e37      # fills the guard half of the backward scratch
 
 
-def run(c, which, dbg=None, save=1, fill=0.0):
+def run(c, which, save=1, fill=0.0):
     """One forward + backward launch pair through the C ABI.  y / c / utt start filled with
     `fill`; save=0 runs the forward alone with c = NULL.  The SIMT backward gets twice the scratch
     mmda_lstm_scratch_bytes reports, the second half filled with SENTINEL; out["scratch_overrun"]
@@ -311,24 +311,6 @@ def main():
     print("ms (copy subtracted): " + json.dumps({
         "fwd_tc": timeit(f_tc) - t_copy, "fwd_simt": timeit(f_simt) - t_copy,
         "bwd_tc": timeit(b_tc) - t_copy, "bwd_simt": timeit(b_simt) - t_copy, "copy": t_copy}), flush=True)
-
-    # ---- per-step phase stamps of CTA 0 (16 slots per step; see TCL_TS in lstm_tc.cu) ----
-    dbg = torch.zeros(16 * (c["Tmax"] + 1), dtype=torch.int64, device=dev)
-    LIB.call("mmda_lstm_tc_set_debug_buffer", P(dbg))
-    for name, fn in (("fwd", f_tc), ("bwd", b_tc)):
-        dbg.zero_()
-        fn(); torch.cuda.synchronize()
-        d = dbg.view(-1, 16)[: c["Tmax"]].cpu().double()
-        lo, hi = 5, c["Tmax"] - 2
-        if hi - lo < 2:
-            continue
-        rel0 = (d[lo:hi] - d[lo:hi, 0:1])
-        rel0[d[lo:hi] == 0] = float("nan")
-        means = rel0.nanmean(0).tolist()
-        step = (d[lo + 1:hi + 1, 0] - d[lo:hi, 0]).mean().item()
-        print(name, "stamps (clk after step start):",
-              {i: round(v) for i, v in enumerate(means) if v == v and i > 0}, "step", round(step), flush=True)
-    LIB.call("mmda_lstm_tc_set_debug_buffer", None)
 
 
 if __name__ == "__main__":
